@@ -33,6 +33,12 @@ streams), strong scaling over the N ranks, each with a parity sample.
 `--impl reference` times the reference's own CPU algorithm (the literal Python/NumPy port in
 oracle/pyref.py -- the reference is pure Python, so there is nothing faster to be fair to) on
 all host cores, on a bounded sample of the same workload.
+
+`--dump-outputs DIR` writes, as DIR/<name>.npy (float64), what the last timed step of each measured path left for
+its caller (rank 0's share with N > 1): the grid's count planes and occupancy map (cfg 5: the map), each as one
+fixed, seeded sample of cells plus the sum of every row, and the ICP transforms and iteration counts (cfg 4: a fixed,
+seeded sample of the pairs).  The inputs are seeded, so two builds run with the same arguments can be compared file
+for file.
 """
 import argparse
 import json
@@ -55,6 +61,9 @@ GRID_BEAMS = 1080
 ICP_BEAMS = 360
 ICP_SCANS = 10000
 FP64_PEAK_TFLOPS = 148 * 64 * 2 * 1.965e9 / 1e12  # nominal B200 vector FP64 (no measured figure)
+DUMP_CELLS = 1 << 19          # cells sampled from each map plane by --dump-outputs
+DUMP_PAIRS = 1 << 16          # cfg-4 pairs sampled by --dump-outputs
+DUMP_MAX_BYTES = 64 << 20     # all files of --dump-outputs together
 
 
 def measured_peaks():
@@ -82,6 +91,42 @@ def ncu_stamp(key):
         return ent if h.hexdigest() == ent["sha1"] else None
     except Exception:
         return None
+
+
+# =============================================================================== --dump-outputs
+
+def seeded_sample(n, k, seed):
+    """Sorted indices of a fixed, seeded sample of k of n elements (all n when k >= n)."""
+    if k >= n:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(seed).choice(n, k, replace=False))
+
+
+def keep_output(args, name, arr):
+    """Hold one output (a device tensor) of a timed step for --dump-outputs, as float64 on the host."""
+    args.outputs[name] = arr.cpu().numpy().astype(np.float64)
+
+
+def keep_grid_outputs(args, prefix, planes, seed):
+    """Grid outputs (2-D device tensors of one shape): every plane at the same seeded sample of cells, and the sum of
+    each of its rows, so that a change in any cell shows while the files stay small."""
+    import torch
+    first = next(iter(planes.values()))
+    idx = seeded_sample(first.numel(), DUMP_CELLS, seed)
+    args.outputs[prefix + "_cells"] = idx.astype(np.float64)
+    idx = torch.from_numpy(idx).to(first.device)
+    for name, plane in planes.items():
+        keep_output(args, "%s_%s_sample" % (prefix, name), plane.reshape(-1)[idx])
+        keep_output(args, "%s_%s_row_sums" % (prefix, name), plane.sum(dim=1, dtype=torch.int64))
+
+
+def write_outputs(outputs, out_dir):
+    total = sum(a.nbytes for a in outputs.values())
+    if total > DUMP_MAX_BYTES:
+        raise SystemExit("--dump-outputs: %d bytes of outputs, more than the %d allowed" % (total, DUMP_MAX_BYTES))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, arr in outputs.items():
+        np.save(os.path.join(out_dir, name + ".npy"), arr)
 
 
 # =============================================================================== clocks
@@ -374,6 +419,11 @@ def bench_grid(args, rank, world, torch, devapi, bdist, synth):
     clocks = sampler.stop()
     total_ms = bdist.max_over_ranks(sum(step_ms))
     ray_avg_ms = sum(ray_ms) / len(ray_ms)
+    if args.dump_outputs and rank == 0:
+        if p2p is not None:
+            keep_grid_outputs(args, "grid", {"pmap": p2p.pmap_dev}, seed=1)
+        else:
+            keep_grid_outputs(args, "grid", {"hit": hit, "miss": miss, "pmap": pmap}, seed=1)
 
     # ---- end to end through the host-buffer API (pinned host arrays in, occupancy map out)
     e2e_steps = max(3, min(args.steps, 10))
@@ -547,6 +597,9 @@ def bench_icp(args, rank, world, torch, devapi, bdist, synth):
     bdist.barrier()
     clocks = sampler.stop()
     total_ms = bdist.max_over_ranks(sum(step_ms))
+    if args.dump_outputs and rank == 0:
+        keep_output(args, "icp_T", T)
+        keep_output(args, "icp_iters", iters)
     it_total = int(iters.sum(dtype=torch.int64).item())
     evals = it_total * ICP_BEAMS * ICP_BEAMS
     flops = it_total * (5 * ICP_BEAMS * ICP_BEAMS + 24 * ICP_BEAMS) + P * 16 * ICP_BEAMS
@@ -673,6 +726,12 @@ def bench_cfg4(args, rank, world, torch, devapi, bdist):
         torch.cuda.synchronize()
         times.append(bdist.max_over_ranks(a.elapsed_time(b)))
     ms = min(times)
+    if args.dump_outputs and rank == 0:
+        idx = seeded_sample(hi - lo, DUMP_PAIRS, seed=2)
+        args.outputs["cfg4_pairs"] = idx.astype(np.float64)
+        idx = torch.from_numpy(idx).cuda()
+        keep_output(args, "cfg4_T", T[idx])
+        keep_output(args, "cfg4_iters", it[idx])
     from oracle import corc                     # the checker, on a sample; never the thing timed
     sample = min(64, hi - lo)
     want_T, want_it = corc.icp_batch(tar[:sample].cpu().numpy(), src[:sample].cpu().numpy(), 30, 1e-3)
@@ -717,6 +776,8 @@ def bench_cfg5(args, rank, world, torch, devapi, bdist, synth):
     b.record()
     torch.cuda.synchronize()
     sm.check()
+    if args.dump_outputs and rank == 0:
+        keep_grid_outputs(args, "cfg5", {"pmap": sm.pmap_dev}, seed=3)
     ms = bdist.max_over_ranks(a.elapsed_time(b)) / reps
     # parity: all 8 streams in one pass on this GPU, (1 + reps) times like the merged object saw them
     S, Hx, Hy = devapi.grid_scale(G, G, GRID_RESO)
@@ -825,7 +886,11 @@ def main():
     ap.add_argument("--only", default="both", choices=["both", "primary"])
     ap.add_argument("--cfg4-pairs", type=int, default=1000000, help="BASELINE.json config 4: total ICP pairs (0 skips it)")
     ap.add_argument("--cfg5-scans", type=int, default=4096, help="BASELINE.json config 5: scans per stream (0 skips it)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the b2slam arm")
+    args.outputs = {}
     args.warmup = max(args.warmup, 3) if args.impl == "b2slam" else args.warmup
 
     if args.impl == "reference":
@@ -900,6 +965,8 @@ def main():
             sec = results[order[1]]
             sec["cpu_baseline"] = cpu.get(order[1])
             line[order[1]] = sec
+        if args.dump_outputs:
+            write_outputs(args.outputs, args.dump_outputs)
         sys.stdout.flush()
         os.dup2(real_stdout, 1)
         print(json.dumps(line))

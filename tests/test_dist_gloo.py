@@ -16,8 +16,9 @@ from conftest import ROOT
 
 def _worker(rank, world, port, out_dir):
     sys.path.insert(0, ROOT)
+    # CPU tensors only: with GPUs visible, init() would bind rank r to GPU r, which a one-GPU machine lacks for rank 1
     os.environ.update(RANK=str(rank), LOCAL_RANK=str(rank), WORLD_SIZE=str(world),
-                      MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port))
+                      MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port), CUDA_VISIBLE_DEVICES="")
     import b2slam.dist as bdist
     import b2slam.synth as synth
     from oracle import corc
