@@ -14,8 +14,9 @@ namespace b2s {
 
 // 1: one RED per visit; 2: warp-aggregated runs; 3: same, lean inner loop;
 // 4: 3 + transposed scratch plane for y-major beams when a workspace is supplied, else 3;
-// 5 (default): 4 + a test-free core phase of the march
-int g_grid_variant = 5;
+// 5: 4 + a test-free core phase of the march; 6 (default): consecutive scans counted in a shared-memory tile, 5 where
+// the tile does not fit
+int g_grid_variant = 6;
 
 // ------------------------------------------------------------------------------------------
 // Per-beam setup shared by all variants.
@@ -429,20 +430,22 @@ __device__ __forceinline__ void load_beam(const ScanInput &in, long long i, int 
     }
 }
 
-// SIGN = +1 applies a batch, SIGN = -1 takes the same batch back out (exact inverse: integer adds).
+// The march of variants 4 / 5 for one warp: lane l ray-casts beam i (flat index scan * beams + beam) when `valid`.
+// All 32 lanes call it together.  SIGN = +1 applies a batch, SIGN = -1 takes the same batch back out (exact inverse:
+// integer adds).
 template <int SIGN, int MODE, bool CORE_PHASE>
-__global__ void __launch_bounds__(256, 8)
-grid_raycast_v4(int32_t *__restrict__ hit, int32_t *__restrict__ miss, int32_t *__restrict__ scratch_t,
-                GridWorkspace *__restrict__ ws, uint8_t *__restrict__ dirty, int xw, int yw, double cells_per_m,
-                double off_x, double off_y, const ScanInput in, long long total, int beams, int32_t *counters)
+__device__ __forceinline__ void raycast_warp_v4(int32_t *__restrict__ hit, int32_t *__restrict__ miss,
+                                                int32_t *__restrict__ scratch_t, GridWorkspace *__restrict__ ws,
+                                                uint8_t *__restrict__ dirty, int xw, int yw, double cells_per_m,
+                                                double off_x, double off_y, const ScanInput &in, long long i, bool valid,
+                                                int beams, int32_t *counters)
 {
-    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     const unsigned lane = threadIdx.x & 31;
     Beam b;
     b.major0 = b.minor0 = b.span = b.inc = b.hit_k = b.steep = b.hx = b.hy = b.sx = b.sy = 0;
     b.slope = 0.0;
     int st = BEAM_NOOP;
-    if (i < total) {
+    if (valid) {
         double fox, foy, fcx, fcy;
         load_beam<MODE>(in, i, beams, fox, foy, fcx, fcy);
         st = beam_setup(fox, foy, fcx, fcy, xw, yw, cells_per_m, off_x, off_y, b);
@@ -541,6 +544,158 @@ grid_raycast_v4(int32_t *__restrict__ hit, int32_t *__restrict__ miss, int32_t *
     for (; t <= tmax; ++t)
         march_step4<false, SIGN>(t, delay, slope, acc, cmaj2, minor2, pitch2, inc2, wmin2, t_em, em_len, dead_key, lane1,
                            plane_base);
+}
+
+template <int SIGN, int MODE, bool CORE_PHASE>
+__global__ void __launch_bounds__(256, 8)
+grid_raycast_v4(int32_t *__restrict__ hit, int32_t *__restrict__ miss, int32_t *__restrict__ scratch_t,
+                GridWorkspace *__restrict__ ws, uint8_t *__restrict__ dirty, int xw, int yw, double cells_per_m,
+                double off_x, double off_y, const ScanInput in, long long total, int beams, int32_t *counters)
+{
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    raycast_warp_v4<SIGN, MODE, CORE_PHASE>(hit, miss, scratch_t, ws, dirty, xw, yw, cells_per_m, off_x, off_y, in, i,
+                                            i < total, beams, counters);
+}
+
+// ------------------------------------------------------------------------------------------
+// Variant 6 (default): consecutive scans counted in a shared-memory tile.
+//
+// The scans of a trajectory overlap: consecutive scans are a few cells apart and each covers a disk of 60-200 cells,
+// so V6_SCANS consecutive scans visit almost the same cells.  A CTA takes V6_SCANS consecutive scans x one sector of
+// V6_SECTOR adjacent beams, finds the bounding box of everything they touch, and -- when that box fits the tile and
+// no ray is clipped by the grid -- counts every visit with an unpredicated shared atomicAdd (ATOMS.POPC.INC: lanes on
+// the same word merge in hardware, no run finding, no divergent region), then adds the tile to `miss` with coalesced
+// full-warp REDs.  Each lane marches its own beam with the reference's float64 recurrence; lanes need not move in
+// step.  A CTA whose box does not fit, or that has a clipped ray, runs the variant-5 march for its beams instead
+// (random scans, map edges), so any input stays exact.  Integer adds commute: the counts are those of variant 5.
+constexpr int V6_SCANS = 16;
+constexpr int V6_SECTOR = 64;     // beams; two warps of one scan, so a warp holds 32 adjacent beams
+constexpr int V6_THREADS = V6_SCANS * V6_SECTOR;  // one beam per thread
+constexpr int V6_TILE_WORDS = 27 * 1024;  // 108 KB: two CTAs of 1024 threads per SM
+
+// [BRES]:51-55 on a shared-memory byte address: acc += slope; if (acc >= 0.5) { addr += dmin; acc -= 1.0; } addr += dmaj
+__device__ __forceinline__ void tile_step(double &acc, unsigned &addr, double slope, unsigned dmin, unsigned dmaj)
+{
+    asm("{\n\t"
+        ".reg .pred p;\n\t"
+        "add.rn.f64 %0, %0, %2;\n\t"
+        "setp.ge.f64 p, %0, 0d3FE0000000000000;\n\t"
+        "@p add.rn.f64 %0, %0, 0dBFF0000000000000;\n\t"
+        "@p add.s32 %1, %1, %3;\n\t"
+        "}"
+        : "+d"(acc), "+r"(addr)
+        : "d"(slope), "r"(dmin));
+    addr += dmaj;
+}
+
+// One beam's misses into the tile: word (x - bx) * pitch + (y - by) counts cell (x, y); the box holds the whole path.
+__device__ __forceinline__ void march_tile(const Beam &b, unsigned tile_base, int bx, int by, int pitch)
+{
+    // tile word of the canonical start; the major axis advances by dmaj bytes per step, the minor axis by dmin
+    const int mx = b.steep ? b.minor0 : b.major0, my = b.steep ? b.major0 : b.minor0;
+    unsigned addr = tile_base + 4u * (unsigned)((mx - bx) * pitch + (my - by));
+    const unsigned dmaj = 4u * (b.steep ? 1u : (unsigned)pitch);
+    const unsigned dmin = 4u * (unsigned)(b.steep ? b.inc * pitch : b.inc);
+    const double slope = b.slope;
+    double acc = 0.0;
+    // the path is k = 0 .. span; every cell but the obstacle's (k = hit_k: span, or 0 when flipped) is a miss
+    if (b.hit_k == 0) tile_step(acc, addr, slope, dmin, dmaj);
+    // unpredicated: ATOMS.POPC.INC, lanes on one word merge (a predicated shared atomic becomes a divergent region)
+#pragma unroll 4
+    for (int n = b.span; n > 0; --n) {
+        asm volatile("red.shared.add.u32 [%0], 1;" ::"r"(addr) : "memory");
+        tile_step(acc, addr, slope, dmin, dmaj);
+    }
+}
+
+template <int MODE>
+__global__ void __launch_bounds__(V6_THREADS, 2)
+grid_raycast_v6(int32_t *__restrict__ hit, int32_t *__restrict__ miss, int32_t *__restrict__ scratch_t,
+                GridWorkspace *__restrict__ ws, uint8_t *__restrict__ dirty, int xw, int yw, double cells_per_m,
+                double off_x, double off_y, const ScanInput in, int scans, int beams, int32_t *counters)
+{
+    extern __shared__ uint32_t tile[];
+    __shared__ int box[5];  // -xmin, xmax, -ymin, ymax over the live beams (max-reduced), clipped flag
+    const int lane = threadIdx.x & 31;
+    const int sectors = (beams + V6_SECTOR - 1) / V6_SECTOR;
+    const int s0 = (int)(blockIdx.x / sectors) * V6_SCANS, b0 = (int)(blockIdx.x % sectors) * V6_SECTOR;
+    const int s = s0 + (int)threadIdx.x / V6_SECTOR, bm = b0 + (int)threadIdx.x % V6_SECTOR;
+    const bool valid = s < scans && bm < beams;
+    const long long i = (long long)s * beams + bm;
+    if (threadIdx.x < 5) box[threadIdx.x] = threadIdx.x < 4 ? (int)0x80808080 : 0;
+    __syncthreads();
+
+    // ---- set-up: bounding box of the sensor and obstacle cells of the live beams, and whether any ray is clipped
+    {
+        const int very_neg = (int)0x80808080;
+        int nx0 = very_neg, x1 = very_neg, ny0 = very_neg, y1 = very_neg;
+        bool clipped = false;
+        Beam b;
+        if (valid) {
+            double fox, foy, fcx, fcy;
+            load_beam<MODE>(in, i, beams, fox, foy, fcx, fcy);
+            if (beam_setup(fox, foy, fcx, fcy, xw, yw, cells_per_m, off_x, off_y, b) == BEAM_OK) {
+                nx0 = -min(b.sx, b.hx);
+                x1 = max(b.sx, b.hx);
+                ny0 = -min(b.sy, b.hy);
+                y1 = max(b.sy, b.hy);
+                clipped = -nx0 < 0 || x1 >= xw || -ny0 < 0 || y1 >= yw;
+            }
+        }
+        nx0 = __reduce_max_sync(0xffffffffu, nx0);
+        x1 = __reduce_max_sync(0xffffffffu, x1);
+        ny0 = __reduce_max_sync(0xffffffffu, ny0);
+        y1 = __reduce_max_sync(0xffffffffu, y1);
+        clipped = __any_sync(0xffffffffu, clipped);
+        if (lane < 4) atomicMax(&box[lane], lane == 0 ? nx0 : lane == 1 ? x1 : lane == 2 ? ny0 : y1);
+        if (lane == 4 && clipped) box[4] = 1;
+    }
+    __syncthreads();
+    const int bx = -box[0], by = -box[2];
+    const bool empty = box[1] < 0;  // no live beam: nothing but status counts
+    const int w = empty ? 0 : box[1] - bx + 1, h = empty ? 0 : box[3] - by + 1;
+    const int pitch = h | 1;  // odd: the words of a y-major warp (one per row) spread over all banks
+    if (box[4] || (long long)w * pitch > V6_TILE_WORDS) {
+        raycast_warp_v4<1, MODE, true>(hit, miss, scratch_t, ws, dirty, xw, yw, cells_per_m, off_x, off_y, in, i, valid,
+                                       beams, counters);
+        return;
+    }
+
+    // ---- private path: the box lies inside the grid
+    for (int k = threadIdx.x; k < w * pitch; k += V6_THREADS) tile[k] = 0;
+    if (!empty) {
+        const int tx0 = bx / GRID_TILE, ty0 = by / GRID_TILE, ny = box[3] / GRID_TILE - ty0 + 1;
+        const int cnt = ((bx + w - 1) / GRID_TILE - tx0 + 1) * ny, tiles_y = grid_tiles(yw);
+        for (int k = threadIdx.x; k < cnt; k += V6_THREADS) dirty[(tx0 + k / ny) * tiles_y + ty0 + k % ny] = 1;
+    }
+    __syncthreads();
+    if (valid) {
+        double fox, foy, fcx, fcy;
+        load_beam<MODE>(in, i, beams, fox, foy, fcx, fcy);
+        Beam b;
+        const int st = beam_setup(fox, foy, fcx, fcy, xw, yw, cells_per_m, off_x, off_y, b);
+        if (st == BEAM_OK) {
+            atomicAdd(hit + (b.hx * yw + b.hy), 1);  // the obstacle cell: last path element, inside the grid here
+            march_tile(b, smem_addr(tile), bx, by, pitch);
+        } else {
+            count_status(st, counters);
+        }
+    }
+    __syncthreads();
+
+    // ---- flush: rows of the box, in 32-cell segments aligned in the plane; all-zero segments are skipped
+    const int warp = threadIdx.x >> 5, nwarps = V6_THREADS / 32;
+    const int g0 = by >> 5, nseg = empty ? 0 : ((by + h - 1) >> 5) - g0 + 1;
+    for (int q = warp; q < w * nseg; q += nwarps) {
+        const int r = q / nseg, y = ((g0 + q % nseg) << 5) + lane;
+        const bool inside = y >= by && y < by + h;
+        const int v = inside ? (int)tile[r * pitch + (y - by)] : 0;
+        if (__any_sync(0xffffffffu, v != 0)) {
+            // every lane adds (0 outside the box); past the last column it adds to a cell of its own row
+            int32_t *p = miss + (size_t)(bx + r) * yw + min(y, yw - 1);
+            asm volatile("red.global.add.s32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
+        }
+    }
 }
 
 // miss[x][y] += scratch_t[y][x] over the recorded bounding box, scratch_t cleared on the way.
@@ -803,12 +958,26 @@ static int raycast_v4_launch(int32_t *hit, int32_t *miss, int xw, int yw, double
                                                                                   xw, yw, cells_per_m, off_x, off_y, \
                                                                                   in, total, beams, counters);       \
     } while (0)
-    if (sign >= 0) {
+    // variant 6 for a batch that is applied; taking one back out stays on the variant-5 march
+#define B2S_V6(FU)                                                                                                 \
+    do {                                                                                                           \
+        const int tile_bytes = V6_TILE_WORDS * (int)sizeof(uint32_t);                                              \
+        B2S_CUDA(cudaFuncSetAttribute(grid_raycast_v6<FU>, cudaFuncAttributeMaxDynamicSharedMemorySize, tile_bytes)); \
+        const long long ctas = (long long)((scans + V6_SCANS - 1) / V6_SCANS) * ((beams + V6_SECTOR - 1) / V6_SECTOR); \
+        B2S_REQUIRE(ctas < (1ll << 31), "b2s_grid_raycast_ws: too many beams for one launch");                  \
+        grid_raycast_v6<FU><<<(unsigned)ctas, V6_THREADS, tile_bytes, st>>>(hit, miss, scratch_t, ws, dirty, xw, yw,  \
+                                                                          cells_per_m, off_x, off_y, in, scans,     \
+                                                                          beams, counters);                         \
+    } while (0)
+    if (sign >= 0 && g_grid_variant >= 6) {
+        if (mode == IN_FUSED) B2S_V6(IN_FUSED); else if (mode == IN_F64) B2S_V6(IN_F64); else B2S_V6(IN_F32);
+    } else if (sign >= 0) {
         if (mode == IN_FUSED) B2S_V4(1, IN_FUSED); else if (mode == IN_F64) B2S_V4(1, IN_F64); else B2S_V4(1, IN_F32);
     } else {
         if (mode == IN_FUSED) B2S_V4(-1, IN_FUSED); else if (mode == IN_F64) B2S_V4(-1, IN_F64); else B2S_V4(-1, IN_F32);
     }
 #undef B2S_V4
+#undef B2S_V6
     B2S_CUDA(cudaGetLastError());
     if (!fold) return B2S_OK;
     long long ftiles = (long long)((xw + 31) / 32) * ((yw + 31) / 32);

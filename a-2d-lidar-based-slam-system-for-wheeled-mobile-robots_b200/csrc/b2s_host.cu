@@ -237,7 +237,7 @@ extern "C" int b2s_tune(const char *key, int value)
     B2S_REQUIRE(key, "b2s_tune: null key");
     ++g_tune_gen;
     if (strcmp(key, "grid_variant") == 0) {
-        B2S_REQUIRE(value >= 1 && value <= 5, "b2s_tune: grid_variant must be 1..5");
+        B2S_REQUIRE(value >= 1 && value <= 6, "b2s_tune: grid_variant must be 1..6");
         g_grid_variant = value;
         return B2S_OK;
     }

@@ -3,6 +3,9 @@
 //   redg32 / redg64 : red.global.add on spread addresses inside an L2-resident 64 MiB plane, A of 32 lanes active
 //   atoms32         : atomicAdd on shared memory, spread addresses inside a 64 KiB tile
 //   bulkred         : cp.reduce.async.bulk.global.shared::cta.add.s32 of ROW-byte rows (TMA reduce)
+//   atoms_popc      : unpredicated atomicAdd(&smem, 1) (ATOMS.POPC.INC), L lanes per word
+//   atoms_walk      : the same instruction from fanned-out "beams" walking a row-major tile, x-major or y-major,
+//                     odd or even row pitch (bank conflicts of the y-major walk)
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdio.h>
@@ -87,6 +90,46 @@ __global__ void __launch_bounds__(256) k_atoms_scatter(int *out, int iters)
     if (threadIdx.x == 0) out[blockIdx.x] = tile[0];
 }
 
+// Unpredicated atomicAdd(&tile[w], 1) with an unused result compiles to ATOMS.POPC.INC (no divergent region).
+// LPW adjacent lanes share one word; the warp's words are consecutive.
+template <int LPW>
+__global__ void __launch_bounds__(256) k_atoms_popc(int *out, int iters)
+{
+    extern __shared__ int tile[];
+    for (int i = threadIdx.x; i < 16384; i += 256) tile[i] = 0;
+    __syncthreads();
+    uint32_t s = blockIdx.x * 256 + threadIdx.x + 1;
+    const int lane = threadIdx.x & 31;
+    for (int i = 0; i < iters; ++i) {
+        uint32_t base = __shfl_sync(0xffffffffu, lcg(s), 0) & 16383u;
+        atomicAdd(&tile[(base + lane / LPW) & 16383], 1);
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) out[blockIdx.x] = tile[0];
+}
+
+// 32 beams fanned out over 1/32 of a radian each, walked from a common origin in a row-major tile of PITCH words
+// per row: at step i lane l sits (l * i) / 64 cells off the warp's common line.  X-major: the step moves along a
+// row (+PITCH per step is the other axis: rows are x); Y-major: the step moves down the row, lanes spread over
+// rows, so their words are PITCH apart -- an even pitch puts them in few banks.
+template <bool YMAJOR, int PITCH>
+__global__ void __launch_bounds__(256) k_atoms_walk(int *out, int iters)
+{
+    extern __shared__ int tile[];
+    for (int i = threadIdx.x; i < PITCH * 160; i += 256) tile[i] = 0;
+    __syncthreads();
+    const int lane = threadIdx.x & 31;
+    for (int it = 0; it < iters; it += 128) {
+        for (int i = 0; i < 128; ++i) {
+            const int spread = (lane * i) >> 6;  // 0 .. 63
+            const int x = YMAJOR ? spread : i, y = YMAJOR ? i : spread;
+            atomicAdd(&tile[x * PITCH + y], 1);
+        }
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) out[blockIdx.x] = tile[0];
+}
+
 // plain (non-atomic) shared-memory read-modify-write, for the ownership-based designs
 __global__ void __launch_bounds__(256) k_smem_rmw(int *out, int iters)
 {
@@ -164,6 +207,9 @@ int main()
         name, active, ms, (double)blocks * 8 * iters * active / (ms * 1e-3) / 1e9, \
         (double)blocks * 8 * iters * active / (ms * 1e-3) / clk / sms, (ms * 1e-3) * clk * sms / ((double)blocks * 8 * iters))
     float ms;
+#define REPORT2(name, active, ms, it) printf("%-26s active=%2d  %8.3f ms  %7.2f Gops/s  %6.3f lane-ops/clk/SM  %6.2f clk per warp-instr per SM\n", \
+        name, active, ms, (double)blocks * 8 * (it) * active / (ms * 1e-3) / 1e9, \
+        (double)blocks * 8 * (it) * active / (ms * 1e-3) / clk / sms, (ms * 1e-3) * clk * sms / ((double)blocks * 8 * (it)))
     ms = time_ms([&] { k_redg<32, false><<<blocks, 256>>>(plane, mask, iters); }); REPORT("redg32 contiguous lanes", 32, ms);
     ms = time_ms([&] { k_redg<16, false><<<blocks, 256>>>(plane, mask, iters); }); REPORT("redg32 contiguous lanes", 16, ms);
     ms = time_ms([&] { k_redg<8, false><<<blocks, 256>>>(plane, mask, iters); }); REPORT("redg32 contiguous lanes", 8, ms);
@@ -193,5 +239,25 @@ int main()
     ms = time_ms([&] { k_bulkred<64><<<blocks, 256>>>(plane, mask, iters); }); REPORT("bulk reduce 64 B rows", 16, ms);
     ms = time_ms([&] { k_bulkred<128><<<blocks, 256>>>(plane, mask, iters); }); REPORT("bulk reduce 128 B rows", 32, ms);
     ms = time_ms([&] { k_bulkred<256><<<blocks, 256>>>(plane, mask, iters); }); REPORT("bulk reduce 256 B rows", 64, ms);
+    {
+        const int tile_bytes = 161 * 160 * 4;  // also holds PITCH = 160
+        CK(cudaFuncSetAttribute(k_atoms_popc<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, 65536));
+        CK(cudaFuncSetAttribute(k_atoms_popc<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, 65536));
+        CK(cudaFuncSetAttribute(k_atoms_popc<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, 65536));
+        CK(cudaFuncSetAttribute(k_atoms_popc<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, 65536));
+        CK(cudaFuncSetAttribute(k_atoms_walk<false, 161>, cudaFuncAttributeMaxDynamicSharedMemorySize, tile_bytes));
+        CK(cudaFuncSetAttribute(k_atoms_walk<true, 161>, cudaFuncAttributeMaxDynamicSharedMemorySize, tile_bytes));
+        CK(cudaFuncSetAttribute(k_atoms_walk<false, 160>, cudaFuncAttributeMaxDynamicSharedMemorySize, tile_bytes));
+        CK(cudaFuncSetAttribute(k_atoms_walk<true, 160>, cudaFuncAttributeMaxDynamicSharedMemorySize, tile_bytes));
+        ms = time_ms([&] { k_atoms_popc<1><<<blocks, 256, 65536>>>(out, iters); }); REPORT("atoms.popc.inc 1 lane/word", 32, ms);
+        ms = time_ms([&] { k_atoms_popc<2><<<blocks, 256, 65536>>>(out, iters); }); REPORT("atoms.popc.inc 2 lanes/word", 32, ms);
+        ms = time_ms([&] { k_atoms_popc<4><<<blocks, 256, 65536>>>(out, iters); }); REPORT("atoms.popc.inc 4 lanes/word", 32, ms);
+        ms = time_ms([&] { k_atoms_popc<32><<<blocks, 256, 65536>>>(out, iters); }); REPORT("atoms.popc.inc 32 lanes/word", 32, ms);
+        const int wi = 2048;  // multiple of 128
+        ms = time_ms([&] { k_atoms_walk<false, 161><<<blocks, 256, tile_bytes>>>(out, wi); }); REPORT2("walk x-major, pitch 161", 32, ms, wi);
+        ms = time_ms([&] { k_atoms_walk<true, 161><<<blocks, 256, tile_bytes>>>(out, wi); }); REPORT2("walk y-major, pitch 161", 32, ms, wi);
+        ms = time_ms([&] { k_atoms_walk<false, 160><<<blocks, 256, tile_bytes>>>(out, wi); }); REPORT2("walk x-major, pitch 160", 32, ms, wi);
+        ms = time_ms([&] { k_atoms_walk<true, 160><<<blocks, 256, tile_bytes>>>(out, wi); }); REPORT2("walk y-major, pitch 160", 32, ms, wi);
+    }
     return 0;
 }

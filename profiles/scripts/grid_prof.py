@@ -1,5 +1,5 @@
 """Minimal grid ray-cast launcher for ncu / timing: the cfg-3 bench launch (16 384 scans x 1080 beams, 4096^2 @ 5 cm).
-   python profiles/scripts/grid_prof.py [variant 1..5] [scans]
+   python profiles/scripts/grid_prof.py [variant 1..6] [scans]
 Prints the CUDA-event time of the ray-cast (+ fold) averaged over 10 launches on zeroed planes, L2 flushed between."""
 import os
 import sys
