@@ -43,7 +43,9 @@ __device__ __forceinline__ double cell_coord(double v, double cells_per_m, doubl
 
 // Coordinates arrive as float64: float32 endpoints are upcast exactly by the callers, the fused
 // ingestion path (ranges + pose) computes them in float64 like the reference does.
-__device__ __forceinline__ int beam_setup(double fox, double foy, double fcx, double fcy, int xw, int yw,
+// The first half of the set-up: sensor and obstacle cells, the span and the beam's status (all that a bounding box
+// needs; no division).
+__device__ __forceinline__ int beam_cells(double fox, double foy, double fcx, double fcy, int xw, int yw,
                                           double cells_per_m, double off_x, double off_y, Beam &b)
 {
     if (isinf(fox)) return BEAM_INF_SKIP;  // [MAP]:30 tests ox only
@@ -53,15 +55,26 @@ __device__ __forceinline__ int beam_setup(double fox, double foy, double fcx, do
     const double dxc = cell_coord(fcx, cells_per_m, off_x), dyc = cell_coord(fcy, cells_per_m, off_y);
     const double lim = 1073741824.0;  // 2^30: keeps every difference inside int32
     if (!(fabs(dxo) < lim && fabs(dyo) < lim && fabs(dxc) < lim && fabs(dyc) < lim)) return BEAM_TOO_LONG;
-    int x0 = __double2int_rz(dxc), y0 = __double2int_rz(dyc);  // sensor cell
-    int x1 = __double2int_rz(dxo), y1 = __double2int_rz(dyo);  // obstacle cell
-    if (x0 == x1 && y0 == y1) return BEAM_NOOP;                // [BRES]:10-11 empty path
+    const int x0 = __double2int_rz(dxc), y0 = __double2int_rz(dyc);  // sensor cell
+    const int x1 = __double2int_rz(dxo), y1 = __double2int_rz(dyo);  // obstacle cell
+    if (x0 == x1 && y0 == y1) return BEAM_NOOP;                      // [BRES]:10-11 empty path
     // no cell of the segment's bounding box inside the grid -> nothing to update
     if (max(x0, x1) < 0 || min(x0, x1) >= xw || max(y0, y1) < 0 || min(y0, y1) >= yw) return BEAM_NOOP;
     b.hx = x1;
     b.hy = y1;
     b.sx = x0;
     b.sy = y0;
+    b.span = max(abs(x1 - x0), abs(y1 - y0));  // the major axis' extent
+    if (b.span > B2S_MAX_PATH_CELLS) return BEAM_TOO_LONG;
+    return BEAM_OK;
+}
+
+__device__ __forceinline__ int beam_setup(double fox, double foy, double fcx, double fcy, int xw, int yw,
+                                          double cells_per_m, double off_x, double off_y, Beam &b)
+{
+    const int st = beam_cells(fox, foy, fcx, fcy, xw, yw, cells_per_m, off_x, off_y, b);
+    if (st != BEAM_OK) return st;
+    int x0 = b.sx, y0 = b.sy, x1 = b.hx, y1 = b.hy;
     const int steep = abs(y1 - y0) > abs(x1 - x0);
     if (steep) {
         int t = x0; x0 = y0; y0 = t;
@@ -72,8 +85,6 @@ __device__ __forceinline__ int beam_setup(double fox, double foy, double fcx, do
         int t = x0; x0 = x1; x1 = t;
         t = y0; y0 = y1; y1 = t;
     }
-    b.span = x1 - x0;
-    if (b.span > B2S_MAX_PATH_CELLS) return BEAM_TOO_LONG;
     b.major0 = x0;
     b.minor0 = y0;
     b.inc = (y0 < y1) ? 1 : -1;
@@ -568,23 +579,47 @@ grid_raycast_v4(int32_t *__restrict__ hit, int32_t *__restrict__ miss, int32_t *
 // full-warp REDs.  Each lane marches its own beam with the reference's float64 recurrence; lanes need not move in
 // step.  A CTA whose box does not fit, or that has a clipped ray, runs the variant-5 march for its beams instead
 // (random scans, map edges), so any input stays exact.  Integer adds commute: the counts are those of variant 5.
+//
+// A CTA's beams form 32 warp-units: 32 adjacent beams of one scan each (unit u: scan u / 2, beams 32 * (u & 1) ..
+// + 31 of the sector).  Layout 1 (default) runs 512 threads, two units per warp: the box pass measures each unit's
+// longest beam, and warp w marches the unit of rank w, then that of rank 31 - w (longest with shortest).  The scans of
+// a CTA differ in length by up to 2x, and the CTA holds its tile until its last warp is done; pairing brings the
+// warps' march lengths within a few percent of each other.  Layout 0 runs 1024 threads, one unit per warp, in order.
 constexpr int V6_SCANS = 16;
-constexpr int V6_SECTOR = 64;     // beams; two warps of one scan, so a warp holds 32 adjacent beams
-constexpr int V6_THREADS = V6_SCANS * V6_SECTOR;  // one beam per thread
-constexpr int V6_TILE_WORDS = 27 * 1024;  // 108 KB: two CTAs of 1024 threads per SM
+constexpr int V6_SECTOR = 64;     // beams; two units of one scan
+constexpr int V6_UNITS = V6_SCANS * V6_SECTOR / 32;
+constexpr int V6_TILE_WORDS = 27 * 1024;  // 108 KB: two CTAs per SM
+int g_grid_tile_layout = 1;
 
-// [BRES]:51-55 on a shared-memory byte address: acc += slope; if (acc >= 0.5) { addr += dmin; acc -= 1.0; } addr += dmaj
+#ifdef B2S_GRID_PHASES
+// Diagnostic build only (profiles/scripts/grid_phases.py): per CTA, V6_PHASE_WORDS clock64 stamps.  Word 0: %smid,
+// 1..5: start, box known, tile zeroed, march done, end; 6: 1 when the CTA fell back; 7: warps; 8 + w: warp w's march end.
+constexpr int V6_PHASE_WORDS = 8 + V6_UNITS;
+__device__ unsigned long long *g_grid_phases;
+extern "C" int b2s_grid_phases_buffer(void *rec)
+{
+    B2S_CUDA(cudaMemcpyToSymbol(g_grid_phases, &rec, sizeof(rec)));
+    return B2S_OK;
+}
+#define V6_STAMP(word, value)                                                                                      \
+    do {                                                                                                           \
+        if (g_grid_phases) g_grid_phases[(size_t)blockIdx.x * V6_PHASE_WORDS + (word)] = (value);                 \
+    } while (0)
+#else
+#define V6_STAMP(word, value) do { } while (0)
+#endif
+
+// [BRES]:51-55 on a shared-memory byte address: acc += slope; if (acc >= 0.5) { addr += dmin; acc -= 1.0; } addr += dmaj.
+// For a finite acc, acc >= 0.5 exactly when the high word, read as a signed int, is >= 0x3FE00000 (0.5 has a zero low
+// word; negative values and -0.0 have the sign bit set).  acc - 0.0 == acc bit for bit (-0.0 included), so subtracting
+// c = 1.0 or 0.0, built from one select on its high word, is the reference's conditional acc -= 1.0: one integer
+// compare instead of an FP64 one, and the second DADD needs no select after it.
 __device__ __forceinline__ void tile_step(double &acc, unsigned &addr, double slope, unsigned dmin, unsigned dmaj)
 {
-    asm("{\n\t"
-        ".reg .pred p;\n\t"
-        "add.rn.f64 %0, %0, %2;\n\t"
-        "setp.ge.f64 p, %0, 0d3FE0000000000000;\n\t"
-        "@p add.rn.f64 %0, %0, 0dBFF0000000000000;\n\t"
-        "@p add.s32 %1, %1, %3;\n\t"
-        "}"
-        : "+d"(acc), "+r"(addr)
-        : "d"(slope), "r"(dmin));
+    acc = __dadd_rn(acc, slope);
+    const bool up = __double2hiint(acc) >= 0x3FE00000;
+    acc = __dsub_rn(acc, __hiloint2double(up ? 0x3FF00000 : 0, 0));
+    if (up) addr += dmin;
     addr += dmaj;
 }
 
@@ -608,38 +643,70 @@ __device__ __forceinline__ void march_tile(const Beam &b, unsigned tile_base, in
     }
 }
 
-template <int MODE>
-__global__ void __launch_bounds__(V6_THREADS, 2)
+// Flat index of this lane's beam in unit u of the CTA whose first scan is s0 and first beam b0; false past the input.
+__device__ __forceinline__ bool v6_beam(int u, int s0, int b0, int scans, int beams, long long &i)
+{
+    const int s = s0 + (u >> 1), bm = b0 + 32 * (u & 1) + (int)(threadIdx.x & 31);
+    i = (long long)s * beams + bm;
+    return s < scans && bm < beams;
+}
+
+// UNITS: warp-units per warp (layout 0: 1, layout 1: 2).
+template <int MODE, int UNITS>
+__global__ void __launch_bounds__(V6_UNITS * 32 / UNITS, 2)
 grid_raycast_v6(int32_t *__restrict__ hit, int32_t *__restrict__ miss, int32_t *__restrict__ scratch_t,
                 GridWorkspace *__restrict__ ws, uint8_t *__restrict__ dirty, int xw, int yw, double cells_per_m,
                 double off_x, double off_y, const ScanInput in, int scans, int beams, int32_t *counters)
 {
+    static_assert(UNITS == 1 || UNITS == 2, "a warp marches one unit, or a long and a short one");
+    constexpr int NWARPS = V6_UNITS / UNITS;
     extern __shared__ uint32_t tile[];
     __shared__ int box[5];  // -xmin, xmax, -ymin, ymax over the live beams (max-reduced), clipped flag
-    const int lane = threadIdx.x & 31;
+    __shared__ int unit_span[V6_UNITS];  // longest live beam of each unit, -1 if none (layout 1)
+    __shared__ int order[V6_UNITS];      // units by decreasing span, ties by index (layout 1)
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+#ifdef B2S_GRID_PHASES
+    if (threadIdx.x == 0) {
+        unsigned smid;
+        asm volatile("mov.u32 %0, %%smid;" : "=r"(smid));
+        V6_STAMP(0, smid);
+        V6_STAMP(1, clock64());
+        V6_STAMP(7, NWARPS);
+    }
+#endif
     const int sectors = (beams + V6_SECTOR - 1) / V6_SECTOR;
     const int s0 = (int)(blockIdx.x / sectors) * V6_SCANS, b0 = (int)(blockIdx.x % sectors) * V6_SECTOR;
-    const int s = s0 + (int)threadIdx.x / V6_SECTOR, bm = b0 + (int)threadIdx.x % V6_SECTOR;
-    const bool valid = s < scans && bm < beams;
-    const long long i = (long long)s * beams + bm;
     if (threadIdx.x < 5) box[threadIdx.x] = threadIdx.x < 4 ? (int)0x80808080 : 0;
     __syncthreads();
 
-    // ---- set-up: bounding box of the sensor and obstacle cells of the live beams, and whether any ray is clipped
+    // ---- box pass: bounding box of the sensor and obstacle cells of the live beams, whether any ray is clipped, and
+    // each unit's longest beam.  Cells only: the division of the set-up is left to the march.
     {
         const int very_neg = (int)0x80808080;
         int nx0 = very_neg, x1 = very_neg, ny0 = very_neg, y1 = very_neg;
         bool clipped = false;
-        Beam b;
-        if (valid) {
-            double fox, foy, fcx, fcy;
-            load_beam<MODE>(in, i, beams, fox, foy, fcx, fcy);
-            if (beam_setup(fox, foy, fcx, fcy, xw, yw, cells_per_m, off_x, off_y, b) == BEAM_OK) {
-                nx0 = -min(b.sx, b.hx);
-                x1 = max(b.sx, b.hx);
-                ny0 = -min(b.sy, b.hy);
-                y1 = max(b.sy, b.hy);
-                clipped = -nx0 < 0 || x1 >= xw || -ny0 < 0 || y1 >= yw;
+#pragma unroll
+        for (int k = 0; k < UNITS; ++k) {
+            const int u = warp + k * NWARPS;
+            long long i;
+            int span = -1;
+            if (v6_beam(u, s0, b0, scans, beams, i)) {
+                double fox, foy, fcx, fcy;
+                load_beam<MODE>(in, i, beams, fox, foy, fcx, fcy);
+                Beam b;
+                if (beam_cells(fox, foy, fcx, fcy, xw, yw, cells_per_m, off_x, off_y, b) == BEAM_OK) {
+                    nx0 = max(nx0, -min(b.sx, b.hx));
+                    x1 = max(x1, max(b.sx, b.hx));
+                    ny0 = max(ny0, -min(b.sy, b.hy));
+                    y1 = max(y1, max(b.sy, b.hy));
+                    clipped |= min(b.sx, b.hx) < 0 || max(b.sx, b.hx) >= xw || min(b.sy, b.hy) < 0 ||
+                               max(b.sy, b.hy) >= yw;
+                    span = b.span;
+                }
+            }
+            if (UNITS > 1) {
+                span = __reduce_max_sync(0xffffffffu, span);
+                if (lane == 0) unit_span[u] = span;
             }
         }
         nx0 = __reduce_max_sync(0xffffffffu, nx0);
@@ -655,47 +722,92 @@ grid_raycast_v6(int32_t *__restrict__ hit, int32_t *__restrict__ miss, int32_t *
     const bool empty = box[1] < 0;  // no live beam: nothing but status counts
     const int w = empty ? 0 : box[1] - bx + 1, h = empty ? 0 : box[3] - by + 1;
     const int pitch = h | 1;  // odd: the words of a y-major warp (one per row) spread over all banks
+    if (threadIdx.x == 0) V6_STAMP(2, clock64());
     if (box[4] || (long long)w * pitch > V6_TILE_WORDS) {
-        raycast_warp_v4<1, MODE, true>(hit, miss, scratch_t, ws, dirty, xw, yw, cells_per_m, off_x, off_y, in, i, valid,
-                                       beams, counters);
+        if (threadIdx.x == 0) V6_STAMP(6, 1);
+#pragma unroll 1
+        for (int k = 0; k < UNITS; ++k) {
+            long long i;
+            const bool valid = v6_beam(warp + k * NWARPS, s0, b0, scans, beams, i);
+            raycast_warp_v4<1, MODE, true>(hit, miss, scratch_t, ws, dirty, xw, yw, cells_per_m, off_x, off_y, in, i,
+                                           valid, beams, counters);
+        }
+#ifdef B2S_GRID_PHASES
+        __syncthreads();
+        if (threadIdx.x == 0) V6_STAMP(5, clock64());
+#endif
         return;
     }
 
     // ---- private path: the box lies inside the grid
-    for (int k = threadIdx.x; k < w * pitch; k += V6_THREADS) tile[k] = 0;
+    if (UNITS > 1 && warp == 0) {
+        const int mine = unit_span[lane];
+        int rank = 0;
+        for (int u = 0; u < V6_UNITS; ++u) {
+            const int o = unit_span[u];
+            rank += (o > mine) || (o == mine && u < lane);
+        }
+        order[rank] = lane;
+    }
+    for (int k = threadIdx.x; k < w * pitch; k += NWARPS * 32) tile[k] = 0;
     if (!empty) {
         const int tx0 = bx / GRID_TILE, ty0 = by / GRID_TILE, ny = box[3] / GRID_TILE - ty0 + 1;
         const int cnt = ((bx + w - 1) / GRID_TILE - tx0 + 1) * ny, tiles_y = grid_tiles(yw);
-        for (int k = threadIdx.x; k < cnt; k += V6_THREADS) dirty[(tx0 + k / ny) * tiles_y + ty0 + k % ny] = 1;
+        for (int k = threadIdx.x; k < cnt; k += NWARPS * 32) dirty[(tx0 + k / ny) * tiles_y + ty0 + k % ny] = 1;
     }
     __syncthreads();
-    if (valid) {
-        double fox, foy, fcx, fcy;
-        load_beam<MODE>(in, i, beams, fox, foy, fcx, fcy);
-        Beam b;
-        const int st = beam_setup(fox, foy, fcx, fcy, xw, yw, cells_per_m, off_x, off_y, b);
-        if (st == BEAM_OK) {
-            atomicAdd(hit + (b.hx * yw + b.hy), 1);  // the obstacle cell: last path element, inside the grid here
-            march_tile(b, smem_addr(tile), bx, by, pitch);
-        } else {
-            count_status(st, counters);
+    if (threadIdx.x == 0) V6_STAMP(3, clock64());
+#pragma unroll 1
+    for (int k = 0; k < UNITS; ++k) {
+        const int u = UNITS == 1 ? warp : order[k == 0 ? warp : V6_UNITS - 1 - warp];
+        long long i;
+        if (v6_beam(u, s0, b0, scans, beams, i)) {
+            double fox, foy, fcx, fcy;
+            load_beam<MODE>(in, i, beams, fox, foy, fcx, fcy);
+            Beam b;
+            const int st = beam_setup(fox, foy, fcx, fcy, xw, yw, cells_per_m, off_x, off_y, b);
+            if (st == BEAM_OK) {
+                atomicAdd(hit + (b.hx * yw + b.hy), 1);  // the obstacle cell: last path element, inside the grid here
+                march_tile(b, smem_addr(tile), bx, by, pitch);
+            } else {
+                count_status(st, counters);
+            }
         }
     }
+#ifdef B2S_GRID_PHASES
+    __syncwarp();
+    if (lane == 0) V6_STAMP(8 + warp, clock64());
+#endif
     __syncthreads();
+    if (threadIdx.x == 0) V6_STAMP(4, clock64());
 
-    // ---- flush: rows of the box, in 32-cell segments aligned in the plane; all-zero segments are skipped
-    const int warp = threadIdx.x >> 5, nwarps = V6_THREADS / 32;
+    // ---- flush: each warp takes whole rows of the box and adds them in 32-cell segments aligned in the plane, loading
+    // four segments before it issues their REDs; all-zero segments are skipped
     const int g0 = by >> 5, nseg = empty ? 0 : ((by + h - 1) >> 5) - g0 + 1;
-    for (int q = warp; q < w * nseg; q += nwarps) {
-        const int r = q / nseg, y = ((g0 + q % nseg) << 5) + lane;
-        const bool inside = y >= by && y < by + h;
-        const int v = inside ? (int)tile[r * pitch + (y - by)] : 0;
-        if (__any_sync(0xffffffffu, v != 0)) {
-            // every lane adds (0 outside the box); past the last column it adds to a cell of its own row
-            int32_t *p = miss + (size_t)(bx + r) * yw + min(y, yw - 1);
-            asm volatile("red.global.add.s32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
+    for (int r = warp; r < w; r += NWARPS) {
+        const uint32_t *row = tile + r * pitch;
+        int32_t *mrow = miss + (size_t)(bx + r) * yw;
+        for (int g = 0; g < nseg; g += 4) {
+            int v[4];
+#pragma unroll
+            for (int j = 0; j < 4; ++j) {
+                const int y = ((g0 + g + j) << 5) + lane;
+                v[j] = (g + j < nseg && y >= by && y < by + h) ? (int)row[y - by] : 0;
+            }
+#pragma unroll
+            for (int j = 0; j < 4; ++j) {
+                if (__any_sync(0xffffffffu, v[j] != 0)) {
+                    // every lane adds (0 outside the box); past the last column it adds to a cell of its own row
+                    const int y = ((g0 + g + j) << 5) + lane;
+                    asm volatile("red.global.add.s32 [%0], %1;" ::"l"(mrow + min(y, yw - 1)), "r"(v[j]) : "memory");
+                }
+            }
         }
     }
+#ifdef B2S_GRID_PHASES
+    __syncthreads();
+    if (threadIdx.x == 0) V6_STAMP(5, clock64());
+#endif
 }
 
 // miss[x][y] += scratch_t[y][x] over the recorded bounding box, scratch_t cleared on the way.
@@ -959,15 +1071,19 @@ static int raycast_v4_launch(int32_t *hit, int32_t *miss, int xw, int yw, double
                                                                                   in, total, beams, counters);       \
     } while (0)
     // variant 6 for a batch that is applied; taking one back out stays on the variant-5 march
-#define B2S_V6(FU)                                                                                                 \
+#define B2S_V6_LAUNCH(FU, UNITS)                                                                                   \
     do {                                                                                                           \
         const int tile_bytes = V6_TILE_WORDS * (int)sizeof(uint32_t);                                              \
-        B2S_CUDA(cudaFuncSetAttribute(grid_raycast_v6<FU>, cudaFuncAttributeMaxDynamicSharedMemorySize, tile_bytes)); \
+        B2S_CUDA(cudaFuncSetAttribute(grid_raycast_v6<FU, UNITS>, cudaFuncAttributeMaxDynamicSharedMemorySize,     \
+                                      tile_bytes));                                                                \
         const long long ctas = (long long)((scans + V6_SCANS - 1) / V6_SCANS) * ((beams + V6_SECTOR - 1) / V6_SECTOR); \
         B2S_REQUIRE(ctas < (1ll << 31), "b2s_grid_raycast_ws: too many beams for one launch");                  \
-        grid_raycast_v6<FU><<<(unsigned)ctas, V6_THREADS, tile_bytes, st>>>(hit, miss, scratch_t, ws, dirty, xw, yw,  \
-                                                                          cells_per_m, off_x, off_y, in, scans,     \
-                                                                          beams, counters);                         \
+        grid_raycast_v6<FU, UNITS><<<(unsigned)ctas, V6_UNITS * 32 / UNITS, tile_bytes, st>>>(                     \
+            hit, miss, scratch_t, ws, dirty, xw, yw, cells_per_m, off_x, off_y, in, scans, beams, counters);        \
+    } while (0)
+#define B2S_V6(FU)                                                                                                 \
+    do {                                                                                                           \
+        if (g_grid_tile_layout == 0) B2S_V6_LAUNCH(FU, 1); else B2S_V6_LAUNCH(FU, 2);                              \
     } while (0)
     if (sign >= 0 && g_grid_variant >= 6) {
         if (mode == IN_FUSED) B2S_V6(IN_FUSED); else if (mode == IN_F64) B2S_V6(IN_F64); else B2S_V6(IN_F32);
@@ -978,6 +1094,7 @@ static int raycast_v4_launch(int32_t *hit, int32_t *miss, int xw, int yw, double
     }
 #undef B2S_V4
 #undef B2S_V6
+#undef B2S_V6_LAUNCH
     B2S_CUDA(cudaGetLastError());
     if (!fold) return B2S_OK;
     long long ftiles = (long long)((xw + 31) / 32) * ((yw + 31) / 32);

@@ -37,6 +37,7 @@ int sm_count()
 }
 
 extern int g_grid_variant;
+extern int g_grid_tile_layout;
 extern int g_icp_src_per_thread;
 extern int g_icp_prune;
 extern int g_icp_block;
@@ -239,6 +240,11 @@ extern "C" int b2s_tune(const char *key, int value)
     if (strcmp(key, "grid_variant") == 0) {
         B2S_REQUIRE(value >= 1 && value <= 6, "b2s_tune: grid_variant must be 1..6");
         g_grid_variant = value;
+        return B2S_OK;
+    }
+    if (strcmp(key, "grid_tile_layout") == 0) {
+        B2S_REQUIRE(value == 0 || value == 1, "b2s_tune: grid_tile_layout must be 0 or 1");
+        g_grid_tile_layout = value;
         return B2S_OK;
     }
     if (strcmp(key, "h2d_chunks") == 0) {

@@ -54,7 +54,8 @@ int b2s_device_count(int *count);
 /* Kernel-variant switch for benchmarking.  Keys: "grid_variant" 1 = one RED per visit, 2 = warp-aggregated
  * runs, 3 = lean loop, 4 = transposed scratch plane, 5 = 4 + test-free core phase, 6 = consecutive scans counted
  * in a shared-memory tile, 5 where the tile does not fit (default; 4..6 need a workspace, else 3; a roll-back runs 5);
- * "icp_prune"
+ * "grid_tile_layout" (variant 6) 0 = 1024 threads, one 32-beam unit per warp, 1 = 512 threads, two units per warp,
+ * longest paired with shortest (default); "icp_prune"
  * 0 = brute force, 1 = per-lane block pruning, 2 = warp-level + per-lane with whole-warp block visits,
  * 3 = warp-level only, 4 = both tests, surviving (point, block) pairs queued and spread over the lanes
  * (default); "icp_block" 0 (automatic) / 8 / 16 / 32 targets per pruning block; "icp_layout" 0 strided /

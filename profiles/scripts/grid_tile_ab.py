@@ -1,9 +1,11 @@
-"""A/B of the ray-cast variants 5 and 6 at the bench launch (cfg 3: seed 12001, 16 384 scans x 1080 beams, 4096^2 @ 5 cm).
+"""A/B of ray-cast variant 5 and the two tile layouts of variant 6 at the bench launch (cfg 3: seed 12001, 16 384 scans x 1080 beams, 4096^2 @ 5 cm).
    python profiles/scripts/grid_tile_ab.py [launches per variant, default 30] [scans, default 16384]
-Alternates the two variants launch by launch in one process, on zeroed planes with L2 flushed before every launch, and
-prints one JSON line: median / min / max ms per launch (CUDA events around ray-cast + fold), the share of variant-6
-CTAs that fall back to the variant-5 march (the kernel's rule, evaluated on the host), registers / shared memory /
-resident CTAs of the kernels (cuobjdump of the built library), and whether the planes are equal byte for byte."""
+Alternates variant 5, variant 6 with grid_tile_layout 0 (1024 threads, one unit per warp) and variant 6 with layout 1
+(512 threads, two units per warp) launch by launch in one process, on zeroed planes with L2 flushed before every
+launch, and prints one JSON line: median / min / max ms per launch (CUDA events around ray-cast + fold), the share of
+variant-6 CTAs that fall back to the variant-5 march (the kernel's rule, evaluated on the host), registers / shared
+memory / resident CTAs of the kernels (cuobjdump of the built library), and whether the planes of all three are equal
+byte for byte."""
 import json
 import os
 import re
@@ -60,9 +62,11 @@ def resources():
             if "grid_raycast_v4ILi1ELi0ELb1E" in fn:
                 res["v5"] = {"regs": int(m.group(1)), "stack": int(m.group(2)), "smem_static": int(m.group(3)),
                              "threads": 256, "smem_dynamic": 0}
-            elif "grid_raycast_v6ILi0E" in fn:
-                res["v6"] = {"regs": int(m.group(1)), "stack": int(m.group(2)), "smem_static": int(m.group(3)),
-                             "threads": 1024, "smem_dynamic": V6_TILE_WORDS * 4}
+            elif "grid_raycast_v6ILi0ELi1E" in fn or "grid_raycast_v6ILi0ELi2E" in fn:
+                units = 1 if "ILi0ELi1E" in fn else 2
+                res["v6_layout%d" % (units - 1)] = {"regs": int(m.group(1)), "stack": int(m.group(2)),
+                                                    "smem_static": int(m.group(3)), "threads": 1024 // units,
+                                                    "smem_dynamic": V6_TILE_WORDS * 4}
     # B200 per SM: 64 K registers, 2048 threads, 228 KB shared memory, 32 CTAs (SHARED includes the 1 KB per CTA
     # that the system reserves)
     for r in res.values():
@@ -80,13 +84,15 @@ def main():
     S, Hx, Hy = devapi.grid_scale(G, G, 0.05)
     host = synth.grid_scans(12001, K, N)
     ox, oy, cx, cy = (torch.from_numpy(a).cuda() for a in host)
-    planes = {v: devapi.new_planes(G, G) for v in (5, 6)}
+    arms = {"v5": (5, 1), "v6_layout0": (6, 0), "v6_layout1": (6, 1)}  # grid_variant, grid_tile_layout
+    planes = {a: devapi.new_planes(G, G) for a in arms}
     ws = devapi.new_workspace(G, G)
     flush = torch.empty(256 * 1024 * 1024, dtype=torch.uint8, device="cuda")
-    ms = {5: [], 6: []}
+    ms = {a: [] for a in arms}
     for it in range(3 + launches):
-        for v in (5, 6):
-            _lib.check(_lib.lib().b2s_tune(b"grid_variant", v))
+        for v, (variant, layout) in arms.items():
+            _lib.check(_lib.lib().b2s_tune(b"grid_variant", variant))
+            _lib.check(_lib.lib().b2s_tune(b"grid_tile_layout", layout))
             hit, miss = planes[v]
             hit.zero_(); miss.zero_(); flush.zero_()
             a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -96,7 +102,8 @@ def main():
             torch.cuda.synchronize()
             if it >= 3:
                 ms[v].append(a.elapsed_time(b))
-    (h5, m5), (h6, m6) = planes[5], planes[6]
+    _lib.check(_lib.lib().b2s_tune(b"grid_tile_layout", 1))
+    (h5, m5), (h0, m0), (h6, m6) = planes["v5"], planes["v6_layout0"], planes["v6_layout1"]
     visits = int(h6.sum(dtype=torch.int64).item() + m6.sum(dtype=torch.int64).item())
     card = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader"],
                           capture_output=True, text=True).stdout.strip().splitlines()
@@ -105,11 +112,13 @@ def main():
     print(json.dumps({
         "workload": "cfg3 bench launch: %d scans x %d beams into %d^2 @ 0.05 m, L2 flushed before every launch" % (K, N, G),
         "device": card[0] if card else None,
-        "v5": stat(ms[5]), "v6": stat(ms[6]),
-        "speedup_median": float(np.median(ms[5]) / np.median(ms[6])),
+        **{a: stat(x) for a, x in ms.items()},
+        "layout1_over_layout0_median": float(np.median(ms["v6_layout1"]) / np.median(ms["v6_layout0"])),
+        "v5_over_layout1_median": float(np.median(ms["v5"]) / np.median(ms["v6_layout1"])),
         "v6_fallback_cta_share": fallback_share(host, G, S, Hx),
         "resources": resources(),
-        "planes_byte_identical": bool(torch.equal(h5, h6) and torch.equal(m5, m6)),
+        "planes_byte_identical": bool(torch.equal(h5, h6) and torch.equal(m5, m6) and torch.equal(h0, h6) and
+                                      torch.equal(m0, m6)),
         "visits": visits}))
 
 
