@@ -47,6 +47,16 @@ constexpr int MAX_CHUNKS = 16;
 int g_tune_gen = 0;    // bumped by every b2s_tune: cached single-pair graphs captured under other settings are stale
 int g_h2d_chunks = 0;  // 0: automatic; 1..MAX_CHUNKS force the pipeline depth of the host-buffer calls (tuning hook)
 
+// Pipeline depth of a host-buffer call: the call's own measured choice `want`, at most `cap`, unless h2d_chunks forces
+// one; never more chunks than there are units (pairs, scans) to cut, never fewer than one.
+static int pipeline_chunks(int want, int cap, int units)
+{
+    int n = want < cap ? want : cap;
+    if (g_h2d_chunks > 0) n = g_h2d_chunks;
+    if (n > units) n = units;
+    return n < 1 ? 1 : n;
+}
+
 ScratchPool *scratch_pool()
 {
     static thread_local ScratchPool *pool = nullptr;
@@ -174,6 +184,82 @@ struct b2s_icp {
     int submitted;
 };
 
+namespace {
+// One host batch in either input form.
+struct HostBatch {
+    bool fused;
+    bool f64;                        // endpoints form: float64 (the reference's dtype) instead of float32
+    const void *ox, *oy, *cx, *cy;   // endpoints form
+    const float *ranges;             // fused form
+    const double *pose4, *beam_cs;   // pose4 [scans][4] = x, y, cos yaw, sin yaw ...
+    double clamp;
+    const double *poses3;            // ... or poses3 [scans][3] = x, y, yaw: the table is built here, chunk by chunk
+};
+
+// The same batch in one device buffer: ox | oy | cx | cy, or ranges | pose table [scans][4] | beam table [beams][2],
+// each region 16-byte aligned.  A streamed step keeps its DeviceBatch until its wait, so a rejected step is taken
+// back out of exactly the bytes it was ray-cast from.
+struct DeviceBatch {
+    bool fused = false, f64 = false;
+    int scans = 0, beams = 0;
+    double clamp = 0.0;
+    char *pts = nullptr, *oy = nullptr, *cx = nullptr, *cy = nullptr;  // pts: ox, or the ranges
+    double *pose = nullptr, *cs = nullptr;
+
+    DeviceBatch() = default;
+    DeviceBatch(const HostBatch &hb, int scans, int beams)
+        : fused(hb.fused), f64(!hb.fused && hb.f64), scans(scans), beams(beams), clamp(hb.clamp) {}
+    size_t el() const { return f64 ? sizeof(double) : sizeof(float); }  // bytes per input coordinate
+    size_t a_pts() const { return ((size_t)scans * beams * el() + 15) & ~(size_t)15; }
+    size_t a_ctr() const { return ((size_t)scans * el() + 15) & ~(size_t)15; }
+    size_t bytes() const
+    {
+        return fused ? a_pts() + (size_t)scans * 4 * sizeof(double) + (size_t)beams * 2 * sizeof(double)
+                     : 2 * a_pts() + 2 * a_ctr();
+    }
+    void bind(void *base)
+    {
+        pts = (char *)base;
+        oy = pts + a_pts();
+        cx = oy + a_pts();
+        cy = cx + a_ctr();
+        pose = (double *)oy;
+        cs = pose + (size_t)scans * 4;
+    }
+    // Copies scans [s0, s1) of hb on stream st; the first chunk also brings the beam table.  With hb.poses3 the rows
+    // [s0, s1) of the pinned pose_table are computed first: the host runs ahead of the device, so the table of chunk
+    // k + 1 (u2T's math.cos / math.sin, [SLAM]:130-137: the same libm calls) is made while chunk k crosses PCIe.
+    int upload(const HostBatch &hb, size_t s0, size_t s1, double *pose_table, cudaStream_t st) const
+    {
+        const size_t ns = s1 - s0;
+        if (!fused) {
+            const size_t e = el();
+            B2S_CUDA(cudaMemcpyAsync(pts + s0 * beams * e, (const char *)hb.ox + s0 * beams * e, ns * beams * e, cudaMemcpyHostToDevice, st));
+            B2S_CUDA(cudaMemcpyAsync(oy + s0 * beams * e, (const char *)hb.oy + s0 * beams * e, ns * beams * e, cudaMemcpyHostToDevice, st));
+            B2S_CUDA(cudaMemcpyAsync(cx + s0 * e, (const char *)hb.cx + s0 * e, ns * e, cudaMemcpyHostToDevice, st));
+            B2S_CUDA(cudaMemcpyAsync(cy + s0 * e, (const char *)hb.cy + s0 * e, ns * e, cudaMemcpyHostToDevice, st));
+            return B2S_OK;
+        }
+        if (s0 == 0) B2S_CUDA(cudaMemcpyAsync(cs, hb.beam_cs, (size_t)beams * 2 * sizeof(double), cudaMemcpyHostToDevice, st));
+        const double *pose4 = hb.pose4;
+        if (hb.poses3) {
+            for (size_t s = s0; s < s1; ++s) {
+                pose_table[4 * s] = hb.poses3[3 * s];
+                pose_table[4 * s + 1] = hb.poses3[3 * s + 1];
+                pose_table[4 * s + 2] = cos(hb.poses3[3 * s + 2]);
+                pose_table[4 * s + 3] = sin(hb.poses3[3 * s + 2]);
+            }
+            pose4 = pose_table;
+        }
+        B2S_CUDA(cudaMemcpyAsync((float *)pts + s0 * beams, hb.ranges + s0 * beams, ns * beams * sizeof(float), cudaMemcpyHostToDevice, st));
+        B2S_CUDA(cudaMemcpyAsync(pose + 4 * s0, pose4 + 4 * s0, ns * 4 * sizeof(double), cudaMemcpyHostToDevice, st));
+        return B2S_OK;
+    }
+    // Ray-casts scans [s0, s1) into m's counts with the given sign; fold: the last launch of the batch
+    int raycast(const b2s_mapping *m, size_t s0, size_t s1, int sign, int32_t *counters, cudaStream_t st, bool fold) const;
+};
+}  // namespace
+
 struct b2s_mapping {
     int device;
     int xw, yw;
@@ -181,30 +267,42 @@ struct b2s_mapping {
     double w_hit, w_miss, thresh;
     // stream: everything ordered (zeroing, last chunk + fold, finalize, read-back); stream2: every other ray-cast
     // chunk, so the ragged end of one chunk (beams differ in length) overlaps the next; copy_stream: H2D
-    cudaStream_t stream, stream2, copy_stream;
-    cudaEvent_t chunk_ready[MAX_CHUNKS], begun, joined;
-    int32_t *hit, *miss;
-    int32_t *counters;
-    void *workspace;
+    cudaStream_t stream = nullptr, stream2 = nullptr, copy_stream = nullptr;
+    cudaEvent_t chunk_ready[MAX_CHUNKS] = {}, begun = nullptr, joined = nullptr;
+    int32_t *hit = nullptr, *miss = nullptr;
+    int32_t *counters = nullptr;
+    void *workspace = nullptr;
     Buf d_in, d_datamap, d_pmap, d_packed;
-    Buf h_pose;  // pinned [scans][4] pose table of the call in flight (b2s_mapping_update_scans)
-    bool pmap_valid;  // d_pmap holds the occupancy of the current counts
-    int8_t *h_packed;  // pinned staging for the dirty tiles
-    int32_t *h_ids;
+    Buf h_pose = {nullptr, 0, true};  // pinned [scans][4] pose table of the call in flight (b2s_mapping_update_scans)
+    bool pmap_valid = false;  // d_pmap holds the occupancy of the current counts
+    int8_t *h_packed = nullptr;  // pinned staging for the dirty tiles
+    int32_t *h_ids = nullptr;
     // Streaming calls (b2s_mapping_submit* / b2s_mapping_wait): two slots of everything a step owns, so that step
     // k + 1 can be uploaded and ray-cast while the map of step k is still on its way back to the host.
     struct Slot {
-        Buf d_in, d_map, h_pose;          // device inputs, device copy of this step's occupancy, pinned pose table
-        int32_t *d_cnt, *h_cnt;           // the ray-cast's B2S_CNT_* words of this step (device / pinned host)
-        cudaEvent_t inputs_free, done;    // last ray-cast of the step enqueued / results on the host
-        bool in_flight, fused;
-        int ticket, scans, beams;
-        double clamp;
+        Buf d_in, d_map, h_pose = {nullptr, 0, true};  // device inputs, device copy of this step's occupancy, pinned pose table
+        int32_t *d_cnt = nullptr, *h_cnt = nullptr;     // the ray-cast's B2S_CNT_* words of this step (device / pinned host)
+        cudaEvent_t inputs_free = nullptr, done = nullptr;  // last ray-cast of the step enqueued / results on the host
+        bool in_flight = false;
+        int ticket = 0;
+        DeviceBatch batch;                              // the step's inputs in d_in
     } slot[2];
-    cudaStream_t d2h_stream;
-    cudaEvent_t finalized;
-    int submitted;
+    cudaStream_t d2h_stream = nullptr;
+    cudaEvent_t finalized = nullptr;
+    int submitted = 0;
 };
+
+int DeviceBatch::raycast(const b2s_mapping *m, size_t s0, size_t s1, int sign, int32_t *counters, cudaStream_t st,
+                         bool fold) const
+{
+    if (fused)
+        return grid_raycast_ranges_signed(m->hit, m->miss, m->xw, m->yw, m->cells_per_m, m->off_x, m->off_y,
+                                          (const float *)pts + s0 * beams, pose + 4 * s0, cs, clamp, (int)(s1 - s0), beams,
+                                          counters, m->workspace, sign, st, fold);
+    return grid_raycast_signed(m->hit, m->miss, m->xw, m->yw, m->cells_per_m, m->off_x, m->off_y, pts + s0 * beams * el(),
+                               oy + s0 * beams * el(), cx + s0 * el(), cy + s0 * el(), f64, (int)(s1 - s0), beams, counters,
+                               m->workspace, sign, st, fold);
+}
 
 extern "C" int b2s_version(void) { return 100; }
 
@@ -463,11 +561,7 @@ extern "C" int b2s_icp_process(b2s_icp *c, const void *tar_xy, const void *src_x
     if ((rc = c->d_T.reserve((size_t)pairs * 9 * sizeof(double)))) return rc;
     if ((rc = c->d_iters.reserve((size_t)pairs * sizeof(int32_t)))) return rc;
     // Pipeline: up to 8 chunks of pairs; chunk k+1 crosses PCIe on the copy stream while chunk k is solved.
-    int nchunk = (int)((tb + sb + (16u << 20) - 1) / (16u << 20));  // ~16 MB of points per chunk (measured best)
-    if (nchunk > 8) nchunk = 8;
-    if (g_h2d_chunks > 0) nchunk = g_h2d_chunks;
-    if (nchunk > pairs) nchunk = pairs;
-    if (nchunk < 1) nchunk = 1;
+    const int nchunk = pipeline_chunks((int)((tb + sb + (16u << 20) - 1) / (16u << 20)), 8, pairs);  // ~16 MB of points per chunk (measured best)
     const size_t tpair = (size_t)2 * n_tar * el, spair = (size_t)2 * n_src * el;
     // (every call ends with a synchronize, so the device input buffers are free to overwrite here)
     for (int k = 0; k < nchunk; ++k) {
@@ -531,13 +625,10 @@ static int icp_sequence_enqueue(b2s_icp *c, Trace &tr, const void *scans_xy, int
         if ((rc = bufs.cs.reserve((size_t)n * 2 * sizeof(double)))) return rc;
         B2S_CUDA(cudaMemcpyAsync(bufs.cs.p, beam_cs, (size_t)n * 2 * sizeof(double), cudaMemcpyHostToDevice, c->copy_stream));
     }
-    int nchunk = (int)(((size_t)scans * scan_bytes + (8u << 20) - 1) / (8u << 20));  // ~8 MB of points per chunk
-    if (beam_cs && nchunk < 4 && pairs >= 4096) nchunk = 4;  // (raw scans are half the bytes: keep the pipeline depth)
-    if (nchunk > 8) nchunk = 8;
-    if (force_chunks > 0) nchunk = force_chunks;
-    if (g_h2d_chunks > 0) nchunk = g_h2d_chunks;
-    if (nchunk > pairs) nchunk = pairs;
-    if (nchunk < 1) nchunk = 1;
+    int want = (int)(((size_t)scans * scan_bytes + (8u << 20) - 1) / (8u << 20));  // ~8 MB of points per chunk
+    if (beam_cs && want < 4 && pairs >= 4096) want = 4;  // (raw scans are half the bytes: keep the pipeline depth)
+    if (force_chunks > 0) want = force_chunks;
+    const int nchunk = pipeline_chunks(want, 8, pairs);
     // chunk k solves pairs [p0, p1) and therefore needs scans [p0, p1]; scan p0 arrived with the previous chunk
     for (int k = 0; k < nchunk; ++k) {
         const size_t p0 = (size_t)pairs * k / nchunk, p1 = (size_t)pairs * (k + 1) / nchunk;
@@ -797,21 +888,6 @@ extern "C" int b2s_mapping_create(b2s_mapping **out, int xw, int yw, double xyre
     m->w_hit = w_hit;
     m->w_miss = w_miss;
     m->thresh = thresh;
-    m->hit = m->miss = m->counters = nullptr;
-    m->workspace = nullptr;
-    m->pmap_valid = false;
-    m->h_packed = nullptr;
-    m->h_ids = nullptr;
-    m->stream = m->stream2 = m->copy_stream = m->d2h_stream = nullptr;
-    for (int k = 0; k < MAX_CHUNKS; ++k) m->chunk_ready[k] = nullptr;
-    m->begun = m->joined = m->finalized = nullptr;
-    m->submitted = 0;
-    for (int k = 0; k < 2; ++k) {
-        m->slot[k].d_cnt = m->slot[k].h_cnt = nullptr;
-        m->slot[k].inputs_free = m->slot[k].done = nullptr;
-        m->slot[k].in_flight = false;
-        m->slot[k].h_pose.pinned = true;
-    }
     const size_t plane = (size_t)xw * yw * sizeof(int32_t);
     cudaError_t e = cudaStreamCreateWithFlags(&m->stream, cudaStreamNonBlocking);
     if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&m->stream2, cudaStreamNonBlocking);
@@ -895,16 +971,24 @@ extern "C" int b2s_mapping_reset(b2s_mapping *m)
 }
 
 namespace {
-// One host batch in either input form.
-struct HostBatch {
-    bool fused;
-    bool f64;                        // endpoints form: float64 (the reference's dtype) instead of float32
-    const void *ox, *oy, *cx, *cy;   // endpoints form
-    const float *ranges;             // fused form
-    const double *pose4, *beam_cs;   // pose4 [scans][4] = x, y, cos yaw, sin yaw ...
-    double clamp;
-    const double *poses3;            // ... or poses3 [scans][3] = x, y, yaw: the table is built here, chunk by chunk
-};
+// The verdict on a batch from its ray-cast's B2S_CNT_* words: a coordinate the reference's int() raises on, or a beam
+// too long to march, rejects the whole batch.
+bool batch_rejected(const int32_t *cnt)
+{
+    return cnt[B2S_CNT_NONFINITE] || cnt[B2S_CNT_OVERFLOW] || cnt[B2S_CNT_TOO_LONG] > 0;
+}
+
+// Status and message of a rejected batch.  The reference raises at the first offending beam in scan order; NaN and
+// inf map to different exception classes, NaN wins when both occur (documented deviation).
+int batch_error(const int32_t *cnt)
+{
+    if (cnt[B2S_CNT_NONFINITE] || cnt[B2S_CNT_OVERFLOW]) {
+        set_error(cnt[B2S_CNT_NONFINITE] ? "cannot convert float NaN to integer" : "cannot convert float infinity to integer");
+        return B2S_ERR_NONFINITE;
+    }
+    set_error("%d beam(s) longer than %d cells: batch rejected", cnt[B2S_CNT_TOO_LONG], B2S_MAX_PATH_CELLS);
+    return B2S_ERR_TOO_LONG;
+}
 
 // Mapping.update for a batch, all-or-nothing like a Python exception raised before the loop.
 //   * the batch is cut into up to 16 chunks of scans; chunk k+1 crosses PCIe on the copy stream while
@@ -924,89 +1008,27 @@ int mapping_update_impl(b2s_mapping *m, const HostBatch &hb, int scans, int beam
     Trace tr(m->stream);
     const size_t total = (size_t)scans * beams;
     int rc;
-    int nchunk = 0;
-    int lo[MAX_CHUNKS + 1] = {0};
-    char *d_a = nullptr, *d_b = nullptr, *d_c = nullptr, *d_d = nullptr;  // ox|oy|cx|cy  or  ranges
-    const size_t el = (!hb.fused && hb.f64) ? sizeof(double) : sizeof(float);  // bytes per input coordinate
-    double *d_pose = nullptr, *d_cs = nullptr;
-    // (the transposed scratch plane of the ray-cast is folded back once, with the last chunk)
-    auto launch = [&](int k, int sign, int32_t *counters, cudaStream_t ks) -> int {
-        const size_t s0 = (size_t)lo[k];
-        const int ns = lo[k + 1] - lo[k];
-        const bool fold = (k == nchunk - 1);
-        if (hb.fused)
-            return grid_raycast_ranges_signed(m->hit, m->miss, m->xw, m->yw, m->cells_per_m, m->off_x, m->off_y,
-                                              (const float *)d_a + s0 * beams, d_pose + 4 * s0, d_cs, hb.clamp, ns, beams,
-                                              counters, m->workspace, sign, ks, fold);
-        return grid_raycast_signed(m->hit, m->miss, m->xw, m->yw, m->cells_per_m, m->off_x, m->off_y,
-                                   d_a + s0 * beams * el, d_b + s0 * beams * el, d_c + s0 * el, d_d + s0 * el, hb.f64, ns,
-                                   beams, counters, m->workspace, sign, ks, fold);
-    };
+    DeviceBatch db(hb, scans, beams);
     if (total > 0) {
-        const size_t pts = total * el, a_pts = (pts + 15) & ~(size_t)15;
-        char *base;
-        if (hb.fused) {
-            const size_t poses = (size_t)scans * 4 * sizeof(double), table = (size_t)beams * 2 * sizeof(double);
-            if ((rc = m->d_in.reserve(a_pts + poses + table))) return rc;
-            base = (char *)m->d_in.p;
-            d_a = base;
-            d_pose = (double *)(base + a_pts);
-            d_cs = (double *)(base + a_pts + poses);
-            B2S_CUDA(cudaMemcpyAsync(d_cs, hb.beam_cs, table, cudaMemcpyHostToDevice, m->copy_stream));
-        } else {
-            const size_t ctr = (size_t)scans * el, a_ctr = (ctr + 15) & ~(size_t)15;
-            if ((rc = m->d_in.reserve(2 * a_pts + 2 * a_ctr))) return rc;
-            base = (char *)m->d_in.p;
-            d_a = base;
-            d_b = base + a_pts;
-            d_c = base + 2 * a_pts;
-            d_d = base + 2 * a_pts + a_ctr;
-        }
+        if ((rc = m->d_in.reserve(db.bytes()))) return rc;
+        db.bind(m->d_in.p);
         // counters[0..3]: the ray-cast kernel's own (B2S_CNT_*); counters[4]: dirty-tile count of this call
         B2S_CUDA(cudaMemsetAsync(m->counters, 0, 2 * B2S_CNT_WORDS * sizeof(int32_t), m->stream));
         // the dirty-tile map describes THIS call
         B2S_CUDA(cudaMemsetAsync((char *)m->workspace + GRID_WS_HEADER, 0, grid_dirty_bytes(m->xw, m->yw), m->stream));
         // ~1M beams per chunk: with consecutive chunks overlapping on two compute streams an extra launch costs
         // little, and the first ray-cast starts after 1/16 of the copy (measured: profiles/scripts/chunk_sweep.py)
-        nchunk = (int)((total * (el / sizeof(float)) + (1u << 20) - 1) >> 20);
-        if (nchunk > MAX_CHUNKS) nchunk = MAX_CHUNKS;
-        if (g_h2d_chunks > 0) nchunk = g_h2d_chunks;
-        if (nchunk > scans) nchunk = scans;
-        if (nchunk < 1) nchunk = 1;
-        for (int k = 0; k <= nchunk; ++k) lo[k] = (int)((long long)scans * k / nchunk);
+        const int nchunk = pipeline_chunks((int)((total * (db.el() / sizeof(float)) + (1u << 20) - 1) >> 20), MAX_CHUNKS, scans);
         if (nchunk > 1) {  // the second compute stream starts after the resets above (single-chunk calls never use it)
             B2S_CUDA(cudaEventRecord(m->begun, m->stream));
             B2S_CUDA(cudaStreamWaitEvent(m->stream2, m->begun, 0));
         }
-        const double *pose4 = hb.pose4;
-        double *table = nullptr;
-        if (hb.fused && hb.poses3) {
-            m->h_pose.pinned = true;
-            if ((rc = m->h_pose.reserve((size_t)scans * 4 * sizeof(double)))) return rc;
-            pose4 = table = (double *)m->h_pose.p;
-        }
-        // per chunk: [pose table] -> copies on the copy stream -> ray-cast on the compute stream once they landed.
-        // The host runs ahead of the device, so the table of chunk k+1 (u2T's math.cos / math.sin, [SLAM]:130-137:
-        // the same libm calls) is computed while chunk k crosses PCIe and is ray-cast.
+        if (hb.fused && hb.poses3 && (rc = m->h_pose.reserve((size_t)scans * 4 * sizeof(double)))) return rc;
+        // per chunk: copies on the copy stream -> ray-cast on a compute stream once they landed
         for (int k = 0; k < nchunk; ++k) {
-            const size_t s0 = (size_t)lo[k], ns = (size_t)(lo[k + 1] - lo[k]);
+            const size_t s0 = (size_t)scans * k / nchunk, s1 = (size_t)scans * (k + 1) / nchunk;
             cudaStream_t cs = m->copy_stream;
-            if (hb.fused) {
-                if (table)
-                    for (size_t s = s0; s < s0 + ns; ++s) {
-                        table[4 * s] = hb.poses3[3 * s];
-                        table[4 * s + 1] = hb.poses3[3 * s + 1];
-                        table[4 * s + 2] = cos(hb.poses3[3 * s + 2]);
-                        table[4 * s + 3] = sin(hb.poses3[3 * s + 2]);
-                    }
-                B2S_CUDA(cudaMemcpyAsync(d_a + s0 * beams * sizeof(float), hb.ranges + s0 * beams, ns * beams * sizeof(float), cudaMemcpyHostToDevice, cs));
-                B2S_CUDA(cudaMemcpyAsync(d_pose + 4 * s0, pose4 + 4 * s0, ns * 4 * sizeof(double), cudaMemcpyHostToDevice, cs));
-            } else {
-                B2S_CUDA(cudaMemcpyAsync(d_a + s0 * beams * el, (const char *)hb.ox + s0 * beams * el, ns * beams * el, cudaMemcpyHostToDevice, cs));
-                B2S_CUDA(cudaMemcpyAsync(d_b + s0 * beams * el, (const char *)hb.oy + s0 * beams * el, ns * beams * el, cudaMemcpyHostToDevice, cs));
-                B2S_CUDA(cudaMemcpyAsync(d_c + s0 * el, (const char *)hb.cx + s0 * el, ns * el, cudaMemcpyHostToDevice, cs));
-                B2S_CUDA(cudaMemcpyAsync(d_d + s0 * el, (const char *)hb.cy + s0 * el, ns * el, cudaMemcpyHostToDevice, cs));
-            }
+            if ((rc = db.upload(hb, s0, s1, (double *)m->h_pose.p, cs))) return rc;
             B2S_CUDA(cudaEventRecord(m->chunk_ready[k], cs));
             tr.mark("h2d chunk done", k, cs);
             // odd chunks run on the second compute stream; the last chunk (which also folds the scratch plane)
@@ -1018,7 +1040,7 @@ int mapping_update_impl(b2s_mapping *m, const HostBatch &hb, int scans, int beam
                 B2S_CUDA(cudaStreamWaitEvent(m->stream, m->joined, 0));
             }
             B2S_CUDA(cudaStreamWaitEvent(ks, m->chunk_ready[k], 0));
-            if ((rc = launch(k, +1, m->counters, ks))) return rc;
+            if ((rc = db.raycast(m, s0, s1, +1, m->counters, ks, last))) return rc;
             tr.mark("ray-cast chunk done", k, ks);
         }
     }
@@ -1045,7 +1067,7 @@ int mapping_update_impl(b2s_mapping *m, const HostBatch &hb, int scans, int beam
         B2S_CUDA(cudaStreamSynchronize(m->stream));
         have_cnt = true;
         const int nd = cnt[B2S_CNT_WORDS];
-        const bool bad = cnt[B2S_CNT_NONFINITE] || cnt[B2S_CNT_OVERFLOW] || cnt[B2S_CNT_TOO_LONG] > 0;
+        const bool bad = batch_rejected(cnt);
         if (!bad && nd <= PACK_CAP) {
             if (nd > 0) {
                 B2S_CUDA(cudaMemcpyAsync(m->h_packed, d_packed, (size_t)nd * tile_bytes, cudaMemcpyDeviceToHost, m->stream));
@@ -1086,10 +1108,9 @@ int mapping_update_impl(b2s_mapping *m, const HostBatch &hb, int scans, int beam
     tr.mark("all enqueued", 0, nullptr);
     B2S_CUDA(cudaStreamSynchronize(m->stream));
     tr.mark("synchronized", 0, nullptr);
-    const int saw_nan = cnt[B2S_CNT_NONFINITE], saw_inf = cnt[B2S_CNT_OVERFLOW];
-    if (saw_nan || saw_inf || cnt[B2S_CNT_TOO_LONG] > 0) {
-        for (int k = 0; k < nchunk; ++k)
-            if ((rc = launch(k, -1, nullptr, m->stream))) return rc;
+    if (batch_rejected(cnt)) {
+        // every chunk is still in m->d_in: one launch over the whole batch takes it back out
+        if ((rc = db.raycast(m, 0, scans, -1, nullptr, m->stream, true))) return rc;
         if (pmap_out) {
             rc = b2s_grid_finalize(m->hit, m->miss, m->xw, m->yw, m->w_hit, m->w_miss, m->thresh, nullptr,
                                    (int8_t *)m->d_pmap.p, m->stream);
@@ -1097,14 +1118,7 @@ int mapping_update_impl(b2s_mapping *m, const HostBatch &hb, int scans, int beam
             B2S_CUDA(cudaMemcpyAsync(pmap_out, m->d_pmap.p, cells, cudaMemcpyDeviceToHost, m->stream));
         }
         B2S_CUDA(cudaStreamSynchronize(m->stream));
-        if (saw_nan || saw_inf) {
-            // the reference raises at the first offending beam in scan order; NaN and inf map to
-            // different exception classes, NaN wins when both occur (documented deviation)
-            set_error(saw_nan ? "cannot convert float NaN to integer" : "cannot convert float infinity to integer");
-            return B2S_ERR_NONFINITE;
-        }
-        set_error("%d beam(s) longer than %d cells: batch rejected", cnt[B2S_CNT_TOO_LONG], B2S_MAX_PATH_CELLS);
-        return B2S_ERR_TOO_LONG;
+        return batch_error(cnt);
     }
     return B2S_OK;
 }
@@ -1181,40 +1195,20 @@ extern "C" int b2s_mapping_update_scans(b2s_mapping *m, const float *ranges, con
 // pair keeps two steps in flight instead: submit enqueues a whole step (its own device input buffers, counters and
 // device copy of the occupancy) and returns; the upload of step k + 1 then overlaps the ray-cast of step k and the
 // read-back of step k - ... on a third stream.  wait(ticket) blocks until that step's map is in pmap_out and gives the
-// step's verdict; a batch the reference would raise on is taken back out of the counts there (sign -1 kernels on the
-// slot's still-resident inputs: exact), but maps of steps submitted in between were finalized with it still applied.
+// step's verdict; a batch the reference would raise on is taken back out of the counts there (one sign -1 ray-cast of
+// the slot's still-resident inputs: exact), but maps of steps submitted in between were finalized with it still applied.
 namespace {
 int mapping_wait_slot(b2s_mapping *m, b2s_mapping::Slot &sl)
 {
     if (!sl.in_flight) return B2S_OK;
     B2S_CUDA(cudaEventSynchronize(sl.done));
     sl.in_flight = false;
-    const int32_t *cnt = sl.h_cnt;
-    const int saw_nan = cnt[B2S_CNT_NONFINITE], saw_inf = cnt[B2S_CNT_OVERFLOW], too_long = cnt[B2S_CNT_TOO_LONG];
-    if (!(saw_nan || saw_inf || too_long > 0)) return B2S_OK;
+    if (!batch_rejected(sl.h_cnt)) return B2S_OK;
     // roll the step back: the inputs are still in the slot's device buffers (the slot is not reused before its wait)
-    const size_t total = (size_t)sl.scans * sl.beams, a_pts = (total * sizeof(float) + 15) & ~(size_t)15;
-    char *base = (char *)sl.d_in.p;
-    int rc;
-    if (sl.fused) {
-        const size_t poses = (size_t)sl.scans * 4 * sizeof(double);
-        rc = grid_raycast_ranges_signed(m->hit, m->miss, m->xw, m->yw, m->cells_per_m, m->off_x, m->off_y, (const float *)base,
-                                        (const double *)(base + a_pts), (const double *)(base + a_pts + poses), sl.clamp,
-                                        sl.scans, sl.beams, nullptr, m->workspace, -1, m->stream, true);
-    } else {
-        const size_t a_ctr = ((size_t)sl.scans * sizeof(float) + 15) & ~(size_t)15;
-        rc = grid_raycast_signed(m->hit, m->miss, m->xw, m->yw, m->cells_per_m, m->off_x, m->off_y, base, base + a_pts,
-                                 base + 2 * a_pts, base + 2 * a_pts + a_ctr, false, sl.scans, sl.beams, nullptr,
-                                 m->workspace, -1, m->stream, true);
-    }
+    int rc = sl.batch.raycast(m, 0, sl.batch.scans, -1, nullptr, m->stream, true);
     if (rc) return rc;
     B2S_CUDA(cudaStreamSynchronize(m->stream));
-    if (saw_nan || saw_inf) {
-        set_error(saw_nan ? "cannot convert float NaN to integer" : "cannot convert float infinity to integer");
-        return B2S_ERR_NONFINITE;
-    }
-    set_error("%d beam(s) longer than %d cells: batch rejected", too_long, B2S_MAX_PATH_CELLS);
-    return B2S_ERR_TOO_LONG;
+    return batch_error(sl.h_cnt);
 }
 
 int mapping_submit_impl(b2s_mapping *m, const HostBatch &hb, int scans, int beams, int zero_first, int8_t *pmap_out,
@@ -1227,16 +1221,12 @@ int mapping_submit_impl(b2s_mapping *m, const HostBatch &hb, int scans, int beam
     int rc;
     if (sl.in_flight && (rc = mapping_wait_slot(m, sl))) return rc;  // its buffers are about to be reused
     const size_t total = (size_t)scans * beams, cells = (size_t)m->xw * m->yw;
-    const size_t a_pts = (total * sizeof(float) + 15) & ~(size_t)15;
-    const size_t poses = (size_t)scans * 4 * sizeof(double), table = (size_t)beams * 2 * sizeof(double);
-    const size_t a_ctr = ((size_t)scans * sizeof(float) + 15) & ~(size_t)15;
-    if ((rc = sl.d_in.reserve(hb.fused ? a_pts + poses + table : 2 * a_pts + 2 * a_ctr))) return rc;
+    const size_t poses = (size_t)scans * 4 * sizeof(double);
+    DeviceBatch db(hb, scans, beams);
+    if ((rc = sl.d_in.reserve(db.bytes()))) return rc;
     if ((rc = sl.d_map.reserve(cells))) return rc;
     if (hb.fused && hb.poses3 && (rc = sl.h_pose.reserve(poses ? poses : 16))) return rc;
-    char *base = (char *)sl.d_in.p;
-    float *d_a = (float *)base;
-    double *d_pose = (double *)(base + a_pts), *d_cs = (double *)(base + a_pts + poses);
-    char *d_b = base + a_pts, *d_c = base + 2 * a_pts, *d_d = base + 2 * a_pts + a_ctr;
+    db.bind(sl.d_in.p);
     cudaStream_t cs = m->copy_stream;
     // the copy stream may overwrite the slot's inputs once the ray-casts that last read them are done
     B2S_CUDA(cudaStreamWaitEvent(cs, sl.inputs_free, 0));
@@ -1249,46 +1239,13 @@ int mapping_submit_impl(b2s_mapping *m, const HostBatch &hb, int scans, int beam
     if (total > 0) {
         // a step submitted while the other slot is in flight has its upload hidden under that step's ray-cast and
         // goes as one launch; a step that starts on an idle device is cut into ~1 M-beam chunks (see the blocking call)
-        int nchunk = other.in_flight ? 1 : (int)((total + (1u << 20) - 1) >> 20);
-        if (nchunk > MAX_CHUNKS) nchunk = MAX_CHUNKS;
-        if (g_h2d_chunks > 0) nchunk = g_h2d_chunks;
-        if (nchunk > scans) nchunk = scans;
-        if (nchunk < 1) nchunk = 1;
-        if (hb.fused) B2S_CUDA(cudaMemcpyAsync(d_cs, hb.beam_cs, table, cudaMemcpyHostToDevice, cs));
-        double *tab = hb.fused && hb.poses3 ? (double *)sl.h_pose.p : nullptr;
-        const double *pose4 = tab ? tab : hb.pose4;
+        const int nchunk = pipeline_chunks(other.in_flight ? 1 : (int)((total + (1u << 20) - 1) >> 20), MAX_CHUNKS, scans);
         for (int k = 0; k < nchunk; ++k) {
-            const size_t s0 = (size_t)scans * k / nchunk, s1 = (size_t)scans * (k + 1) / nchunk, ns = s1 - s0;
-            if (hb.fused) {
-                if (tab)
-                    for (size_t s = s0; s < s1; ++s) {
-                        tab[4 * s] = hb.poses3[3 * s];
-                        tab[4 * s + 1] = hb.poses3[3 * s + 1];
-                        tab[4 * s + 2] = cos(hb.poses3[3 * s + 2]);
-                        tab[4 * s + 3] = sin(hb.poses3[3 * s + 2]);
-                    }
-                B2S_CUDA(cudaMemcpyAsync(d_a + s0 * beams, hb.ranges + s0 * beams, ns * beams * sizeof(float), cudaMemcpyHostToDevice, cs));
-                B2S_CUDA(cudaMemcpyAsync(d_pose + 4 * s0, pose4 + 4 * s0, ns * 4 * sizeof(double), cudaMemcpyHostToDevice, cs));
-            } else {
-                const size_t el = sizeof(float);
-                B2S_CUDA(cudaMemcpyAsync((char *)d_a + s0 * beams * el, (const char *)hb.ox + s0 * beams * el, ns * beams * el, cudaMemcpyHostToDevice, cs));
-                B2S_CUDA(cudaMemcpyAsync(d_b + s0 * beams * el, (const char *)hb.oy + s0 * beams * el, ns * beams * el, cudaMemcpyHostToDevice, cs));
-                B2S_CUDA(cudaMemcpyAsync(d_c + s0 * el, (const char *)hb.cx + s0 * el, ns * el, cudaMemcpyHostToDevice, cs));
-                B2S_CUDA(cudaMemcpyAsync(d_d + s0 * el, (const char *)hb.cy + s0 * el, ns * el, cudaMemcpyHostToDevice, cs));
-            }
+            const size_t s0 = (size_t)scans * k / nchunk, s1 = (size_t)scans * (k + 1) / nchunk;
+            if ((rc = db.upload(hb, s0, s1, (double *)sl.h_pose.p, cs))) return rc;
             B2S_CUDA(cudaEventRecord(m->chunk_ready[k], cs));
             B2S_CUDA(cudaStreamWaitEvent(m->stream, m->chunk_ready[k], 0));
-            const bool fold = (k == nchunk - 1);
-            if (hb.fused)
-                rc = grid_raycast_ranges_signed(m->hit, m->miss, m->xw, m->yw, m->cells_per_m, m->off_x, m->off_y,
-                                                d_a + s0 * beams, d_pose + 4 * s0, d_cs, hb.clamp, (int)ns, beams, sl.d_cnt,
-                                                m->workspace, +1, m->stream, fold);
-            else
-                rc = grid_raycast_signed(m->hit, m->miss, m->xw, m->yw, m->cells_per_m, m->off_x, m->off_y,
-                                         (char *)d_a + s0 * beams * sizeof(float), d_b + s0 * beams * sizeof(float),
-                                         d_c + s0 * sizeof(float), d_d + s0 * sizeof(float), false, (int)ns, beams, sl.d_cnt,
-                                         m->workspace, +1, m->stream, fold);
-            if (rc) return rc;
+            if ((rc = db.raycast(m, s0, s1, +1, sl.d_cnt, m->stream, k == nchunk - 1))) return rc;
         }
     }
     B2S_CUDA(cudaEventRecord(sl.inputs_free, m->stream));
@@ -1303,11 +1260,8 @@ int mapping_submit_impl(b2s_mapping *m, const HostBatch &hb, int scans, int beam
     B2S_CUDA(cudaMemcpyAsync(sl.h_cnt, sl.d_cnt, B2S_CNT_WORDS * sizeof(int32_t), cudaMemcpyDeviceToHost, m->d2h_stream));
     B2S_CUDA(cudaEventRecord(sl.done, m->d2h_stream));
     sl.in_flight = true;
-    sl.fused = hb.fused;
     sl.ticket = ticket;
-    sl.scans = scans;
-    sl.beams = beams;
-    sl.clamp = hb.clamp;
+    sl.batch = db;
     m->pmap_valid = false;  // the incremental read-back of update() starts over after streamed steps
     m->submitted = ticket + 1;
     if (ticket_out) *ticket_out = ticket;
