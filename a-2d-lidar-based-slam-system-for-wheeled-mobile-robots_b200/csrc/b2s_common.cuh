@@ -34,6 +34,13 @@ inline int cuda_fail(cudaError_t e, const char *what)
 
 int sm_count();
 
+constexpr int ICP_MAX_POINTS = 2304;  // source points per scan of the ICP kernel; see icp_points_per_thread
+
+// laserToNumpy of raw ranges [scans][beams] into float64 points [scans][2][beams] (b2s_next.cu); beam_cs [beams][2]
+// 16-byte aligned, clamp > 0 replaces +inf.  The points are those the ICP kernel's fused form makes from the ranges.
+int laser_points(const float *ranges, const double *beam_cs, double clamp, int scans, int beams, double *xy,
+                 cudaStream_t stream);
+
 // Growable device / pinned-host staging buffer.
 struct Buf {
     void *p = nullptr;

@@ -182,6 +182,10 @@ struct b2s_icp {
     cudaStream_t d2h_stream;
     cudaEvent_t solved;
     int submitted;
+    // Map observation (b2s_icp_set_map / b2s_icp_map_observation): the static map obs_x | obs_y, kept until replaced;
+    // the call's uploads (beam table | poses | ranges), and the target (+ virtual ranges) and source clouds it builds.
+    Buf d_map, d_map_in, d_map_tar, d_map_src;
+    int map_count = 0;
 };
 
 namespace {
@@ -465,6 +469,7 @@ extern "C" int b2s_icp_destroy(b2s_icp *c)
         if (sl.inputs_free) cudaEventDestroy(sl.inputs_free);
         if (sl.done) cudaEventDestroy(sl.done);
     }
+    c->d_map.release(); c->d_map_in.release(); c->d_map_tar.release(); c->d_map_src.release();
     if (c->solved) cudaEventDestroy(c->solved);
     if (c->d2h_stream) cudaStreamDestroy(c->d2h_stream);
     for (int k = 0; k < MAX_CHUNKS; ++k)
@@ -811,6 +816,115 @@ extern "C" int b2s_icp_wait(b2s_icp *c, int ticket)
     if (!sl.in_flight || sl.ticket != ticket) return B2S_OK;
     B2S_CUDA(cudaEventSynchronize(sl.done));
     sl.in_flight = false;
+    return B2S_OK;
+}
+
+static const char NAN_TO_INT[] = "cannot convert float NaN to integer";  // int(nan) in the reference
+
+extern "C" int b2s_icp_set_map(b2s_icp *c, const double *obs_x, const double *obs_y, int count)
+{
+    B2S_REQUIRE(c, "b2s_icp_set_map: null handle");
+    B2S_REQUIRE(count >= 0 && (count == 0 || (obs_x && obs_y)), "b2s_icp_set_map: bad arguments");
+    c->map_count = 0;
+    for (int i = 0; i < count; ++i)
+        if (obs_x[i] != obs_x[i] || obs_y[i] != obs_y[i]) {
+            set_error("%s", NAN_TO_INT);
+            return B2S_ERR_NONFINITE;
+        }
+    if (count == 0) return B2S_OK;
+    DeviceGuard g(c->device);
+    int rc;
+    if ((rc = c->d_map.reserve((size_t)count * 2 * sizeof(double)))) return rc;
+    double *d = (double *)c->d_map.p;
+    B2S_CUDA(cudaMemcpyAsync(d, obs_x, (size_t)count * sizeof(double), cudaMemcpyHostToDevice, c->stream));
+    B2S_CUDA(cudaMemcpyAsync(d + count, obs_y, (size_t)count * sizeof(double), cudaMemcpyHostToDevice, c->stream));
+    B2S_CUDA(cudaStreamSynchronize(c->stream));
+    c->map_count = count;
+    return B2S_OK;
+}
+
+// The pipeline of icp_sequence_enqueue: the ranges and poses of chunk k + 1 cross PCIe on the copy stream while chunk k
+// is solved, and the chunks alternate between stream and stream2.  Per chunk: the virtual scans straight into the
+// target layout, laserToNumpy of the ranges into the source layout, then the float64 ICP on the two.
+extern "C" int b2s_icp_map_observation(b2s_icp *c, const float *ranges, const double *poses3, const double *beam_cs,
+                                       double clamp_inf_to, int scans, int n, double angle_min, double angle_increment,
+                                       double far_range, int max_iter, double tol, double *T_out, int32_t *iters_out,
+                                       double *virtual_out)
+{
+    B2S_REQUIRE(c, "b2s_icp_map_observation: null handle");
+    B2S_REQUIRE(scans >= 0 && n > 0 && max_iter >= 0, "b2s_icp_map_observation: bad sizes");
+    B2S_REQUIRE(n <= ICP_MAX_POINTS, "b2s_icp_batch: more than 2304 source points per scan is not supported");
+    B2S_REQUIRE(c->map_count > 0, "b2s_icp_map_observation: no static map set (b2s_icp_set_map)");
+    if (scans == 0) return B2S_OK;
+    B2S_REQUIRE(ranges && poses3 && beam_cs && T_out, "b2s_icp_map_observation: null pointer");
+    B2S_REQUIRE(clamp_inf_to == clamp_inf_to && tol == tol, "b2s_icp_map_observation: NaN clamp / tolerance");
+    B2S_REQUIRE(angle_increment != 0.0 && angle_increment == angle_increment, "b2s_icp_map_observation: angle_increment");
+    // the reference's int() raises on the first obstacle's bin of a NaN pose; +-inf poses only give bins no obstacle wins
+    for (size_t i = 0; i < (size_t)scans * 3; ++i)
+        if (poses3[i] != poses3[i]) {
+            set_error("%s", NAN_TO_INT);
+            return B2S_ERR_NONFINITE;
+        }
+    DeviceGuard g(c->device);
+    Trace tr(c->stream);
+    const size_t cs_bytes = (size_t)n * 2 * sizeof(double), pose_bytes = (size_t)scans * 3 * sizeof(double);
+    const size_t pose_off = cs_bytes, range_off = (pose_off + pose_bytes + 15) & ~(size_t)15;
+    const size_t cloud = (size_t)scans * 2 * n;  // doubles of one cloud set
+    int rc;
+    if ((rc = c->d_map_in.reserve(range_off + (size_t)scans * n * sizeof(float)))) return rc;
+    if ((rc = c->d_map_tar.reserve((cloud + (virtual_out ? (size_t)scans * n : 0)) * sizeof(double)))) return rc;
+    if ((rc = c->d_map_src.reserve(cloud * sizeof(double)))) return rc;
+    if ((rc = c->d_T.reserve((size_t)scans * 9 * sizeof(double)))) return rc;
+    if ((rc = c->d_iters.reserve((size_t)scans * sizeof(int32_t)))) return rc;
+    char *in = (char *)c->d_map_in.p;
+    const double *d_cs = (const double *)in, *d_pose = (const double *)(in + pose_off);
+    const float *d_ranges = (const float *)(in + range_off);
+    double *d_tar = (double *)c->d_map_tar.p, *d_src = (double *)c->d_map_src.p, *d_virt = virtual_out ? d_tar + cloud : nullptr;
+    const double *map_x = (const double *)c->d_map.p, *map_y = map_x + c->map_count;
+    // at most ~8 MB of uploads and ~2500 scans per chunk (about three waves of ICP CTAs).  Measured on the course map,
+    // 360 beams (profiles/r6): 3000 scans 0.932 / 0.906 / 0.966 ms at 1 / 2 / 4 chunks, 9999 scans 2.79 / 2.69 / 2.63 ms
+    // at 1 / 2 / 4 chunks
+    int want = (int)(((size_t)scans * ((size_t)n * sizeof(float) + 3 * sizeof(double)) + (8u << 20) - 1) / (8u << 20));
+    if (want < (scans + 2499) / 2500) want = (scans + 2499) / 2500;
+    const int nchunk = pipeline_chunks(want, 8, scans);
+    B2S_CUDA(cudaMemcpyAsync(in, beam_cs, cs_bytes, cudaMemcpyHostToDevice, c->copy_stream));
+    for (int k = 0; k < nchunk; ++k) {
+        const size_t s0 = (size_t)scans * k / nchunk, s1 = (size_t)scans * (k + 1) / nchunk;
+        B2S_CUDA(cudaMemcpyAsync(in + pose_off + s0 * 3 * sizeof(double), poses3 + s0 * 3, (s1 - s0) * 3 * sizeof(double),
+                                 cudaMemcpyHostToDevice, c->copy_stream));
+        B2S_CUDA(cudaMemcpyAsync(in + range_off + s0 * n * sizeof(float), ranges + s0 * n, (s1 - s0) * n * sizeof(float),
+                                 cudaMemcpyHostToDevice, c->copy_stream));
+        B2S_CUDA(cudaEventRecord(c->chunk_ready[k], c->copy_stream));
+        tr.mark("h2d chunk done", k, c->copy_stream);
+    }
+    for (int k = 0; k < nchunk; ++k) {
+        const size_t s0 = (size_t)scans * k / nchunk, s1 = (size_t)scans * (k + 1) / nchunk;
+        const int ns = (int)(s1 - s0);
+        cudaStream_t ks = (k & 1) ? c->stream2 : c->stream;
+        B2S_CUDA(cudaStreamWaitEvent(ks, c->chunk_ready[k], 0));
+        double *tar = d_tar + s0 * 2 * n, *src = d_src + s0 * 2 * n;
+        if ((rc = b2s_virtual_scan_batch(map_x, map_y, c->map_count, d_pose + s0 * 3, ns, angle_min, angle_increment, n,
+                                         far_range, d_cs, d_virt ? d_virt + s0 * n : nullptr, tar, ks)))
+            return rc;
+        tr.mark("virtual scan chunk done", k, ks);
+        if ((rc = laser_points(d_ranges + s0 * n, d_cs, clamp_inf_to, ns, n, src, ks))) return rc;
+        if ((rc = b2s_icp_batch_f64(tar, src, ns, n, n, max_iter, tol, (double *)c->d_T.p + s0 * 9,
+                                    (int32_t *)c->d_iters.p + s0, ks)))
+            return rc;
+        tr.mark("icp chunk done", k, ks);
+    }
+    if (nchunk > 1) {
+        B2S_CUDA(cudaEventRecord(c->joined, c->stream2));
+        B2S_CUDA(cudaStreamWaitEvent(c->stream, c->joined, 0));
+    }
+    B2S_CUDA(cudaMemcpyAsync(T_out, c->d_T.p, (size_t)scans * 9 * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
+    if (iters_out)
+        B2S_CUDA(cudaMemcpyAsync(iters_out, c->d_iters.p, (size_t)scans * sizeof(int32_t), cudaMemcpyDeviceToHost, c->stream));
+    if (virtual_out)
+        B2S_CUDA(cudaMemcpyAsync(virtual_out, d_virt, (size_t)scans * n * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
+    tr.mark("results d2h done", 0, c->stream);
+    B2S_CUDA(cudaStreamSynchronize(c->stream));
+    tr.mark("synchronized", 0, nullptr);
     return B2S_OK;
 }
 

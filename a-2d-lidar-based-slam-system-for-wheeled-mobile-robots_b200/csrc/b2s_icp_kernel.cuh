@@ -1004,8 +1004,6 @@ static int launch_icp_r(const TIn *tar_xy, const TIn *src_xy, int pairs, int n_s
 // Points per thread: work is proportional to the register slots (threads x points per thread, idle ones included).
 // Three is the measured optimum on B200 (360 and 1080 beams) and is taken unless it wastes more than 10 % over the
 // leanest choice; then 4, then 2.
-constexpr int ICP_MAX_POINTS = 2304;  // per scan; see icp_points_per_thread
-
 static int icp_points_per_thread(int n_src)
 {
     if (g_icp_src_per_thread) return g_icp_src_per_thread;

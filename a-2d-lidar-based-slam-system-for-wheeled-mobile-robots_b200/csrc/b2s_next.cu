@@ -4,7 +4,9 @@
 //                 over a stream of per-pair transforms -> a prefix sum of the yaw increments followed by a
 //                 prefix sum of the rotated translations (one CTA, blocked scan).
 //   virtual scan  W9 localization.py:128-150 (laserEstimation): min range per bearing bin over the static-map
-//                 obstacle cells -> one thread per obstacle, atomicMin on the float64 bit pattern.
+//                 obstacle cells -> one thread per obstacle, atomicMin on the float64 bit pattern.  The batched form
+//                 reduces each pose's bins in shared memory and can write them as the ICP's target cloud.
+//   laserToNumpy  [ICP]:216-229 / [SLAM]:115-123 of float32 ranges into float64 points (the ICP's source cloud).
 #include "b2s_common.cuh"
 
 #include <math.h>
@@ -82,11 +84,35 @@ pose_chain_kernel(const double *__restrict__ T, int pairs, double x0, double y0,
     }
 }
 
-__global__ void __launch_bounds__(256)
-virtual_scan_init_kernel(double *__restrict__ ranges, int beams, double far_range)
+// One obstacle of laserEstimation (localization.py:137-146): its range and bearing bin seen from (x, y, yaw).  Both the
+// single-pose and the batched kernel call this, so their bins cannot drift apart.  The _rn intrinsics keep the compiler
+// from contracting the subtractions or the division with the last multiply of an inlined atan2 / hypot.  Returns false
+// where int() would raise (NaN) or overflow, and for a NaN distance: such an obstacle never lowers a bin.
+__device__ __forceinline__ bool vscan_bin(double ox, double oy, double x, double y, double yaw, double angle_min,
+                                          double angle_increment, int beams, int &index, double &dist)
 {
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < beams) ranges[i] = far_range;
+    dist = hypot(__dsub_rn(x, ox), __dsub_rn(y, oy));                                              // :138
+    const double bin = __ddiv_rn(__dsub_rn(__dsub_rn(atan2(__dsub_rn(oy, y), __dsub_rn(ox, x)), angle_min), yaw),
+                                 angle_increment);                                                 // :139
+    if (!(fabs(bin) < 2.0e9) || !(dist == dist)) return false;
+    index = (int)bin;   // truncation toward zero
+    index %= beams;     // the two while loops, :141-144
+    if (index < 0) index += beams;
+    return true;
+}
+
+// distances are >= 0, so the IEEE bit patterns order like the values: the bins are min-reduced on the bits
+__device__ __forceinline__ unsigned long long range_bits(double d) { return (unsigned long long)__double_as_longlong(d); }
+
+// far_range into rows [scans][beams] of stride `stride` (the initial bins of the single-pose kernel and
+// the merge target of the batched one)
+__global__ void __launch_bounds__(256)
+virtual_scan_fill_kernel(double *p, int scans, int beams, size_t stride, double far_range)
+{
+    const size_t j = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= (size_t)scans * beams) return;
+    const size_t k = j / beams;
+    p[k * stride + (j - k * beams)] = far_range;
 }
 
 __global__ void __launch_bounds__(256)
@@ -96,15 +122,112 @@ virtual_scan_kernel(const double *__restrict__ obs_x, const double *__restrict__
 {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= count) return;
-    const double ox = obs_x[i], oy = obs_y[i];
-    const double dist = hypot(x - ox, y - oy);                                        // localization.py:138
-    const double bin = (atan2(oy - y, ox - x) - angle_min - yaw) / angle_increment;    // localization.py:139
-    if (!(fabs(bin) < 2.0e9) || !(dist == dist)) return;                               // int() would raise / overflow
-    int index = (int)bin;                                                              // truncation toward zero
-    index %= beams;                                                                    // the two while loops, :141-144
-    if (index < 0) index += beams;
-    // distances are >= 0, so the IEEE bit patterns order like the values: atomicMin on the bits
-    atomicMin(reinterpret_cast<unsigned long long *>(ranges) + index, (unsigned long long)__double_as_longlong(dist));
+    int index;
+    double dist;
+    if (vscan_bin(obs_x[i], obs_y[i], x, y, yaw, angle_min, angle_increment, beams, index, dist))
+        atomicMin(reinterpret_cast<unsigned long long *>(ranges) + index, range_bits(dist));
+}
+
+// Batched virtual scan: CTA (k, s) reduces obstacle slice s of pose k into bins in shared memory.  With one slice per
+// pose (slices == 1) the CTA owns the pose and writes its ranges and target points itself.  Otherwise it merges only
+// the bins it lowered below far_range into `merge` [scans][beams] (set to far_range beforehand) with a global
+// atomicMin, and virtual_scan_points_kernel forms the points once every slice is done.  Rows of `merge` are
+// merge_stride doubles apart: [scans][beams] ranges, or the x rows of the target [scans][2][beams].
+constexpr int VSCAN_THREADS = 256;
+
+__global__ void __launch_bounds__(VSCAN_THREADS)
+virtual_scan_batch_kernel(const double *__restrict__ obs_x, const double *__restrict__ obs_y, int count, int per_slice,
+                          const double *__restrict__ poses3, double angle_min, double angle_increment, int beams,
+                          double far_range, const double2 *__restrict__ beam_cs, double *__restrict__ ranges,
+                          double *__restrict__ tar_xy, double *__restrict__ merge, size_t merge_stride)
+{
+    extern __shared__ unsigned long long bins[];
+    const int k = blockIdx.x;
+    const double x = poses3[3 * k], y = poses3[3 * k + 1], yaw = poses3[3 * k + 2];
+    const unsigned long long far = range_bits(far_range);
+    for (int i = threadIdx.x; i < beams; i += VSCAN_THREADS) bins[i] = far;
+    __syncthreads();
+    const int c0 = blockIdx.y * per_slice, c1 = min(count, c0 + per_slice);
+    for (int c = c0 + threadIdx.x; c < c1; c += VSCAN_THREADS) {
+        int index;
+        double dist;
+        if (vscan_bin(obs_x[c], obs_y[c], x, y, yaw, angle_min, angle_increment, beams, index, dist))
+            atomicMin(bins + index, range_bits(dist));
+    }
+    __syncthreads();
+    if (merge) {
+        unsigned long long *m = reinterpret_cast<unsigned long long *>(merge + (size_t)k * merge_stride);
+        for (int i = threadIdx.x; i < beams; i += VSCAN_THREADS)
+            if (bins[i] < far) atomicMin(m + i, bins[i]);
+        return;
+    }
+    const size_t row = (size_t)k * beams;
+    for (int i = threadIdx.x; i < beams; i += VSCAN_THREADS) {
+        const double r = __longlong_as_double((long long)bins[i]);
+        if (ranges) ranges[row + i] = r;
+        if (tar_xy) {  // laserToNumpy: np.cos(a) * r, np.sin(a) * r -- one IEEE multiply each
+            const double2 cs = beam_cs[i];
+            tar_xy[2 * row + i] = __dmul_rn(cs.x, r);
+            tar_xy[2 * row + beams + i] = __dmul_rn(cs.y, r);
+        }
+    }
+}
+
+// Points of the merged ranges (multi-slice path).  `ranges` may alias the x row of tar_xy: each thread reads its range
+// before it writes the two coordinates.
+__global__ void __launch_bounds__(256)
+virtual_scan_points_kernel(const double *ranges, const double2 *__restrict__ beam_cs, int scans, int beams,
+                           size_t range_stride, double *tar_xy)
+{
+    const size_t j = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= (size_t)scans * beams) return;
+    const size_t k = j / beams;
+    const int i = (int)(j - k * beams);
+    const double r = ranges[k * range_stride + i];
+    const double2 cs = beam_cs[i];
+    tar_xy[2 * k * beams + i] = __dmul_rn(cs.x, r);
+    tar_xy[2 * k * beams + beams + i] = __dmul_rn(cs.y, r);
+}
+
+// laserToNumpy of raw float32 ranges into float64 points [scans][2][beams], with the arithmetic of the ICP kernel's
+// RANGES form (b2s_icp_kernel.cuh, icp_batch_kernel's `point`): +inf -> clamp when clamp > 0, then one IEEE multiply.
+__global__ void __launch_bounds__(256)
+laser_points_kernel(const float *__restrict__ ranges, const double2 *__restrict__ beam_cs, double clamp, int scans,
+                    int beams, double *__restrict__ xy)
+{
+    const size_t j = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= (size_t)scans * beams) return;
+    const size_t k = j / beams;
+    const int i = (int)(j - k * beams);
+    double r = (double)ranges[j];
+    if (clamp > 0.0 && r == INFINITY) r = clamp;  // [SLAM]:119 (only +inf compares equal)
+    const double2 cs = beam_cs[i];
+    xy[2 * k * beams + i] = __dmul_rn(cs.x, r);
+    xy[2 * k * beams + beams + i] = __dmul_rn(cs.y, r);
+}
+
+// Slices per pose: one CTA per pose when the poses alone fill the device a few times over; otherwise the obstacles are
+// cut into slices of at least VSCAN_MIN_SLICE cells so that a small batch over a large map still spreads over every SM.
+constexpr int VSCAN_MIN_SLICE = 1024;
+
+static int vscan_slices(int count, int scans)
+{
+    const long long want_ctas = (long long)sm_count() * 8;
+    if (count <= VSCAN_MIN_SLICE || scans >= want_ctas) return 1;
+    const long long by_size = (count + VSCAN_MIN_SLICE - 1) / VSCAN_MIN_SLICE;
+    const long long by_fill = (want_ctas + scans - 1) / scans;
+    return (int)(by_size < by_fill ? by_size : by_fill);
+}
+
+int laser_points(const float *ranges, const double *beam_cs, double clamp, int scans, int beams, double *xy,
+                 cudaStream_t st)
+{
+    const size_t total = (size_t)scans * beams;
+    if (total == 0) return B2S_OK;
+    laser_points_kernel<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(ranges, reinterpret_cast<const double2 *>(beam_cs),
+                                                                        clamp, scans, beams, xy);
+    B2S_CUDA(cudaGetLastError());
+    return B2S_OK;
 }
 
 }  // namespace b2s
@@ -127,11 +250,53 @@ extern "C" int b2s_virtual_scan(const double *obs_x, const double *obs_y, int co
     B2S_REQUIRE(count >= 0 && beams > 0 && ranges && (count == 0 || (obs_x && obs_y)), "b2s_virtual_scan: bad arguments");
     B2S_REQUIRE(angle_increment != 0.0 && angle_increment == angle_increment, "b2s_virtual_scan: angle_increment");
     cudaStream_t st = (cudaStream_t)stream;
-    virtual_scan_init_kernel<<<(beams + 255) / 256, 256, 0, st>>>(ranges, beams, far_range);
+    virtual_scan_fill_kernel<<<(beams + 255) / 256, 256, 0, st>>>(ranges, 1, beams, beams, far_range);
     B2S_CUDA(cudaGetLastError());
     if (count > 0) {
         virtual_scan_kernel<<<(count + 255) / 256, 256, 0, st>>>(obs_x, obs_y, count, x, y, yaw, angle_min,
                                                                  angle_increment, beams, ranges);
+        B2S_CUDA(cudaGetLastError());
+    }
+    return B2S_OK;
+}
+
+extern "C" int b2s_virtual_scan_batch(const double *obs_x, const double *obs_y, int count, const double *poses3, int scans,
+                                      double angle_min, double angle_increment, int beams, double far_range,
+                                      const double *beam_cs, double *ranges, double *tar_xy, void *stream)
+{
+    B2S_REQUIRE(count >= 0 && scans >= 0 && beams > 0, "b2s_virtual_scan_batch: bad sizes");
+    B2S_REQUIRE(beams <= B2S_VSCAN_MAX_BEAMS, "b2s_virtual_scan_batch: more than 6144 beams per scan is not supported");
+    B2S_REQUIRE((count == 0 || (obs_x && obs_y)) && (scans == 0 || poses3) && (ranges || tar_xy),
+                "b2s_virtual_scan_batch: null pointer");
+    B2S_REQUIRE(!tar_xy || (beam_cs && (uintptr_t)beam_cs % 16 == 0),
+                "b2s_virtual_scan_batch: tar_xy needs a 16-byte aligned beam table");
+    B2S_REQUIRE(angle_increment != 0.0 && angle_increment == angle_increment, "b2s_virtual_scan_batch: angle_increment");
+    if (scans == 0) return B2S_OK;
+    cudaStream_t st = (cudaStream_t)stream;
+    const int slices = vscan_slices(count, scans);
+    const int per_slice = count > 0 ? (count + slices - 1) / slices : 0;
+    const size_t smem = (size_t)beams * sizeof(unsigned long long);
+    const double2 *cs = reinterpret_cast<const double2 *>(beam_cs);
+    if (slices == 1) {
+        virtual_scan_batch_kernel<<<dim3(scans, 1), VSCAN_THREADS, smem, st>>>(obs_x, obs_y, count, per_slice, poses3, angle_min,
+                                                                               angle_increment, beams, far_range, cs, ranges,
+                                                                               tar_xy, nullptr, 0);
+        B2S_CUDA(cudaGetLastError());
+        return B2S_OK;
+    }
+    // merged ranges go to `ranges`, or without it to the x rows of tar_xy, which the points kernel then overwrites
+    double *merge = ranges ? ranges : tar_xy;
+    const size_t stride = ranges ? (size_t)beams : (size_t)2 * beams;
+    const size_t total = (size_t)scans * beams;
+    const unsigned blocks = (unsigned)((total + 255) / 256);
+    virtual_scan_fill_kernel<<<blocks, 256, 0, st>>>(merge, scans, beams, stride, far_range);
+    B2S_CUDA(cudaGetLastError());
+    virtual_scan_batch_kernel<<<dim3(scans, slices), VSCAN_THREADS, smem, st>>>(obs_x, obs_y, count, per_slice, poses3, angle_min,
+                                                                                angle_increment, beams, far_range, cs, nullptr,
+                                                                                nullptr, merge, stride);
+    B2S_CUDA(cudaGetLastError());
+    if (tar_xy) {
+        virtual_scan_points_kernel<<<blocks, 256, 0, st>>>(merge, cs, scans, beams, stride, tar_xy);
         B2S_CUDA(cudaGetLastError());
     }
     return B2S_OK;

@@ -123,3 +123,26 @@ def icp_batch(tar, src, max_iter=30, tol=1e-3, T_out=None, iters_out=None):
             _stream())
     _lib.check(rc)
     return T_out, iters_out
+
+
+def virtual_scan_batch(obs_x, obs_y, poses, angle_min, angle_increment, beams, far_range=100.0, beam_cs=None,
+                       ranges=None, tar_xy=None):
+    """b2s_virtual_scan_batch: laserEstimation for K poses at once.  obs_x, obs_y float64 (C,) obstacle cell centres,
+    poses float64 (K,3) = x, y, yaw.  ranges (K,beams) float64 receives what scan.virtual_scan gives per pose;
+    tar_xy (K,2,beams) float64 (needs beam_cs float64 (beams,2), scan.beam_table) receives their laserToNumpy points,
+    the target layout of icp_batch.  Without either output, ranges is allocated.  Returns (ranges, tar_xy)."""
+    K, C, beams = poses.shape[0], obs_x.shape[0], int(beams)
+    if ranges is None and tar_xy is None:
+        ranges = torch.empty((K, beams), dtype=torch.float64, device=poses.device)
+    for t, shape, name in ((poses, (K, 3), "poses"), (obs_y, (C,), "obs_y"), (ranges, (K, beams), "ranges"),
+                           (tar_xy, (K, 2, beams), "tar_xy"), (beam_cs, (beams, 2), "beam_cs")):
+        if t is not None and tuple(t.shape) != shape:
+            raise ValueError("%s must have shape %s, got %s" % (name, shape, tuple(t.shape)))
+    rc = _lib.lib().b2s_virtual_scan_batch(
+        _chk(obs_x, torch.float64, "obs_x"), _chk(obs_y, torch.float64, "obs_y"), C,
+        _chk(poses, torch.float64, "poses"), K, float(angle_min), float(angle_increment), beams, float(far_range),
+        None if beam_cs is None else _chk(beam_cs, torch.float64, "beam_cs"),
+        None if ranges is None else _chk(ranges, torch.float64, "ranges"),
+        None if tar_xy is None else _chk(tar_xy, torch.float64, "tar_xy"), _stream())
+    _lib.check(rc)
+    return ranges, tar_xy

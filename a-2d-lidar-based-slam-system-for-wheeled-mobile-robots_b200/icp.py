@@ -197,15 +197,11 @@ class ICP(object):
 
     def submit_scans(self, ranges, angle_min, angle_max, clamp_inf_to=None, max_iter=None, tolerance=None):
         """process_scans (raw ranges, no pose chain) without the wait; see submit_sequence."""
-        from b2slam import scan
         ranges = np.ascontiguousarray(ranges, dtype=np.float32)
         if ranges.ndim != 2 or ranges.shape[1] < 1:
             raise ValueError("expected ranges (K,N) with N >= 1, got %s" % (ranges.shape,))
         K, N = ranges.shape
-        key = (float(angle_min), float(angle_max), N)
-        if getattr(self, "_beam_key", None) != key:
-            self._beam_cs = scan.beam_table(angle_min, angle_max, N)
-            self._beam_key = key
+        self._beam_table(angle_min, angle_max, N)
         P = max(K - 1, 0)
         k, (T, iters) = self._stream_out(P)
         t = ctypes.c_int(-1)
@@ -242,6 +238,65 @@ class ICP(object):
             _lib.ptr(T) if K > 1 else None, _lib.ptr(iters) if K > 1 else None))
         return traj, T.reshape(K - 1, 3, 3), iters
 
+    def _beam_table(self, angle_min, angle_max, N):
+        from b2slam import scan
+        key = (float(angle_min), float(angle_max), N)
+        if getattr(self, "_beam_key", None) != key:
+            self._beam_cs = scan.beam_table(angle_min, angle_max, N)
+            self._beam_key = key
+        return self._beam_cs
+
+    # ------------------------------------------------------------------ map observation (W9 localization)
+
+    def set_static_map(self, obstacle_xy):
+        """The localization node's static map (self.obstacle): obstacle_xy (2, C) world coordinates of the occupied
+        cell centres, as scan.virtual_scan takes them.  Uploaded once and kept on the device until replaced; C = 0
+        clears it.  A NaN coordinate raises ValueError (the reference's int() raises on it) and clears the map."""
+        obstacle_xy = np.asarray(obstacle_xy, dtype=np.float64)
+        if obstacle_xy.ndim != 2 or obstacle_xy.shape[0] != 2:
+            raise ValueError("expected obstacle_xy (2, C), got %s" % (obstacle_xy.shape,))
+        ox = np.ascontiguousarray(obstacle_xy[0])
+        oy = np.ascontiguousarray(obstacle_xy[1])
+        C = ox.shape[0]
+        _lib.check(self._L.b2s_icp_set_map(self._h, _lib.ptr(ox) if C else None, _lib.ptr(oy) if C else None, C))
+
+    def map_observation(self, ranges, poses, angle_min, angle_max, angle_increment=None, clamp_inf_to=None,
+                        far_range=100.0, max_iter=None, tolerance=None, return_virtual=False):
+        """calc_map_observation ([LOC9]:152-157) for a recorded stream: for scan k the virtual scan of the static map
+        (set_static_map) at poses[k] (laserEstimation, [LOC9]:128-150) is the target, laserToNumpy(ranges[k]) the
+        source, T[k] = ICP.process(target, source).  Everything runs on the device: the same transforms as
+        process_batch(stack(laser_to_points(virtual_k)[:2]), stack(laser_to_points(ranges_k, ...)[:2])), bit for bit.
+
+        ranges (K,N) float32 (LaserScan.ranges), poses (K,3) = x, y, yaw.  The virtual scan bins with angle_increment
+        (default (angle_max - angle_min) / (N - 1); pass the LaserScan's own field where it differs); both clouds
+        take their beam angles from linspace(angle_min, angle_max, N) like laserToNumpy.  clamp_inf_to: the W12 inf
+        clamp of the source.  Returns (T (K,3,3), iterations (K,)), and the virtual ranges (K,N) float64 with
+        return_virtual=True.  A NaN pose raises ValueError like the reference's int().
+        """
+        ranges = np.ascontiguousarray(ranges, dtype=np.float32)
+        if ranges.ndim != 2 or ranges.shape[1] < 1:
+            raise ValueError("expected ranges (K,N) with N >= 1, got %s" % (ranges.shape,))
+        K, N = ranges.shape
+        poses = np.ascontiguousarray(poses, dtype=np.float64)
+        if poses.shape != (K, 3):
+            raise ValueError("expected poses (%d,3), got %s" % (K, poses.shape))
+        if angle_increment is None:
+            if N < 2:
+                raise ValueError("a one-beam scan needs an explicit angle_increment")
+            angle_increment = (float(angle_max) - float(angle_min)) / (N - 1)
+        cs = self._beam_table(angle_min, angle_max, N)
+        T = np.empty((K, 9))
+        iters = np.empty(K, dtype=np.int32)
+        virt = np.empty((K, N)) if return_virtual else None
+        _lib.check(self._L.b2s_icp_map_observation(
+            self._h, _lib.ptr(ranges), _lib.ptr(poses), _lib.ptr(cs), float(clamp_inf_to or 0.0), K, N,
+            float(angle_min), float(angle_increment), float(far_range),
+            self.max_iter if max_iter is None else int(max_iter),
+            self.tolerance if tolerance is None else float(tolerance),
+            _lib.ptr(T), _lib.ptr(iters), _lib.ptr(virt)))
+        T = T.reshape(K, 3, 3)
+        return (T, iters, virt) if return_virtual else (T, iters)
+
     def process_scans(self, ranges, angle_min, angle_max, clamp_inf_to=None, state=None, max_iter=None,
                       tolerance=None):
         """process_sequence / odometry fed with what the sensor delivers: ranges (K,N) float32 (LaserScan.ranges of
@@ -252,15 +307,11 @@ class ICP(object):
 
         Returns (T (K-1,3,3), iterations (K-1,)), or with state=(x, y, yaw) (trajectory (K,3), T, iterations).
         """
-        from b2slam import scan
         ranges = np.ascontiguousarray(ranges, dtype=np.float32)
         if ranges.ndim != 2 or ranges.shape[1] < 1:
             raise ValueError("expected ranges (K,N) with N >= 1, got %s" % (ranges.shape,))
         K, N = ranges.shape
-        key = (float(angle_min), float(angle_max), N)
-        if getattr(self, "_beam_key", None) != key:
-            self._beam_cs = scan.beam_table(angle_min, angle_max, N)
-            self._beam_key = key
+        self._beam_table(angle_min, angle_max, N)
         P = max(K - 1, 0)
         T = np.empty((P, 9))
         iters = np.empty(P, dtype=np.int32)

@@ -99,12 +99,8 @@ def _raycast_polygon(poly, px, py, ang):
     return t.min(axis=-1)
 
 
-def room_sequence(seed, scans, n_beams, chunk=512):
-    """cfg 2: `scans` scans of one polygon room from a smooth trajectory (seed 9001).
-
-    Steps are <= 0.1 m and <= 0.05 rad per scan.  Returns (xy float32 (scans, 2, n_beams)
-    in the sensor frame, poses float64 (scans, 3)).
-    """
+def _room_ranges(seed, scans, n_beams, chunk=512):
+    """The room, trajectory and noisy float64 ranges (scans, n_beams) behind room_sequence."""
     rng = _rng(seed)
     poly = _room_polygon(rng)
     poses = np.zeros((scans, 3))
@@ -124,15 +120,59 @@ def room_sequence(seed, scans, n_beams, chunk=512):
         x, y = nx, ny
         th = th + w
     phi = beam_angles(n_beams)[None, :]
-    out = np.empty((scans, 2, n_beams), dtype=np.float32)
+    r = np.empty((scans, n_beams))
     for s in range(0, scans, chunk):
         e = min(scans, s + chunk)
         ang = phi + poses[s:e, 2:3]
-        r = _raycast_polygon(poly, poses[s:e, 0], poses[s:e, 1], ang)
-        r = noisy(rng, np.minimum(r, RANGE_MAX))
-        out[s:e, 0, :] = r * np.cos(phi)
-        out[s:e, 1, :] = r * np.sin(phi)
+        r[s:e] = noisy(rng, np.minimum(_raycast_polygon(poly, poses[s:e, 0], poses[s:e, 1], ang), RANGE_MAX))
+    return poly, r, poses, rng
+
+
+def room_sequence(seed, scans, n_beams, chunk=512):
+    """cfg 2: `scans` scans of one polygon room from a smooth trajectory (seed 9001).
+
+    Steps are <= 0.1 m and <= 0.05 rad per scan.  Returns (xy float32 (scans, 2, n_beams)
+    in the sensor frame, poses float64 (scans, 3)).
+    """
+    _, r, poses, _ = _room_ranges(seed, scans, n_beams, chunk)
+    phi = beam_angles(n_beams)[None, :]
+    out = np.empty((scans, 2, n_beams), dtype=np.float32)
+    out[:, 0, :] = r * np.cos(phi)
+    out[:, 1, :] = r * np.sin(phi)
     return out, poses
+
+
+def _wall_cells(poly, reso, cells, half_width):
+    """Centres (2, C) of the cells of a cells x cells map at `reso` m, centred on the origin, that lie within
+    half_width of an edge of the polygon: the room rasterised into the obstacle list of a static map."""
+    c = (np.arange(cells) + 0.5) * reso - cells * reso / 2.0
+    keep = []
+    for row in range(0, cells, 256):  # rows of the map in blocks: bounded memory on fine maps
+        gx, gy = np.meshgrid(c[row:row + 256], c, indexing="ij")
+        near = np.zeros(gx.shape, dtype=bool)
+        for a, b in zip(poly, np.roll(poly, -1, axis=0)):
+            e = b - a
+            t = np.clip(((gx - a[0]) * e[0] + (gy - a[1]) * e[1]) / (e @ e), 0.0, 1.0)
+            near |= np.hypot(gx - a[0] - t * e[0], gy - a[1] - t * e[1]) <= half_width
+        keep.append(np.stack([gx[near], gy[near]]))
+    return np.concatenate(keep, axis=1)
+
+
+def room_map_observation(seed, scans, n_beams, pose_sigma=(0.03, 0.03, 0.02)):
+    """The map observation of W9 localization ([LOC9]:152-157) on the cfg-2 room: a static map, the scans of
+    room_sequence's trajectory and the EKF prior poses at which the map is observed.
+
+    Returns a dict: ranges float32 (scans, n_beams) (beam angles linspace(-pi, pi, n_beams)), poses float64 (scans, 3)
+    the true poses, prior float64 (scans, 3) the poses perturbed by N(0, pose_sigma) (m, m, rad), and two obstacle lists
+    (2, C) of wall cell centres: obstacles_course on the course map's grid (129 x 129 cells at 0.155 m,
+    course_agv_gazebo/config/map.yaml; walls 0.2 m either side) and obstacles_fine on a finer, larger one
+    (2600 x 2600 cells at 0.01 m; walls 0.25 m either side), more than 2 * 10^5 cells.
+    """
+    poly, r, poses, rng = _room_ranges(seed, scans, n_beams)
+    prior = poses + rng.normal(0.0, 1.0, size=poses.shape) * np.asarray(pose_sigma)
+    return {"ranges": r.astype(np.float32), "poses": poses, "prior": prior,
+            "obstacles_course": _wall_cells(poly, 0.155, 129, 0.2),
+            "obstacles_fine": _wall_cells(poly, 0.01, 2600, 0.25)}
 
 
 # ------------------------------------------------------------------ cfg 3 / 5: grid streams

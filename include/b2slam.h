@@ -190,6 +190,16 @@ int b2s_virtual_scan(const double *obs_x, const double *obs_y, int count, double
 int b2s_virtual_scan_host(const double *obs_x, const double *obs_y, int count, double x, double y,
                           double yaw, double angle_min, double angle_increment, int beams,
                           double far_range, double *ranges);
+/* laserEstimation (W9 localization.py:128-150) for `scans` poses at once: poses3 [scans][3] = x, y, yaw.
+ * ranges [scans][beams] (may be NULL) gets exactly what b2s_virtual_scan gives per pose; tar_xy [scans][2][beams]
+ * (may be NULL; needs beam_cs [beams][2], 16-byte aligned) gets laserToNumpy of those ranges, the target layout of
+ * b2s_icp_batch_f64.  At least one of the two is set; beams <= B2S_VSCAN_MAX_BEAMS (the bins of a pose live in
+ * shared memory).  Like b2s_virtual_scan, an obstacle whose bin is NaN or overflows int is skipped: the host-buffer
+ * caller rejects NaN poses before the launch. */
+#define B2S_VSCAN_MAX_BEAMS 6144
+int b2s_virtual_scan_batch(const double *obs_x, const double *obs_y, int count, const double *poses3, int scans,
+                           double angle_min, double angle_increment, int beams, double far_range,
+                           const double *beam_cs, double *ranges, double *tar_xy, void *stream);
 
 /* Sum of per-GPU count deltas (no reference counterpart: the reference is single-process).
  * In-place ncclAllReduce(int32, sum) of both planes on an existing communicator. */
@@ -305,6 +315,20 @@ int b2s_icp_submit_sequence(b2s_icp *icp, const void *scans_xy, int is_f64, int 
 int b2s_icp_submit_scans(b2s_icp *icp, const float *ranges, const double *beam_cs, double clamp_inf_to, int scans, int n,
                          int max_iter, double tol, double *T_out, int32_t *iters_out, int *ticket_out);
 int b2s_icp_wait(b2s_icp *icp, int ticket);
+/* The static map of the localization node (self.obstacle): obstacle cell centres, uploaded once and kept on the
+ * device until replaced.  count == 0 clears it.  A NaN coordinate is rejected (B2S_ERR_NONFINITE, the map is then
+ * cleared): the reference's int() raises on it.  +-inf coordinates are kept; they never win a bin. */
+int b2s_icp_set_map(b2s_icp *icp, const double *obs_x, const double *obs_y, int count);
+/* calc_map_observation ([LOC9]:152-157) for a recorded stream: for scan k, target = laserToNumpy(virtual scan of the
+ * map at poses3[k]), source = laserToNumpy(ranges[k]) (clamp_inf_to > 0: the W12 inf clamp), T_out[k] =
+ * ICP.process(target, source).  beam_cs [n][2] = cos, sin of linspace(angle_min, angle_max, n); the virtual scan bins
+ * with angle_min / angle_increment.  virtual_out [scans][n] (may be NULL) receives the virtual ranges, iters_out
+ * [scans] (may be NULL) the iteration counts.  A NaN pose fails with B2S_ERR_NONFINITE before anything runs; no map
+ * set is B2S_ERR_INVALID_ARG.  Same transforms as b2s_icp_process on the float64 point pairs, bit for bit. */
+int b2s_icp_map_observation(b2s_icp *icp, const float *ranges, const double *poses3, const double *beam_cs,
+                            double clamp_inf_to, int scans, int n, double angle_min, double angle_increment,
+                            double far_range, int max_iter, double tol, double *T_out, int32_t *iters_out,
+                            double *virtual_out);
 int b2s_icp_find_nearest(b2s_icp *icp, const double *src_xy, int n, const double *tar_xy, int m,
                          double *dist_out, int64_t *idx_out);
 int b2s_icp_get_transform(b2s_icp *icp, const double *src_xy, const double *tar_xy, int n,
