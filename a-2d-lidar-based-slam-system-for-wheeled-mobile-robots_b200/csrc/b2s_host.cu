@@ -150,38 +150,76 @@ struct Trace {
     }
 };
 
+// The streams and events of an object's chunked pipeline, shared by ICP and Mapping.  stream: everything ordered and
+// the blocking calls' read-back; stream2: every other chunk's compute, so that the ragged end of one chunk (ICP pairs
+// need 2..max_iter iterations, beams differ in length) overlaps the next chunk instead of idling the device;
+// copy_stream: H2D, chunk k followed by chunk_ready[k]; d2h_stream: the streaming calls' read-back, after `handoff` on
+// stream.  Slot: one streaming call in flight, with inputs_free (its inputs may be overwritten) and done (its
+// results are on the host).
+template <class Slot>
+struct StreamSet {
+    cudaStream_t stream = nullptr, stream2 = nullptr, copy_stream = nullptr, d2h_stream = nullptr;
+    cudaEvent_t chunk_ready[MAX_CHUNKS] = {}, joined = nullptr, handoff = nullptr;
+    Slot slot[2];
+
+    cudaError_t create()
+    {
+        cudaStream_t *streams[] = {&stream, &stream2, &copy_stream, &d2h_stream};
+        cudaEvent_t *events[] = {&joined, &handoff, &slot[0].inputs_free, &slot[0].done, &slot[1].inputs_free, &slot[1].done};
+        cudaError_t e = cudaSuccess;
+        for (cudaStream_t *s : streams)
+            if (e == cudaSuccess) e = cudaStreamCreateWithFlags(s, cudaStreamNonBlocking);
+        for (cudaEvent_t *ev : events)
+            if (e == cudaSuccess) e = cudaEventCreateWithFlags(ev, cudaEventDisableTiming);
+        for (cudaEvent_t &ev : chunk_ready)
+            if (e == cudaSuccess) e = cudaEventCreateWithFlags(&ev, cudaEventDisableTiming);
+        return e;
+    }
+    // Waits for all four streams, lets the owner free its buffers, then destroys the handles.
+    template <class FreeBuffers>
+    void teardown(FreeBuffers free_buffers)
+    {
+        cudaStream_t streams[] = {stream, stream2, copy_stream, d2h_stream};
+        for (cudaStream_t s : streams)
+            if (s) cudaStreamSynchronize(s);
+        free_buffers();
+        cudaEvent_t events[] = {joined, handoff, slot[0].inputs_free, slot[0].done, slot[1].inputs_free, slot[1].done};
+        for (cudaEvent_t ev : events)
+            if (ev) cudaEventDestroy(ev);
+        for (cudaEvent_t ev : chunk_ready)
+            if (ev) cudaEventDestroy(ev);
+        for (cudaStream_t s : streams)
+            if (s) cudaStreamDestroy(s);
+    }
+};
+
 }  // namespace b2s
 
 using namespace b2s;
 
-struct b2s_icp {
-    int device;
-    // stream: results / read-back; stream2: every other chunk's solve, so that the long-tail CTAs of one chunk (pairs
-    // need 2..max_iter iterations) overlap the next chunk instead of idling the device; copy_stream: H2D
-    cudaStream_t stream, stream2, copy_stream;
-    cudaEvent_t chunk_ready[MAX_CHUNKS], joined;
+// Streaming sequence calls (b2s_icp_submit_sequence / _scans, b2s_icp_wait): two slots of device buffers, so the
+// scans of call k + 1 cross PCIe while call k is being solved and its transforms are read back.
+struct IcpSlot {
+    Buf d_scans, d_T, d_iters, d_cs;
+    cudaEvent_t inputs_free = nullptr, done = nullptr;
+    bool in_flight = false;
+    int ticket = 0;
+};
+
+struct b2s_icp : StreamSet<IcpSlot> {
+    int device = 0;
     Buf d_tar, d_src, d_T, d_iters, d_aux;
     // The per-scan call of the ROS node (ICP.process: ONE pair) is launch-bound, so its device work -- two uploads,
     // the solve, two read-backs -- is captured once into a CUDA graph and replayed with one launch.  The graph is
     // tied to the sizes, parameters and buffer addresses below and re-captured when any of them changes.
-    Buf h_one;  // pinned staging: [tar][src][T (9 doubles)][iterations]
-    cudaGraphExec_t one_exec;
+    Buf h_one = {nullptr, 0, true};  // pinned staging: [tar][src][T (9 doubles)][iterations]
+    cudaGraphExec_t one_exec = nullptr;
     struct {
         int is_f64, n_src, n_tar, max_iter, tune_gen;
         double tol;
         void *d_tar, *d_src, *d_T, *d_iters, *h;
-    } one_key;
-    // Streaming sequence calls (b2s_icp_submit_sequence / _scans, b2s_icp_wait): two slots of device buffers, so the
-    // scans of call k + 1 cross PCIe while call k is being solved and its transforms are read back.
-    struct Slot {
-        Buf d_scans, d_T, d_iters, d_cs;
-        cudaEvent_t inputs_free, done;
-        bool in_flight;
-        int ticket;
-    } slot[2];
-    cudaStream_t d2h_stream;
-    cudaEvent_t solved;
-    int submitted;
+    } one_key = {};
+    int submitted = 0;
     // Map observation (b2s_icp_set_map / b2s_icp_map_observation): the static map obs_x | obs_y, kept until replaced;
     // the call's uploads (beam table | poses | ranges), and the target (+ virtual ranges) and source clouds it builds.
     Buf d_map, d_map_in, d_map_tar, d_map_src;
@@ -264,15 +302,24 @@ struct DeviceBatch {
 };
 }  // namespace
 
-struct b2s_mapping {
+// Streaming calls (b2s_mapping_submit* / b2s_mapping_wait): two slots of everything a step owns, so that step k + 1
+// can be uploaded and ray-cast while the map of step k is still on its way back to the host.
+struct MappingSlot {
+    Buf d_in, d_map, h_pose = {nullptr, 0, true};  // device inputs, device copy of this step's occupancy, pinned pose table
+    int32_t *d_cnt = nullptr, *h_cnt = nullptr;     // the ray-cast's B2S_CNT_* words of this step (device / pinned host)
+    cudaEvent_t inputs_free = nullptr, done = nullptr;  // last ray-cast of the step enqueued / results on the host
+    bool in_flight = false;
+    int ticket = 0;
+    DeviceBatch batch;                              // the step's inputs in d_in
+};
+
+// stream carries the zeroing, the last chunk with its fold, the finalize and the blocking read-back.
+struct b2s_mapping : StreamSet<MappingSlot> {
     int device;
     int xw, yw;
     double xyreso, cells_per_m, off_x, off_y;
     double w_hit, w_miss, thresh;
-    // stream: everything ordered (zeroing, last chunk + fold, finalize, read-back); stream2: every other ray-cast
-    // chunk, so the ragged end of one chunk (beams differ in length) overlaps the next; copy_stream: H2D
-    cudaStream_t stream = nullptr, stream2 = nullptr, copy_stream = nullptr;
-    cudaEvent_t chunk_ready[MAX_CHUNKS] = {}, begun = nullptr, joined = nullptr;
+    cudaEvent_t begun = nullptr;
     int32_t *hit = nullptr, *miss = nullptr;
     int32_t *counters = nullptr;
     void *workspace = nullptr;
@@ -281,18 +328,6 @@ struct b2s_mapping {
     bool pmap_valid = false;  // d_pmap holds the occupancy of the current counts
     int8_t *h_packed = nullptr;  // pinned staging for the dirty tiles
     int32_t *h_ids = nullptr;
-    // Streaming calls (b2s_mapping_submit* / b2s_mapping_wait): two slots of everything a step owns, so that step
-    // k + 1 can be uploaded and ray-cast while the map of step k is still on its way back to the host.
-    struct Slot {
-        Buf d_in, d_map, h_pose = {nullptr, 0, true};  // device inputs, device copy of this step's occupancy, pinned pose table
-        int32_t *d_cnt = nullptr, *h_cnt = nullptr;     // the ray-cast's B2S_CNT_* words of this step (device / pinned host)
-        cudaEvent_t inputs_free = nullptr, done = nullptr;  // last ray-cast of the step enqueued / results on the host
-        bool in_flight = false;
-        int ticket = 0;
-        DeviceBatch batch;                              // the step's inputs in d_in
-    } slot[2];
-    cudaStream_t d2h_stream = nullptr;
-    cudaEvent_t finalized = nullptr;
     int submitted = 0;
 };
 
@@ -421,28 +456,7 @@ extern "C" int b2s_icp_create(b2s_icp **out, int device)
     b2s_icp *c = new (std::nothrow) b2s_icp();
     if (!c) return B2S_ERR_NOMEM;
     c->device = device;
-    c->stream = c->stream2 = c->copy_stream = c->d2h_stream = nullptr;
-    c->joined = c->solved = nullptr;
-    c->submitted = 0;
-    for (int k = 0; k < 2; ++k) {
-        c->slot[k].inputs_free = c->slot[k].done = nullptr;
-        c->slot[k].in_flight = false;
-    }
-    c->one_exec = nullptr;
-    memset(&c->one_key, 0, sizeof(c->one_key));
-    c->h_one.pinned = true;
-    for (int k = 0; k < MAX_CHUNKS; ++k) c->chunk_ready[k] = nullptr;
-    cudaError_t e = cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking);
-    if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&c->stream2, cudaStreamNonBlocking);
-    if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&c->copy_stream, cudaStreamNonBlocking);
-    if (e == cudaSuccess) e = cudaEventCreateWithFlags(&c->joined, cudaEventDisableTiming);
-    if (e == cudaSuccess) e = cudaEventCreateWithFlags(&c->solved, cudaEventDisableTiming);
-    if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&c->d2h_stream, cudaStreamNonBlocking);
-    for (int k = 0; k < 2 && e == cudaSuccess; ++k) {
-        e = cudaEventCreateWithFlags(&c->slot[k].inputs_free, cudaEventDisableTiming);
-        if (e == cudaSuccess) e = cudaEventCreateWithFlags(&c->slot[k].done, cudaEventDisableTiming);
-    }
-    for (int k = 0; k < MAX_CHUNKS && e == cudaSuccess; ++k) e = cudaEventCreateWithFlags(&c->chunk_ready[k], cudaEventDisableTiming);
+    cudaError_t e = c->create();
     if (e != cudaSuccess) {
         int rc = cuda_fail(e, "b2s_icp_create");
         b2s_icp_destroy(c);
@@ -456,28 +470,15 @@ extern "C" int b2s_icp_destroy(b2s_icp *c)
 {
     if (!c) return B2S_OK;
     DeviceGuard g(c->device);
-    if (c->stream) cudaStreamSynchronize(c->stream);
-    if (c->stream2) cudaStreamSynchronize(c->stream2);
-    if (c->copy_stream) cudaStreamSynchronize(c->copy_stream);
-    if (c->one_exec) cudaGraphExecDestroy(c->one_exec);
-    c->d_tar.release(); c->d_src.release(); c->d_T.release(); c->d_iters.release(); c->d_aux.release();
-    c->h_one.release();
-    if (c->d2h_stream) cudaStreamSynchronize(c->d2h_stream);
-    for (int k = 0; k < 2; ++k) {
-        b2s_icp::Slot &sl = c->slot[k];
-        sl.d_scans.release(); sl.d_T.release(); sl.d_iters.release(); sl.d_cs.release();
-        if (sl.inputs_free) cudaEventDestroy(sl.inputs_free);
-        if (sl.done) cudaEventDestroy(sl.done);
-    }
-    c->d_map.release(); c->d_map_in.release(); c->d_map_tar.release(); c->d_map_src.release();
-    if (c->solved) cudaEventDestroy(c->solved);
-    if (c->d2h_stream) cudaStreamDestroy(c->d2h_stream);
-    for (int k = 0; k < MAX_CHUNKS; ++k)
-        if (c->chunk_ready[k]) cudaEventDestroy(c->chunk_ready[k]);
-    if (c->joined) cudaEventDestroy(c->joined);
-    if (c->copy_stream) cudaStreamDestroy(c->copy_stream);
-    if (c->stream2) cudaStreamDestroy(c->stream2);
-    if (c->stream) cudaStreamDestroy(c->stream);
+    c->teardown([c] {
+        if (c->one_exec) cudaGraphExecDestroy(c->one_exec);
+        c->d_tar.release(); c->d_src.release(); c->d_T.release(); c->d_iters.release(); c->d_aux.release();
+        c->h_one.release();
+        for (IcpSlot &sl : c->slot) {
+            sl.d_scans.release(); sl.d_T.release(); sl.d_iters.release(); sl.d_cs.release();
+        }
+        c->d_map.release(); c->d_map_in.release(); c->d_map_tar.release(); c->d_map_src.release();
+    });
     delete c;
     return B2S_OK;
 }
@@ -546,6 +547,47 @@ static int icp_process_one_graph(b2s_icp *c, const void *tar_xy, const void *src
     return B2S_OK;
 }
 
+// The chunked pipeline of the ICP calls: `units` (pairs or scans) cut into nchunk chunks.  All uploads
+// upload(k, u0, u1, stream) of chunks k = [u0, u1) are enqueued on the copy stream first, so that chunk k + 1 crosses
+// PCIe while chunk k is solved; then solve(k, u0, u1, stream) of each chunk, alternating between stream and stream2.
+// Everything after it (read-back, pose chain) is ordered on c->stream.
+template <class Upload, class Solve>
+static int icp_pipeline(b2s_icp *c, Trace &tr, int units, int nchunk, Upload upload, Solve solve)
+{
+    int rc;
+    for (int k = 0; k < nchunk; ++k) {
+        if ((rc = upload(k, (size_t)units * k / nchunk, (size_t)units * (k + 1) / nchunk, c->copy_stream))) return rc;
+        B2S_CUDA(cudaEventRecord(c->chunk_ready[k], c->copy_stream));
+        tr.mark("h2d chunk done", k, c->copy_stream);
+    }
+    for (int k = 0; k < nchunk; ++k) {
+        cudaStream_t ks = (k & 1) ? c->stream2 : c->stream;
+        B2S_CUDA(cudaStreamWaitEvent(ks, c->chunk_ready[k], 0));
+        if ((rc = solve(k, (size_t)units * k / nchunk, (size_t)units * (k + 1) / nchunk, ks))) return rc;
+        tr.mark("icp chunk done", k, ks);
+    }
+    if (nchunk > 1) {
+        B2S_CUDA(cudaEventRecord(c->joined, c->stream2));
+        B2S_CUDA(cudaStreamWaitEvent(c->stream, c->joined, 0));
+    }
+    return B2S_OK;
+}
+
+// The ending of the blocking ICP calls: the transforms and iteration counts of `pairs` pairs from c->d_T / c->d_iters
+// (T_out / iters_out may be NULL), then the synchronize of c->stream.
+static int icp_read_back(b2s_icp *c, Trace &tr, int pairs, double *T_out, int32_t *iters_out)
+{
+    if (T_out && pairs > 0)
+        B2S_CUDA(cudaMemcpyAsync(T_out, c->d_T.p, (size_t)pairs * 9 * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
+    if (iters_out && pairs > 0)
+        B2S_CUDA(cudaMemcpyAsync(iters_out, c->d_iters.p, (size_t)pairs * sizeof(int32_t), cudaMemcpyDeviceToHost,
+                                 c->stream));
+    tr.mark("results d2h done", 0, c->stream);
+    B2S_CUDA(cudaStreamSynchronize(c->stream));
+    tr.mark("synchronized", 0, nullptr);
+    return B2S_OK;
+}
+
 extern "C" int b2s_icp_process(b2s_icp *c, const void *tar_xy, const void *src_xy, int is_f64,
                                int pairs, int n_src, int n_tar, int max_iter, double tol,
                                double *T_out, int32_t *iters_out)
@@ -565,46 +607,28 @@ extern "C" int b2s_icp_process(b2s_icp *c, const void *tar_xy, const void *src_x
     if ((rc = c->d_src.reserve(sb))) return rc;
     if ((rc = c->d_T.reserve((size_t)pairs * 9 * sizeof(double)))) return rc;
     if ((rc = c->d_iters.reserve((size_t)pairs * sizeof(int32_t)))) return rc;
-    // Pipeline: up to 8 chunks of pairs; chunk k+1 crosses PCIe on the copy stream while chunk k is solved.
     const int nchunk = pipeline_chunks((int)((tb + sb + (16u << 20) - 1) / (16u << 20)), 8, pairs);  // ~16 MB of points per chunk (measured best)
     const size_t tpair = (size_t)2 * n_tar * el, spair = (size_t)2 * n_src * el;
+    char *d_tar = (char *)c->d_tar.p, *d_src = (char *)c->d_src.p;
     // (every call ends with a synchronize, so the device input buffers are free to overwrite here)
-    for (int k = 0; k < nchunk; ++k) {
-        const size_t p0 = (size_t)pairs * k / nchunk, p1 = (size_t)pairs * (k + 1) / nchunk;
-        B2S_CUDA(cudaMemcpyAsync((char *)c->d_tar.p + p0 * tpair, (const char *)tar_xy + p0 * tpair, (p1 - p0) * tpair,
-                                 cudaMemcpyHostToDevice, c->copy_stream));
-        B2S_CUDA(cudaMemcpyAsync((char *)c->d_src.p + p0 * spair, (const char *)src_xy + p0 * spair, (p1 - p0) * spair,
-                                 cudaMemcpyHostToDevice, c->copy_stream));
-        B2S_CUDA(cudaEventRecord(c->chunk_ready[k], c->copy_stream));
-        tr.mark("h2d chunk done", k, c->copy_stream);
-    }
-    for (int k = 0; k < nchunk; ++k) {
-        const size_t p0 = (size_t)pairs * k / nchunk, p1 = (size_t)pairs * (k + 1) / nchunk;
-        cudaStream_t ks = (k & 1) ? c->stream2 : c->stream;
-        B2S_CUDA(cudaStreamWaitEvent(ks, c->chunk_ready[k], 0));
+    auto upload = [&](int, size_t p0, size_t p1, cudaStream_t st) -> int {
+        B2S_CUDA(cudaMemcpyAsync(d_tar + p0 * tpair, (const char *)tar_xy + p0 * tpair, (p1 - p0) * tpair,
+                                 cudaMemcpyHostToDevice, st));
+        B2S_CUDA(cudaMemcpyAsync(d_src + p0 * spair, (const char *)src_xy + p0 * spair, (p1 - p0) * spair,
+                                 cudaMemcpyHostToDevice, st));
+        return B2S_OK;
+    };
+    auto solve = [&](int, size_t p0, size_t p1, cudaStream_t ks) {
         double *dT = (double *)c->d_T.p + p0 * 9;
         int32_t *dI = (int32_t *)c->d_iters.p + p0;
         if (is_f64)
-            rc = b2s_icp_batch_f64((const double *)((char *)c->d_tar.p + p0 * tpair), (const double *)((char *)c->d_src.p + p0 * spair),
-                                   (int)(p1 - p0), n_src, n_tar, max_iter, tol, dT, dI, ks);
-        else
-            rc = b2s_icp_batch_f32((const float *)((char *)c->d_tar.p + p0 * tpair), (const float *)((char *)c->d_src.p + p0 * spair),
-                                   (int)(p1 - p0), n_src, n_tar, max_iter, tol, dT, dI, ks);
-        if (rc) return rc;
-        tr.mark("icp chunk done", k, ks);
-    }
-    if (nchunk > 1) {
-        B2S_CUDA(cudaEventRecord(c->joined, c->stream2));
-        B2S_CUDA(cudaStreamWaitEvent(c->stream, c->joined, 0));
-    }
-    B2S_CUDA(cudaMemcpyAsync(T_out, c->d_T.p, (size_t)pairs * 9 * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
-    if (iters_out)
-        B2S_CUDA(cudaMemcpyAsync(iters_out, c->d_iters.p, (size_t)pairs * sizeof(int32_t), cudaMemcpyDeviceToHost,
-                                 c->stream));
-    tr.mark("results d2h done", 0, c->stream);
-    B2S_CUDA(cudaStreamSynchronize(c->stream));
-    tr.mark("synchronized", 0, nullptr);
-    return B2S_OK;
+            return b2s_icp_batch_f64((const double *)(d_tar + p0 * tpair), (const double *)(d_src + p0 * spair), (int)(p1 - p0),
+                                     n_src, n_tar, max_iter, tol, dT, dI, ks);
+        return b2s_icp_batch_f32((const float *)(d_tar + p0 * tpair), (const float *)(d_src + p0 * spair), (int)(p1 - p0),
+                                 n_src, n_tar, max_iter, tol, dT, dI, ks);
+    };
+    if ((rc = icp_pipeline(c, tr, pairs, nchunk, upload, solve))) return rc;
+    return icp_read_back(c, tr, pairs, T_out, iters_out);
 }
 
 // LiDAR odometry over a scan sequence ([LOC9]:159-168, [SLAM]:109-113: the target of pair k is scan k, the source
@@ -634,42 +658,31 @@ static int icp_sequence_enqueue(b2s_icp *c, Trace &tr, const void *scans_xy, int
     if (beam_cs && want < 4 && pairs >= 4096) want = 4;  // (raw scans are half the bytes: keep the pipeline depth)
     if (force_chunks > 0) want = force_chunks;
     const int nchunk = pipeline_chunks(want, 8, pairs);
+    char *d_scans = (char *)bufs.scans.p;
     // chunk k solves pairs [p0, p1) and therefore needs scans [p0, p1]; scan p0 arrived with the previous chunk
-    for (int k = 0; k < nchunk; ++k) {
-        const size_t p0 = (size_t)pairs * k / nchunk, p1 = (size_t)pairs * (k + 1) / nchunk;
-        const size_t s0 = k == 0 ? 0 : p0 + 1, s1 = p1 + 1;
-        B2S_CUDA(cudaMemcpyAsync((char *)bufs.scans.p + s0 * scan_bytes, (const char *)scans_xy + s0 * scan_bytes,
-                                 (s1 - s0) * scan_bytes, cudaMemcpyHostToDevice, c->copy_stream));
-        B2S_CUDA(cudaEventRecord(c->chunk_ready[k], c->copy_stream));
-        tr.mark("h2d chunk done", k, c->copy_stream);
-    }
-    for (int k = 0; k < nchunk; ++k) {
-        const size_t p0 = (size_t)pairs * k / nchunk, p1 = (size_t)pairs * (k + 1) / nchunk;
-        cudaStream_t ks = (k & 1) ? c->stream2 : c->stream;
-        B2S_CUDA(cudaStreamWaitEvent(ks, c->chunk_ready[k], 0));
-        const char *tar = (const char *)bufs.scans.p + p0 * scan_bytes;
+    auto upload = [&](int k, size_t p0, size_t p1, cudaStream_t st) -> int {
+        const size_t s0 = k == 0 ? 0 : p0 + 1;
+        B2S_CUDA(cudaMemcpyAsync(d_scans + s0 * scan_bytes, (const char *)scans_xy + s0 * scan_bytes, (p1 + 1 - s0) * scan_bytes,
+                                 cudaMemcpyHostToDevice, st));
+        return B2S_OK;
+    };
+    auto solve = [&](int, size_t p0, size_t p1, cudaStream_t ks) {
+        const char *tar = d_scans + p0 * scan_bytes;
         double *dT = (double *)bufs.T.p + p0 * 9;
         int32_t *dI = (int32_t *)bufs.iters.p + p0;
         if (beam_cs)
-            rc = b2s_icp_batch_ranges((const float *)tar, (const float *)(tar + scan_bytes), (const double *)bufs.cs.p, clamp,
-                                      (int)(p1 - p0), n, max_iter, tol, dT, dI, ks);
-        else if (is_f64)
-            rc = b2s_icp_batch_f64((const double *)tar, (const double *)(tar + scan_bytes), (int)(p1 - p0), n, n, max_iter, tol,
-                                   dT, dI, ks);
-        else
-            rc = b2s_icp_batch_f32((const float *)tar, (const float *)(tar + scan_bytes), (int)(p1 - p0), n, n, max_iter, tol,
-                                   dT, dI, ks);
-        if (rc) return rc;
-        tr.mark("icp chunk done", k, ks);
-    }
-    if (nchunk > 1) {  // everything downstream (read-back, pose chain) is ordered on c->stream
-        B2S_CUDA(cudaEventRecord(c->joined, c->stream2));
-        B2S_CUDA(cudaStreamWaitEvent(c->stream, c->joined, 0));
-    }
-    return B2S_OK;
+            return b2s_icp_batch_ranges((const float *)tar, (const float *)(tar + scan_bytes), (const double *)bufs.cs.p, clamp,
+                                        (int)(p1 - p0), n, max_iter, tol, dT, dI, ks);
+        if (is_f64)
+            return b2s_icp_batch_f64((const double *)tar, (const double *)(tar + scan_bytes), (int)(p1 - p0), n, n, max_iter, tol,
+                                     dT, dI, ks);
+        return b2s_icp_batch_f32((const float *)tar, (const float *)(tar + scan_bytes), (int)(p1 - p0), n, n, max_iter, tol,
+                                 dT, dI, ks);
+    };
+    return icp_pipeline(c, tr, pairs, nchunk, upload, solve);
 }
 
-// Read-back shared by the sequence calls: optional pose chain, then trajectory / transforms / iteration counts.
+// Ending of the blocking sequence calls: optional pose chain and trajectory, then transforms and iteration counts.
 static int icp_sequence_finish(b2s_icp *c, Trace &tr, int scans, const double *state, double *traj_out, double *T_out,
                                int32_t *iters_out)
 {
@@ -682,15 +695,7 @@ static int icp_sequence_finish(b2s_icp *c, Trace &tr, int scans, const double *s
         tr.mark("pose chain done", 0, c->stream);
         B2S_CUDA(cudaMemcpyAsync(traj_out, c->d_aux.p, (size_t)scans * 3 * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
     }
-    if (T_out && pairs > 0)
-        B2S_CUDA(cudaMemcpyAsync(T_out, c->d_T.p, (size_t)pairs * 9 * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
-    if (iters_out && pairs > 0)
-        B2S_CUDA(cudaMemcpyAsync(iters_out, c->d_iters.p, (size_t)pairs * sizeof(int32_t), cudaMemcpyDeviceToHost,
-                                 c->stream));
-    tr.mark("results d2h done", 0, c->stream);
-    B2S_CUDA(cudaStreamSynchronize(c->stream));
-    tr.mark("synchronized", 0, nullptr);
-    return B2S_OK;
+    return icp_read_back(c, tr, pairs, T_out, iters_out);
 }
 
 extern "C" int b2s_icp_process_sequence(b2s_icp *c, const void *scans_xy, int is_f64, int scans, int n,
@@ -757,8 +762,8 @@ static int icp_submit(b2s_icp *c, const void *scans_data, int is_f64, const doub
 {
     DeviceGuard g(c->device);
     const int ticket = c->submitted;
-    b2s_icp::Slot &sl = c->slot[ticket & 1];
-    b2s_icp::Slot &other = c->slot[(ticket & 1) ^ 1];
+    IcpSlot &sl = c->slot[ticket & 1];
+    IcpSlot &other = c->slot[(ticket & 1) ^ 1];
     if (sl.in_flight) {
         B2S_CUDA(cudaEventSynchronize(sl.done));
         sl.in_flight = false;
@@ -773,8 +778,8 @@ static int icp_submit(b2s_icp *c, const void *scans_data, int is_f64, const doub
                                                 other.in_flight ? 2 : 0)))
         return rc;
     B2S_CUDA(cudaEventRecord(sl.inputs_free, c->stream));
-    B2S_CUDA(cudaEventRecord(c->solved, c->stream));
-    B2S_CUDA(cudaStreamWaitEvent(c->d2h_stream, c->solved, 0));
+    B2S_CUDA(cudaEventRecord(c->handoff, c->stream));
+    B2S_CUDA(cudaStreamWaitEvent(c->d2h_stream, c->handoff, 0));
     if (pairs > 0) {
         B2S_CUDA(cudaMemcpyAsync(T_out, sl.d_T.p, (size_t)pairs * 9 * sizeof(double), cudaMemcpyDeviceToHost, c->d2h_stream));
         if (iters_out)
@@ -812,7 +817,7 @@ extern "C" int b2s_icp_wait(b2s_icp *c, int ticket)
     B2S_REQUIRE(c, "b2s_icp_wait: null handle");
     B2S_REQUIRE(ticket >= 0 && ticket < c->submitted, "b2s_icp_wait: unknown ticket");
     DeviceGuard g(c->device);
-    b2s_icp::Slot &sl = c->slot[ticket & 1];
+    IcpSlot &sl = c->slot[ticket & 1];
     if (!sl.in_flight || sl.ticket != ticket) return B2S_OK;
     B2S_CUDA(cudaEventSynchronize(sl.done));
     sl.in_flight = false;
@@ -843,9 +848,8 @@ extern "C" int b2s_icp_set_map(b2s_icp *c, const double *obs_x, const double *ob
     return B2S_OK;
 }
 
-// The pipeline of icp_sequence_enqueue: the ranges and poses of chunk k + 1 cross PCIe on the copy stream while chunk k
-// is solved, and the chunks alternate between stream and stream2.  Per chunk: the virtual scans straight into the
-// target layout, laserToNumpy of the ranges into the source layout, then the float64 ICP on the two.
+// The ranges and poses go through icp_pipeline.  Per chunk: the virtual scans straight into the target layout,
+// laserToNumpy of the ranges into the source layout, then the float64 ICP on the two.
 extern "C" int b2s_icp_map_observation(b2s_icp *c, const float *ranges, const double *poses3, const double *beam_cs,
                                        double clamp_inf_to, int scans, int n, double angle_min, double angle_increment,
                                        double far_range, int max_iter, double tol, double *T_out, int32_t *iters_out,
@@ -888,44 +892,28 @@ extern "C" int b2s_icp_map_observation(b2s_icp *c, const float *ranges, const do
     if (want < (scans + 2499) / 2500) want = (scans + 2499) / 2500;
     const int nchunk = pipeline_chunks(want, 8, scans);
     B2S_CUDA(cudaMemcpyAsync(in, beam_cs, cs_bytes, cudaMemcpyHostToDevice, c->copy_stream));
-    for (int k = 0; k < nchunk; ++k) {
-        const size_t s0 = (size_t)scans * k / nchunk, s1 = (size_t)scans * (k + 1) / nchunk;
+    auto upload = [&](int, size_t s0, size_t s1, cudaStream_t st) -> int {
         B2S_CUDA(cudaMemcpyAsync(in + pose_off + s0 * 3 * sizeof(double), poses3 + s0 * 3, (s1 - s0) * 3 * sizeof(double),
-                                 cudaMemcpyHostToDevice, c->copy_stream));
+                                 cudaMemcpyHostToDevice, st));
         B2S_CUDA(cudaMemcpyAsync(in + range_off + s0 * n * sizeof(float), ranges + s0 * n, (s1 - s0) * n * sizeof(float),
-                                 cudaMemcpyHostToDevice, c->copy_stream));
-        B2S_CUDA(cudaEventRecord(c->chunk_ready[k], c->copy_stream));
-        tr.mark("h2d chunk done", k, c->copy_stream);
-    }
-    for (int k = 0; k < nchunk; ++k) {
-        const size_t s0 = (size_t)scans * k / nchunk, s1 = (size_t)scans * (k + 1) / nchunk;
+                                 cudaMemcpyHostToDevice, st));
+        return B2S_OK;
+    };
+    auto solve = [&](int k, size_t s0, size_t s1, cudaStream_t ks) {
         const int ns = (int)(s1 - s0);
-        cudaStream_t ks = (k & 1) ? c->stream2 : c->stream;
-        B2S_CUDA(cudaStreamWaitEvent(ks, c->chunk_ready[k], 0));
         double *tar = d_tar + s0 * 2 * n, *src = d_src + s0 * 2 * n;
         if ((rc = b2s_virtual_scan_batch(map_x, map_y, c->map_count, d_pose + s0 * 3, ns, angle_min, angle_increment, n,
                                          far_range, d_cs, d_virt ? d_virt + s0 * n : nullptr, tar, ks)))
             return rc;
         tr.mark("virtual scan chunk done", k, ks);
         if ((rc = laser_points(d_ranges + s0 * n, d_cs, clamp_inf_to, ns, n, src, ks))) return rc;
-        if ((rc = b2s_icp_batch_f64(tar, src, ns, n, n, max_iter, tol, (double *)c->d_T.p + s0 * 9,
-                                    (int32_t *)c->d_iters.p + s0, ks)))
-            return rc;
-        tr.mark("icp chunk done", k, ks);
-    }
-    if (nchunk > 1) {
-        B2S_CUDA(cudaEventRecord(c->joined, c->stream2));
-        B2S_CUDA(cudaStreamWaitEvent(c->stream, c->joined, 0));
-    }
-    B2S_CUDA(cudaMemcpyAsync(T_out, c->d_T.p, (size_t)scans * 9 * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
-    if (iters_out)
-        B2S_CUDA(cudaMemcpyAsync(iters_out, c->d_iters.p, (size_t)scans * sizeof(int32_t), cudaMemcpyDeviceToHost, c->stream));
+        return b2s_icp_batch_f64(tar, src, ns, n, n, max_iter, tol, (double *)c->d_T.p + s0 * 9,
+                                 (int32_t *)c->d_iters.p + s0, ks);
+    };
+    if ((rc = icp_pipeline(c, tr, scans, nchunk, upload, solve))) return rc;
     if (virtual_out)
         B2S_CUDA(cudaMemcpyAsync(virtual_out, d_virt, (size_t)scans * n * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
-    tr.mark("results d2h done", 0, c->stream);
-    B2S_CUDA(cudaStreamSynchronize(c->stream));
-    tr.mark("synchronized", 0, nullptr);
-    return B2S_OK;
+    return icp_read_back(c, tr, scans, T_out, iters_out);
 }
 
 extern "C" int b2s_icp_find_nearest(b2s_icp *c, const double *src_xy, int n, const double *tar_xy,
@@ -1003,19 +991,11 @@ extern "C" int b2s_mapping_create(b2s_mapping **out, int xw, int yw, double xyre
     m->w_miss = w_miss;
     m->thresh = thresh;
     const size_t plane = (size_t)xw * yw * sizeof(int32_t);
-    cudaError_t e = cudaStreamCreateWithFlags(&m->stream, cudaStreamNonBlocking);
-    if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&m->stream2, cudaStreamNonBlocking);
-    if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&m->copy_stream, cudaStreamNonBlocking);
-    for (int k = 0; k < MAX_CHUNKS && e == cudaSuccess; ++k) e = cudaEventCreateWithFlags(&m->chunk_ready[k], cudaEventDisableTiming);
+    cudaError_t e = m->create();
     if (e == cudaSuccess) e = cudaEventCreateWithFlags(&m->begun, cudaEventDisableTiming);
-    if (e == cudaSuccess) e = cudaEventCreateWithFlags(&m->joined, cudaEventDisableTiming);
-    if (e == cudaSuccess) e = cudaEventCreateWithFlags(&m->finalized, cudaEventDisableTiming);
-    if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&m->d2h_stream, cudaStreamNonBlocking);
-    for (int k = 0; k < 2 && e == cudaSuccess; ++k) {
-        e = cudaEventCreateWithFlags(&m->slot[k].inputs_free, cudaEventDisableTiming);
-        if (e == cudaSuccess) e = cudaEventCreateWithFlags(&m->slot[k].done, cudaEventDisableTiming);
-        if (e == cudaSuccess) e = cudaMalloc((void **)&m->slot[k].d_cnt, B2S_CNT_WORDS * sizeof(int32_t));
-        if (e == cudaSuccess) e = cudaMallocHost((void **)&m->slot[k].h_cnt, B2S_CNT_WORDS * sizeof(int32_t));
+    for (MappingSlot &sl : m->slot) {
+        if (e == cudaSuccess) e = cudaMalloc((void **)&sl.d_cnt, B2S_CNT_WORDS * sizeof(int32_t));
+        if (e == cudaSuccess) e = cudaMallocHost((void **)&sl.h_cnt, B2S_CNT_WORDS * sizeof(int32_t));
     }
     if (e == cudaSuccess) e = cudaMalloc((void **)&m->hit, plane);
     if (e == cudaSuccess) e = cudaMalloc((void **)&m->miss, plane);
@@ -1039,35 +1019,23 @@ extern "C" int b2s_mapping_destroy(b2s_mapping *m)
 {
     if (!m) return B2S_OK;
     DeviceGuard g(m->device);
-    if (m->stream) cudaStreamSynchronize(m->stream);
-    if (m->stream2) cudaStreamSynchronize(m->stream2);
-    if (m->hit) cudaFree(m->hit);
-    if (m->miss) cudaFree(m->miss);
-    if (m->counters) cudaFree(m->counters);
-    if (m->workspace) cudaFree(m->workspace);
-    if (m->h_packed) cudaFreeHost(m->h_packed);
-    if (m->h_ids) cudaFreeHost(m->h_ids);
-    m->d_packed.release();
-    m->d_in.release(); m->d_datamap.release(); m->d_pmap.release();
-    m->h_pose.release();
-    if (m->d2h_stream) cudaStreamSynchronize(m->d2h_stream);
-    for (int k = 0; k < 2; ++k) {
-        b2s_mapping::Slot &sl = m->slot[k];
-        sl.d_in.release(); sl.d_map.release(); sl.h_pose.release();
-        if (sl.d_cnt) cudaFree(sl.d_cnt);
-        if (sl.h_cnt) cudaFreeHost(sl.h_cnt);
-        if (sl.inputs_free) cudaEventDestroy(sl.inputs_free);
-        if (sl.done) cudaEventDestroy(sl.done);
-    }
-    if (m->finalized) cudaEventDestroy(m->finalized);
-    if (m->d2h_stream) cudaStreamDestroy(m->d2h_stream);
-    for (int k = 0; k < MAX_CHUNKS; ++k)
-        if (m->chunk_ready[k]) cudaEventDestroy(m->chunk_ready[k]);
-    if (m->begun) cudaEventDestroy(m->begun);
-    if (m->joined) cudaEventDestroy(m->joined);
-    if (m->copy_stream) cudaStreamDestroy(m->copy_stream);
-    if (m->stream2) cudaStreamDestroy(m->stream2);
-    if (m->stream) cudaStreamDestroy(m->stream);
+    m->teardown([m] {
+        if (m->hit) cudaFree(m->hit);
+        if (m->miss) cudaFree(m->miss);
+        if (m->counters) cudaFree(m->counters);
+        if (m->workspace) cudaFree(m->workspace);
+        if (m->h_packed) cudaFreeHost(m->h_packed);
+        if (m->h_ids) cudaFreeHost(m->h_ids);
+        m->d_packed.release();
+        m->d_in.release(); m->d_datamap.release(); m->d_pmap.release();
+        m->h_pose.release();
+        for (MappingSlot &sl : m->slot) {
+            sl.d_in.release(); sl.d_map.release(); sl.h_pose.release();
+            if (sl.d_cnt) cudaFree(sl.d_cnt);
+            if (sl.h_cnt) cudaFreeHost(sl.h_cnt);
+        }
+        if (m->begun) cudaEventDestroy(m->begun);
+    });
     delete m;
     return B2S_OK;
 }
@@ -1312,7 +1280,7 @@ extern "C" int b2s_mapping_update_scans(b2s_mapping *m, const float *ranges, con
 // step's verdict; a batch the reference would raise on is taken back out of the counts there (one sign -1 ray-cast of
 // the slot's still-resident inputs: exact), but maps of steps submitted in between were finalized with it still applied.
 namespace {
-int mapping_wait_slot(b2s_mapping *m, b2s_mapping::Slot &sl)
+int mapping_wait_slot(b2s_mapping *m, MappingSlot &sl)
 {
     if (!sl.in_flight) return B2S_OK;
     B2S_CUDA(cudaEventSynchronize(sl.done));
@@ -1330,8 +1298,8 @@ int mapping_submit_impl(b2s_mapping *m, const HostBatch &hb, int scans, int beam
 {
     DeviceGuard g(m->device);
     const int ticket = m->submitted;
-    b2s_mapping::Slot &sl = m->slot[ticket & 1];
-    b2s_mapping::Slot &other = m->slot[(ticket & 1) ^ 1];
+    MappingSlot &sl = m->slot[ticket & 1];
+    MappingSlot &other = m->slot[(ticket & 1) ^ 1];
     int rc;
     if (sl.in_flight && (rc = mapping_wait_slot(m, sl))) return rc;  // its buffers are about to be reused
     const size_t total = (size_t)scans * beams, cells = (size_t)m->xw * m->yw;
@@ -1368,8 +1336,8 @@ int mapping_submit_impl(b2s_mapping *m, const HostBatch &hb, int scans, int beam
                                m->stream);
         if (rc) return rc;
     }
-    B2S_CUDA(cudaEventRecord(m->finalized, m->stream));
-    B2S_CUDA(cudaStreamWaitEvent(m->d2h_stream, m->finalized, 0));
+    B2S_CUDA(cudaEventRecord(m->handoff, m->stream));
+    B2S_CUDA(cudaStreamWaitEvent(m->d2h_stream, m->handoff, 0));
     if (pmap_out) B2S_CUDA(cudaMemcpyAsync(pmap_out, sl.d_map.p, cells, cudaMemcpyDeviceToHost, m->d2h_stream));
     B2S_CUDA(cudaMemcpyAsync(sl.h_cnt, sl.d_cnt, B2S_CNT_WORDS * sizeof(int32_t), cudaMemcpyDeviceToHost, m->d2h_stream));
     B2S_CUDA(cudaEventRecord(sl.done, m->d2h_stream));
@@ -1409,7 +1377,7 @@ extern "C" int b2s_mapping_wait(b2s_mapping *m, int ticket)
     B2S_REQUIRE(m, "b2s_mapping_wait: null handle");
     B2S_REQUIRE(ticket >= 0 && ticket < m->submitted, "b2s_mapping_wait: unknown ticket");
     DeviceGuard g(m->device);
-    b2s_mapping::Slot &sl = m->slot[ticket & 1];
+    MappingSlot &sl = m->slot[ticket & 1];
     if (!sl.in_flight || sl.ticket != ticket) return B2S_OK;  // already waited for (or superseded and waited implicitly)
     return mapping_wait_slot(m, sl);
 }
