@@ -32,6 +32,7 @@ SIGNATURES = {
     "b2s_measure_fp64_peak": (_i32, [ctypes.POINTER(_dbl)]),
     "b2s_icp_batch_f32": (_i32, [_vp, _vp, _i32, _i32, _i32, _i32, _dbl, _vp, _vp, _vp]),
     "b2s_icp_batch_f64": (_i32, [_vp, _vp, _i32, _i32, _i32, _i32, _dbl, _vp, _vp, _vp]),
+    "b2s_icp_batch_f64_err": (_i32, [_vp, _vp, _i32, _i32, _i32, _i32, _dbl, _vp, _vp, _vp, _vp]),
     "b2s_icp_batch_ranges": (_i32, [_vp, _vp, _vp, _dbl, _i32, _i32, _i32, _dbl, _vp, _vp, _vp]),
     "b2s_nearest_f64": (_i32, [_vp, _i32, _vp, _i32, _vp, _vp, _vp]),
     "b2s_rigid_fit_f64": (_i32, [_vp, _vp, _i32, _vp, _vp]),
@@ -57,6 +58,7 @@ SIGNATURES = {
     "b2s_virtual_scan": (_i32, [_vp, _vp, _i32, _dbl, _dbl, _dbl, _dbl, _dbl, _i32, _dbl, _vp, _vp]),
     "b2s_virtual_scan_host": (_i32, [_vp, _vp, _i32, _dbl, _dbl, _dbl, _dbl, _dbl, _i32, _dbl, _vp]),
     "b2s_virtual_scan_batch": (_i32, [_vp, _vp, _i32, _vp, _i32, _dbl, _dbl, _i32, _dbl, _vp, _vp, _vp, _vp]),
+    "b2s_relocalize_select": (_i32, [_vp, _vp, _vp, _i32, _i32, _vp, _vp, _vp]),
     "b2s_grid_allreduce": (_i32, [_vp, _vp, _sz, _vp, _vp]),
     "b2s_grid_merge_p2p": (_i32, [_vp, _vp, _vp, _i32, _sz, _sz, _vp, _vp, _dbl, _dbl, _dbl, _vp]),
     "b2s_grid_merge_p2p_tiles": (_i32, [_vp, _vp, _vp, _vp, _i32, _i32, _i32, _i32, _i32, _vp, _vp, _dbl, _dbl,
@@ -93,6 +95,8 @@ SIGNATURES = {
     "b2s_icp_set_map": (_i32, [_vp, _vp, _vp, _i32]),
     "b2s_icp_map_observation": (_i32, [_vp, _vp, _vp, _vp, _dbl, _i32, _i32, _dbl, _dbl, _dbl, _i32, _dbl, _vp, _vp,
                                        _vp]),
+    "b2s_icp_relocalize": (_i32, [_vp, _vp, _vp, _vp, _dbl, _i32, _i32, _i32, _dbl, _dbl, _dbl, _i32, _dbl, _vp, _vp,
+                                  _vp, _vp, _vp]),
     "b2s_icp_find_nearest": (_i32, [_vp, _vp, _i32, _vp, _i32, _vp, _vp]),
     "b2s_icp_get_transform": (_i32, [_vp, _vp, _vp, _i32, _vp]),
     "b2s_mapping_create": (_i32, [_pp, _i32, _i32, _dbl, _dbl, _dbl, _dbl, _i32]),

@@ -40,6 +40,8 @@ constexpr int ICP_MAX_POINTS = 2304;  // source points per scan of the ICP kerne
 // 16-byte aligned, clamp > 0 replaces +inf.  The points are those the ICP kernel's fused form makes from the ranges.
 int laser_points(const float *ranges, const double *beam_cs, double clamp, int scans, int beams, double *xy,
                  cudaStream_t stream);
+// `copies` consecutive copies of the `row` doubles at src into dst (b2s_next.cu).
+int replicate_row(const double *src, size_t row, size_t copies, double *dst, cudaStream_t stream);
 
 // Growable device / pinned-host staging buffer.
 struct Buf {

@@ -916,6 +916,83 @@ extern "C" int b2s_icp_map_observation(b2s_icp *c, const float *ranges, const do
     return icp_read_back(c, tr, scans, T_out, iters_out);
 }
 
+// Relocalization: the map observation of every scan at every candidate.  The H virtual scans depend on the candidate
+// only, so they are built once into the target layout and shared by all scans; per scan, laserToNumpy forms its source
+// cloud once, replicated into the H source rows, and the H-pair ICP runs with its score output, the scans alternating
+// between stream and stream2.  One selection launch over all scans follows on stream, then the read-back.
+extern "C" int b2s_icp_relocalize(b2s_icp *c, const float *ranges, const double *candidates3, const double *beam_cs,
+                                  double clamp_inf_to, int scans, int hyps, int n, double angle_min, double angle_increment,
+                                  double far_range, int max_iter, double tol, int32_t *best_out, double *pose_out,
+                                  double *score_out, int32_t *iters_out, double *T_out)
+{
+    B2S_REQUIRE(scans >= 0 && hyps > 0 && n > 0 && max_iter >= 0 && (long long)scans * hyps <= 0x7fffffffLL,
+                "b2s_icp_relocalize: bad sizes");
+    B2S_REQUIRE(n <= ICP_MAX_POINTS, "b2s_icp_batch: more than 2304 source points per scan is not supported");
+    B2S_REQUIRE(angle_increment != 0.0 && angle_increment == angle_increment, "b2s_icp_relocalize: angle_increment");
+    B2S_REQUIRE(clamp_inf_to == clamp_inf_to && tol == tol, "b2s_icp_relocalize: NaN clamp / tolerance");
+    B2S_REQUIRE(c, "b2s_icp_relocalize: null handle");
+    B2S_REQUIRE(c->map_count > 0, "b2s_icp_relocalize: no static map set (b2s_icp_set_map)");
+    if (scans == 0) return B2S_OK;
+    B2S_REQUIRE(ranges && candidates3 && beam_cs && best_out && pose_out, "b2s_icp_relocalize: null pointer");
+    for (size_t i = 0; i < (size_t)hyps * 3; ++i)  // as in b2s_icp_map_observation
+        if (candidates3[i] != candidates3[i]) {
+            set_error("%s", NAN_TO_INT);
+            return B2S_ERR_NONFINITE;
+        }
+    DeviceGuard g(c->device);
+    Trace tr(c->stream);
+    const size_t H = (size_t)hyps, K = (size_t)scans, cloud = H * 2 * n;  // doubles of one set of H clouds
+    const size_t cs_bytes = (size_t)n * 2 * sizeof(double), cand_bytes = H * 3 * sizeof(double);
+    const size_t cand_off = cs_bytes, range_off = (cand_off + cand_bytes + 15) & ~(size_t)15;
+    // d_aux: scores [K][H] | best [K] | poses [K][3] (+ one scan's source cloud per compute stream)
+    const size_t score_bytes = K * H * sizeof(double), best_off = score_bytes;
+    const size_t pose_off = (best_off + K * sizeof(int32_t) + 15) & ~(size_t)15, cloud_off = pose_off + K * 3 * sizeof(double);
+    int rc;
+    if ((rc = c->d_map_in.reserve(range_off + K * n * sizeof(float)))) return rc;
+    if ((rc = c->d_map_tar.reserve(cloud * sizeof(double)))) return rc;
+    if ((rc = c->d_map_src.reserve(2 * cloud * sizeof(double)))) return rc;
+    if ((rc = c->d_T.reserve(K * H * 9 * sizeof(double)))) return rc;
+    if ((rc = c->d_iters.reserve(K * H * sizeof(int32_t)))) return rc;
+    if ((rc = c->d_aux.reserve(cloud_off + 2 * cs_bytes))) return rc;
+    char *in = (char *)c->d_map_in.p, *aux = (char *)c->d_aux.p;
+    const double *d_cs = (const double *)in, *d_cand = (const double *)(in + cand_off);
+    const float *d_ranges = (const float *)(in + range_off);
+    double *d_tar = (double *)c->d_map_tar.p, *d_T = (double *)c->d_T.p, *d_score = (double *)aux;
+    int32_t *d_iters = (int32_t *)c->d_iters.p, *d_best = (int32_t *)(aux + best_off);
+    double *d_pose = (double *)(aux + pose_off);
+    const double *map_x = (const double *)c->d_map.p, *map_y = map_x + c->map_count;
+    // (every call ends with a synchronize, so the device buffers are free to overwrite here)
+    B2S_CUDA(cudaMemcpyAsync(in, beam_cs, cs_bytes, cudaMemcpyHostToDevice, c->stream));
+    B2S_CUDA(cudaMemcpyAsync(in + cand_off, candidates3, cand_bytes, cudaMemcpyHostToDevice, c->stream));
+    B2S_CUDA(cudaMemcpyAsync(in + range_off, ranges, K * n * sizeof(float), cudaMemcpyHostToDevice, c->stream));
+    if ((rc = b2s_virtual_scan_batch(map_x, map_y, c->map_count, d_cand, hyps, angle_min, angle_increment, n, far_range,
+                                     d_cs, nullptr, d_tar, c->stream)))
+        return rc;
+    tr.mark("virtual scans done", 0, c->stream);
+    B2S_CUDA(cudaEventRecord(c->chunk_ready[0], c->stream));  // the uploads and targets, for stream2
+    B2S_CUDA(cudaStreamWaitEvent(c->stream2, c->chunk_ready[0], 0));
+    for (size_t k = 0; k < K; ++k) {
+        cudaStream_t ks = (k & 1) ? c->stream2 : c->stream;
+        double *one = (double *)(aux + cloud_off) + (k & 1) * 2 * n, *src = (double *)c->d_map_src.p + (k & 1) * cloud;
+        if ((rc = laser_points(d_ranges + k * n, d_cs, clamp_inf_to, 1, n, one, ks))) return rc;
+        if ((rc = replicate_row(one, (size_t)2 * n, H, src, ks))) return rc;
+        if ((rc = b2s_icp_batch_f64_err(d_tar, src, hyps, n, n, max_iter, tol, d_T + k * H * 9, d_iters + k * H,
+                                        d_score + k * H, ks)))
+            return rc;
+        tr.mark("relocalize scan done", (int)k, ks);
+    }
+    if (K > 1) {
+        B2S_CUDA(cudaEventRecord(c->joined, c->stream2));
+        B2S_CUDA(cudaStreamWaitEvent(c->stream, c->joined, 0));
+    }
+    if ((rc = b2s_relocalize_select(d_score, d_T, d_cand, scans, hyps, d_best, d_pose, c->stream))) return rc;
+    tr.mark("select done", 0, c->stream);
+    B2S_CUDA(cudaMemcpyAsync(best_out, d_best, K * sizeof(int32_t), cudaMemcpyDeviceToHost, c->stream));
+    B2S_CUDA(cudaMemcpyAsync(pose_out, d_pose, K * 3 * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
+    if (score_out) B2S_CUDA(cudaMemcpyAsync(score_out, d_score, score_bytes, cudaMemcpyDeviceToHost, c->stream));
+    return icp_read_back(c, tr, (int)(K * H), T_out, iters_out);
+}
+
 extern "C" int b2s_icp_find_nearest(b2s_icp *c, const double *src_xy, int n, const double *tar_xy,
                                     int m, double *dist_out, int64_t *idx_out)
 {

@@ -8,7 +8,7 @@ extern "C" int b2s_icp_batch_f32(const float *tar_xy, const float *src_xy, int p
                                  int n_tar, int max_iter, double tol, double *T_out,
                                  int32_t *iters_out, void *stream)
 {
-    return launch_icp<float>(tar_xy, src_xy, pairs, n_src, n_tar, max_iter, tol, T_out, iters_out, stream);
+    return launch_icp<float>(tar_xy, src_xy, pairs, n_src, n_tar, max_iter, tol, T_out, iters_out, nullptr, stream);
 }
 
 extern "C" int b2s_icp_batch_ranges(const float *tar_ranges, const float *src_ranges, const double *beam_cs,

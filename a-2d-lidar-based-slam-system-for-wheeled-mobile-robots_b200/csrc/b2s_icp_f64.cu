@@ -8,5 +8,12 @@ extern "C" int b2s_icp_batch_f64(const double *tar_xy, const double *src_xy, int
                                  int n_tar, int max_iter, double tol, double *T_out,
                                  int32_t *iters_out, void *stream)
 {
-    return launch_icp<double>(tar_xy, src_xy, pairs, n_src, n_tar, max_iter, tol, T_out, iters_out, stream);
+    return launch_icp<double>(tar_xy, src_xy, pairs, n_src, n_tar, max_iter, tol, T_out, iters_out, nullptr, stream);
+}
+
+extern "C" int b2s_icp_batch_f64_err(const double *tar_xy, const double *src_xy, int pairs, int n_src, int n_tar,
+                                     int max_iter, double tol, double *T_out, int32_t *iters_out, double *err_out,
+                                     void *stream)
+{
+    return launch_icp<double>(tar_xy, src_xy, pairs, n_src, n_tar, max_iter, tol, T_out, iters_out, err_out, stream);
 }

@@ -362,11 +362,15 @@ static __device__ __noinline__ unsigned collective_nearest_padded(double px, dou
 // RANGES = true is the fused-ingestion form (SURVEY 8f-1): tar_xy / src_xy hold raw ranges (one float per beam, n == m)
 // and the points are formed here exactly as laserToNumpy does ([ICP]:216-229, [SLAM]:115-123): float64
 // (cos a * r, sin a * r) with the beam table computed by the host's NumPy, +inf -> clamp when clamp > 0.
-template <typename TIn, int R, int PRUNE, int NN_BLK, bool RANGES = false>
+//
+// ERR = true writes each pair's mean error of its last iteration ([ICP]:75) to err_out[pair].  It is a template
+// parameter rather than a null test so that the instances without it compile to exactly the code they had before.
+template <typename TIn, int R, int PRUNE, int NN_BLK, bool RANGES = false, bool ERR = false>
 __global__ void __maxnreg__(R <= 3 ? (NN_BLK == 8 && PRUNE != 5 ? B2S_ICP_REGS_BLK8 : B2S_ICP_REGS_BLK16) : 104) icp_batch_kernel(const TIn *__restrict__ tar_xy, const TIn *__restrict__ src_xy, int n,
                                  int m, int max_iter, double tol, double *__restrict__ T_out,
                                  int32_t *__restrict__ iters_out, int use_bulk,
-                                 const double2 *__restrict__ beam_cs = nullptr, double clamp = 0.0)
+                                 const double2 *__restrict__ beam_cs = nullptr, double clamp = 0.0,
+                                 double *__restrict__ err_out = nullptr)
 {
     constexpr int ROWS = RANGES ? 1 : 2;  // values per point in the input arrays
     auto point = [&](const TIn *scan, int count, int i, double &x, double &y) {
@@ -554,7 +558,7 @@ __global__ void __maxnreg__(R <= 3 ? (NN_BLK == 8 && PRUNE != 5 ? B2S_ICP_REGS_B
         for (int r = 0; r < R; ++r) srcm[tid + r * blockDim.x] = make_double2(sx[r], sy[r]);
     }
 
-    double prev_err = 0.0;
+    double prev_err = 0.0, err = 0.0;  // err after the loop: the mean error of the last iteration run
     int iters = 0;
     for (int it = 0; it < max_iter; ++it) {
         // ---- nearest neighbour ([ICP]:99-106)
@@ -889,11 +893,12 @@ __global__ void __maxnreg__(R <= 3 ? (NN_BLK == 8 && PRUNE != 5 ? B2S_ICP_REGS_B
             if (QUEUED) srcm[tid + r * blockDim.x] = make_double2(sx[r], sy[r]);
         }
         ++iters;
-        const double err = dsum / (double)n;
+        err = dsum / (double)n;
         if (fabs(prev_err - err) < tol) break;  // [ICP]:76, uniform across the CTA
         prev_err = err;
     }
 
+    if (ERR && tid == 0) err_out[pair] = err;  // (here rather than below: err is not held across the final fit)
     double T[6];
     double unused = 0.0;
     double ox_[R], oy_[R];
@@ -936,7 +941,7 @@ static size_t icp_smem_bytes(int n_tar, size_t in_bytes, int threads)
 
 template <typename TIn, int R, int PRUNE, int NN_BLK>
 static int launch_icp_rp(const TIn *tar_xy, const TIn *src_xy, int pairs, int n_src, int n_tar, int max_iter,
-                        double tol, double *T_out, int32_t *iters_out, void *stream)
+                        double tol, double *T_out, int32_t *iters_out, double *err_out, void *stream)
 {
     int threads = (n_src + R - 1) / R;
     threads = ((threads + 31) / 32) * 32;
@@ -944,34 +949,37 @@ static int launch_icp_rp(const TIn *tar_xy, const TIn *src_xy, int pairs, int n_
     B2S_REQUIRE(threads <= 1024, "b2s_icp_batch: too many source points per scan");
     const size_t smem = icp_smem_bytes<PRUNE, NN_BLK, R>(n_tar, (size_t)n_tar * 2 * sizeof(TIn), threads);
     B2S_REQUIRE(smem <= 227 * 1024, "b2s_icp_batch: n_tar too large for shared memory");
+    // the score output exists for float64 clouds only (the relocalization's virtual scans and laserToNumpy points)
+    constexpr bool HAS_ERR = sizeof(TIn) == 8;
+    auto kernel = icp_batch_kernel<TIn, R, PRUNE, NN_BLK>;
+    if (HAS_ERR && err_out) kernel = icp_batch_kernel<TIn, R, PRUNE, NN_BLK, false, HAS_ERR>;
     // opt-in above 48 KB; the attribute is per device and per function, and setting it is cheap
     if (smem > 48 * 1024)
-        B2S_CUDA(cudaFuncSetAttribute(icp_batch_kernel<TIn, R, PRUNE, NN_BLK>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                      (int)smem));
+        B2S_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     // bulk copy needs 16-byte aligned source and size: every pair's target block must qualify
     const size_t pair_bytes = (size_t)2 * n_tar * sizeof(TIn);
     const int use_bulk = (((uintptr_t)tar_xy % 16 == 0) && (pair_bytes % 16 == 0) ? 1 : 0) | (g_icp_layout << 1);
     if (threads > 512) {  // (large scans only: the query is not free)
         cudaFuncAttributes fa;
-        B2S_CUDA(cudaFuncGetAttributes(&fa, icp_batch_kernel<TIn, R, PRUNE, NN_BLK>));
+        B2S_CUDA(cudaFuncGetAttributes(&fa, kernel));
         B2S_REQUIRE(threads <= fa.maxThreadsPerBlock, "b2s_icp_batch: scan too large for one CTA's registers");
     }
-    icp_batch_kernel<TIn, R, PRUNE, NN_BLK><<<pairs, threads, smem, (cudaStream_t)stream>>>(
-        tar_xy, src_xy, n_src, n_tar, max_iter, tol, T_out, iters_out, use_bulk);
+    kernel<<<pairs, threads, smem, (cudaStream_t)stream>>>(
+        tar_xy, src_xy, n_src, n_tar, max_iter, tol, T_out, iters_out, use_bulk, nullptr, 0.0, err_out);
     B2S_CUDA(cudaGetLastError());
     return B2S_OK;
 }
 
 template <typename TIn, int R>
 static int launch_icp_r(const TIn *tar_xy, const TIn *src_xy, int pairs, int n_src, int n_tar, int max_iter,
-                        double tol, double *T_out, int32_t *iters_out, void *stream)
+                        double tol, double *T_out, int32_t *iters_out, double *err_out, void *stream)
 {
     // the block bounds live in the staging area: [ceil(m/blk)] float4 must fit in 2*m*sizeof(TIn)
     const int blk = (g_icp_block == 8 || g_icp_block == 16 || g_icp_block == 32) ? g_icp_block
                     : (g_icp_prune == 4 ? 8 : g_icp_prune >= 2 ? (n_tar <= 600 ? 8 : 16) : (n_tar <= 600 ? 16 : 32));  // measured best per mode
     const bool fits = (size_t)((n_tar + blk - 1) / blk) * 16 <= (size_t)2 * n_tar * sizeof(TIn);
 #define B2S_ICP_GO(P, B) \
-    return launch_icp_rp<TIn, R, P, B>(tar_xy, src_xy, pairs, n_src, n_tar, max_iter, tol, T_out, iters_out, stream)
+    return launch_icp_rp<TIn, R, P, B>(tar_xy, src_xy, pairs, n_src, n_tar, max_iter, tol, T_out, iters_out, err_out, stream)
     if (g_icp_prune && fits) {
         if (g_icp_prune == 4) {  // (block numbers travel in one byte; beyond that the collective search takes over)
             if (blk == 8 && (n_tar + 7) / 8 <= QBLOCKS) {
@@ -1088,9 +1096,10 @@ static int launch_icp_ranges(const float *tar_r, const float *src_r, const doubl
     }
 }
 
+// err_out [pairs] (may be NULL): the reference's mean_error ([ICP]:75) of each pair's last iteration.
 template <typename TIn>
 static int launch_icp(const TIn *tar_xy, const TIn *src_xy, int pairs, int n_src, int n_tar,
-                      int max_iter, double tol, double *T_out, int32_t *iters_out, void *stream)
+                      int max_iter, double tol, double *T_out, int32_t *iters_out, double *err_out, void *stream)
 {
     B2S_REQUIRE(pairs >= 0 && n_src > 0 && n_tar > 0 && max_iter >= 0, "b2s_icp_batch: bad sizes");
     if (pairs == 0) return B2S_OK;
@@ -1099,9 +1108,9 @@ static int launch_icp(const TIn *tar_xy, const TIn *src_xy, int pairs, int n_src
     B2S_REQUIRE(n_src <= ICP_MAX_POINTS, "b2s_icp_batch: more than 2304 source points per scan is not supported");
     const int r = icp_points_per_thread(n_src);
     switch (r) {
-    case 2: return launch_icp_r<TIn, 2>(tar_xy, src_xy, pairs, n_src, n_tar, max_iter, tol, T_out, iters_out, stream);
-    case 3: return launch_icp_r<TIn, 3>(tar_xy, src_xy, pairs, n_src, n_tar, max_iter, tol, T_out, iters_out, stream);
-    default: return launch_icp_r<TIn, 4>(tar_xy, src_xy, pairs, n_src, n_tar, max_iter, tol, T_out, iters_out, stream);
+    case 2: return launch_icp_r<TIn, 2>(tar_xy, src_xy, pairs, n_src, n_tar, max_iter, tol, T_out, iters_out, err_out, stream);
+    case 3: return launch_icp_r<TIn, 3>(tar_xy, src_xy, pairs, n_src, n_tar, max_iter, tol, T_out, iters_out, err_out, stream);
+    default: return launch_icp_r<TIn, 4>(tar_xy, src_xy, pairs, n_src, n_tar, max_iter, tol, T_out, iters_out, err_out, stream);
     }
 }
 

@@ -7,6 +7,8 @@
 //                 obstacle cells -> one thread per obstacle, atomicMin on the float64 bit pattern.  The batched form
 //                 reduces each pose's bins in shared memory and can write them as the ICP's target cloud.
 //   laserToNumpy  [ICP]:216-229 / [SLAM]:115-123 of float32 ranges into float64 points (the ICP's source cloud).
+//   relocalize    the selection among map observations at many candidate poses: per scan the lowest finite
+//                 mean_error ([ICP]:75), ties to the lower index, composed with its candidate ([ICP]:185-190).
 #include "b2s_common.cuh"
 
 #include <math.h>
@@ -206,6 +208,87 @@ laser_points_kernel(const float *__restrict__ ranges, const double2 *__restrict_
     xy[2 * k * beams + beams + i] = __dmul_rn(cs.y, r);
 }
 
+// `copies` consecutive copies of one row of `row` doubles: the source cloud of a scan for every hypothesis of a
+// relocalization (the ICP kernel reads pair p's source at p * row).
+__global__ void __launch_bounds__(256)
+replicate_row_kernel(const double *__restrict__ src, size_t row, size_t copies, double *__restrict__ dst)
+{
+    const size_t total = row * copies;
+    for (size_t j = (size_t)blockIdx.x * blockDim.x + threadIdx.x; j < total; j += (size_t)gridDim.x * blockDim.x)
+        dst[j] = src[j % row];
+}
+
+// Relocalization selection: CTA k reduces the scores of scan k's hypotheses to the smallest (score, h) among those
+// whose score and transform are finite, then composes the winner's pose.  (score, h) with the lower h winning equal
+// scores is a strict total order in which every h occurs once, so the minimum is one element whatever the order of
+// the comparisons: the result does not depend on the CTA's thread count or on how the reduction is cut.
+constexpr int SELECT_THREADS = 256;
+
+__device__ __forceinline__ void select_better(double &bs, int &bh, double s, int h)
+{
+    if (h >= 0 && (bh < 0 || s < bs || (s == bs && h < bh))) {
+        bs = s;
+        bh = h;
+    }
+}
+
+__global__ void __launch_bounds__(SELECT_THREADS)
+relocalize_select_kernel(const double *__restrict__ score, const double *__restrict__ T,
+                         const double *__restrict__ cand, int hyps, int32_t *__restrict__ best_out,
+                         double *__restrict__ pose_out)
+{
+    __shared__ double ws[SELECT_THREADS / 32];
+    __shared__ int wh[SELECT_THREADS / 32];
+    const int k = blockIdx.x;
+    const double *sk = score + (size_t)k * hyps;
+    const double *Tk = T + (size_t)k * hyps * 9;
+    double bs = 0.0;
+    int bh = -1;  // -1: nothing finite yet
+    for (int h = threadIdx.x; h < hyps; h += blockDim.x) {
+        const double s = sk[h];
+        bool finite = fabs(s) < INFINITY;  // false for NaN and +-inf
+        for (int i = 0; i < 9; ++i) finite = finite && fabs(Tk[(size_t)h * 9 + i]) < INFINITY;
+        if (finite) select_better(bs, bh, s, h);
+    }
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        const double os = __shfl_xor_sync(0xffffffffu, bs, o);
+        const int oh = __shfl_xor_sync(0xffffffffu, bh, o);
+        select_better(bs, bh, os, oh);
+    }
+    if (lane == 0) {
+        ws[warp] = bs;
+        wh[warp] = bh;
+    }
+    __syncthreads();
+    if (threadIdx.x != 0) return;
+    for (int w = 1; w < (int)(blockDim.x >> 5); ++w) select_better(bs, bh, ws[w], wh[w]);
+    best_out[k] = bh;
+    double *pose = pose_out + 3 * (size_t)k;
+    if (bh < 0) {
+        pose[0] = pose[1] = pose[2] = __longlong_as_double(0x7ff8000000000000LL);
+        return;
+    }
+    // [ICP]:185-190, the pose-chain step of one transform
+    const double *t = Tk + (size_t)bh * 9;
+    const double x = cand[3 * (size_t)bh], y = cand[3 * (size_t)bh + 1], yaw = cand[3 * (size_t)bh + 2];
+    const double c = cos(yaw), s = sin(yaw);
+    pose[0] = x + c * t[2] - s * t[5];
+    pose[1] = y + s * t[2] + c * t[5];
+    pose[2] = yaw + atan2(t[3], t[0]);
+}
+
+int replicate_row(const double *src, size_t row, size_t copies, double *dst, cudaStream_t st)
+{
+    const size_t total = row * copies;
+    if (total == 0) return B2S_OK;
+    const size_t want = (total + 255) / 256, cap = (size_t)sm_count() * 16;
+    replicate_row_kernel<<<(unsigned)(want < cap ? want : cap), 256, 0, st>>>(src, row, copies, dst);
+    B2S_CUDA(cudaGetLastError());
+    return B2S_OK;
+}
+
 // Slices per pose: one CTA per pose when the poses alone fill the device a few times over; otherwise the obstacles are
 // cut into slices of at least VSCAN_MIN_SLICE cells so that a small batch over a large map still spreads over every SM.
 constexpr int VSCAN_MIN_SLICE = 1024;
@@ -299,6 +382,18 @@ extern "C" int b2s_virtual_scan_batch(const double *obs_x, const double *obs_y, 
         virtual_scan_points_kernel<<<blocks, 256, 0, st>>>(merge, cs, scans, beams, stride, tar_xy);
         B2S_CUDA(cudaGetLastError());
     }
+    return B2S_OK;
+}
+
+extern "C" int b2s_relocalize_select(const double *score, const double *T, const double *candidates3, int scans, int hyps,
+                                     int32_t *best_out, double *pose_out, void *stream)
+{
+    B2S_REQUIRE(scans >= 0 && hyps > 0, "b2s_relocalize_select: bad sizes");
+    if (scans == 0) return B2S_OK;
+    B2S_REQUIRE(score && T && candidates3 && best_out && pose_out, "b2s_relocalize_select: null pointer");
+    relocalize_select_kernel<<<scans, SELECT_THREADS, 0, (cudaStream_t)stream>>>(score, T, candidates3, hyps, best_out,
+                                                                                 pose_out);
+    B2S_CUDA(cudaGetLastError());
     return B2S_OK;
 }
 

@@ -125,6 +125,44 @@ def icp_batch(tar, src, max_iter=30, tol=1e-3, T_out=None, iters_out=None):
     return T_out, iters_out
 
 
+def icp_batch_err(tar, src, max_iter=30, tol=1e-3, T_out=None, iters_out=None, err_out=None):
+    """b2s_icp_batch_f64_err: icp_batch on float64 tar (P,2,M), src (P,2,N) that also returns each pair's mean_error
+    of its last iteration ([ICP]:75-76) in err_out (P,) float64.  Returns (T_out, iters_out, err_out)."""
+    P, _, M = tar.shape
+    N = src.shape[2]
+    if T_out is None:
+        T_out = torch.empty((P, 3, 3), dtype=torch.float64, device=tar.device)
+    if iters_out is None:
+        iters_out = torch.empty(P, dtype=torch.int32, device=tar.device)
+    if err_out is None:
+        err_out = torch.empty(P, dtype=torch.float64, device=tar.device)
+    rc = _lib.lib().b2s_icp_batch_f64_err(
+        _chk(tar, torch.float64, "tar"), _chk(src, torch.float64, "src"), P, N, M, int(max_iter), float(tol),
+        _chk(T_out, torch.float64, "T_out"), _chk(iters_out, torch.int32, "iters"), _chk(err_out, torch.float64, "err"),
+        _stream())
+    _lib.check(rc)
+    return T_out, iters_out, err_out
+
+
+def relocalize_select(score, T, candidates, best_out=None, pose_out=None):
+    """b2s_relocalize_select: score (K,H) float64, T (K,H,3,3) float64, candidates (H,3) float64 CUDA tensors ->
+    (best (K,) int32, pose (K,3) float64): per scan the lowest-index smallest score among the hypotheses whose score
+    and T are finite (-1 and a NaN pose when none is), and candidates[best] composed with T[best] ([ICP]:185-190)."""
+    K, H = score.shape
+    for t, shape, name in ((T, (K, H, 3, 3), "T"), (candidates, (H, 3), "candidates")):
+        if tuple(t.shape) != shape:
+            raise ValueError("%s must have shape %s, got %s" % (name, shape, tuple(t.shape)))
+    if best_out is None:
+        best_out = torch.empty(K, dtype=torch.int32, device=score.device)
+    if pose_out is None:
+        pose_out = torch.empty((K, 3), dtype=torch.float64, device=score.device)
+    rc = _lib.lib().b2s_relocalize_select(
+        _chk(score, torch.float64, "score"), _chk(T, torch.float64, "T"), _chk(candidates, torch.float64, "candidates"),
+        K, H, _chk(best_out, torch.int32, "best_out"), _chk(pose_out, torch.float64, "pose_out"), _stream())
+    _lib.check(rc)
+    return best_out, pose_out
+
+
 def virtual_scan_batch(obs_x, obs_y, poses, angle_min, angle_increment, beams, far_range=100.0, beam_cs=None,
                        ranges=None, tar_xy=None):
     """b2s_virtual_scan_batch: laserEstimation for K poses at once.  obs_x, obs_y float64 (C,) obstacle cell centres,

@@ -297,6 +297,57 @@ class ICP(object):
         T = T.reshape(K, 3, 3)
         return (T, iters, virt) if return_virtual else (T, iters)
 
+    def relocalize(self, ranges, candidates, angle_min, angle_max, angle_increment=None, clamp_inf_to=None,
+                   far_range=100.0, max_iter=None, tolerance=None, return_T=False):
+        """Relocalization in the static map (set_static_map) for a robot whose pose is unknown: at start-up, after the
+        EKF has diverged, or where a recorded stream starts at an unknown place.  The map observation is run at every
+        candidate pose and the best one is kept; the caller supplies the candidates (synth.room_relocalization shows
+        one grid layout).
+
+        ranges (K,N) float32, or (N,) for one scan; candidates (H,3) float64 x, y, yaw, shared by the K scans.
+        Hypothesis (k, h) is map_observation(ranges[k:k+1], candidates[h:h+1], ...) bit for bit (T and iterations);
+        the H virtual scans are built once per call.  score[k, h] is the reference's mean_error of the last iteration
+        that ran ([ICP]:75-76): the mean matched distance before that iteration's move, unmatched (inf / NaN)
+        distances counting 0.  best[k] is the h with the smallest score among the hypotheses whose score and T are
+        finite, the lowest h on ties, or -1 when none is (then pose[k] is NaN).  pose[k] is the sensor pose in the map
+        frame, candidates[best[k]] composed with T[k, best[k]] by the pose-chain step of [ICP]:185-190.
+
+        Scans with +inf ranges need clamp_inf_to for meaningful scores: without it their inf points count as distance
+        0 for every hypothesis.
+
+        Returns (best (K,) int32, pose (K,3), score (K,H), iterations (K,H) int32), plus T (K,H,3,3) with
+        return_T=True; for one (N,) scan the K axis is dropped.  Errors are those of map_observation: a NaN candidate
+        raises ValueError like the reference's int(), before any device work.
+        """
+        ranges = np.asarray(ranges, dtype=np.float32)
+        one = ranges.ndim == 1
+        ranges = np.ascontiguousarray(ranges[None] if one else ranges)
+        if ranges.ndim != 2 or ranges.shape[1] < 1:
+            raise ValueError("expected ranges (K,N) or (N,) with N >= 1, got %s" % (ranges.shape,))
+        K, N = ranges.shape
+        candidates = np.ascontiguousarray(candidates, dtype=np.float64)
+        if candidates.ndim != 2 or candidates.shape[1] != 3 or candidates.shape[0] < 1:
+            raise ValueError("expected candidates (H,3) with H >= 1, got %s" % (candidates.shape,))
+        H = candidates.shape[0]
+        if angle_increment is None:
+            if N < 2:
+                raise ValueError("a one-beam scan needs an explicit angle_increment")
+            angle_increment = (float(angle_max) - float(angle_min)) / (N - 1)
+        cs = self._beam_table(angle_min, angle_max, N)
+        best = np.empty(K, dtype=np.int32)
+        pose = np.empty((K, 3))
+        score = np.empty((K, H))
+        iters = np.empty((K, H), dtype=np.int32)
+        T = np.empty((K, H, 3, 3)) if return_T else None
+        _lib.check(self._L.b2s_icp_relocalize(
+            self._h, _lib.ptr(ranges), _lib.ptr(candidates), _lib.ptr(cs), float(clamp_inf_to or 0.0), K, H, N,
+            float(angle_min), float(angle_increment), float(far_range),
+            self.max_iter if max_iter is None else int(max_iter),
+            self.tolerance if tolerance is None else float(tolerance),
+            _lib.ptr(best), _lib.ptr(pose), _lib.ptr(score), _lib.ptr(iters), _lib.ptr(T)))
+        out = (best, pose, score, iters) + ((T,) if return_T else ())
+        return tuple(a[0] for a in out) if one else out
+
     def process_scans(self, ranges, angle_min, angle_max, clamp_inf_to=None, state=None, max_iter=None,
                       tolerance=None):
         """process_sequence / odometry fed with what the sensor delivers: ranges (K,N) float32 (LaserScan.ranges of

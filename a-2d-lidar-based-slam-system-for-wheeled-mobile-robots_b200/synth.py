@@ -175,6 +175,53 @@ def room_map_observation(seed, scans, n_beams, pose_sigma=(0.03, 0.03, 0.02)):
             "obstacles_fine": _wall_cells(poly, 0.01, 2600, 0.25)}
 
 
+def _polygon_inside(poly, x, y):
+    """Even-odd point-in-polygon test of the points (x, y)."""
+    inside = np.zeros(x.shape, dtype=bool)
+    for a, b in zip(poly, np.roll(poly, -1, axis=0)):
+        crosses = (a[1] > y) != (b[1] > y)
+        with np.errstate(divide="ignore", invalid="ignore"):
+            xc = a[0] + (y - a[1]) * (b[0] - a[0]) / (b[1] - a[1])
+        inside ^= crosses & (x < xc)
+    return inside
+
+
+def _polygon_wall_distance(poly, x, y):
+    """Distance from the points (x, y) to the nearest edge of the polygon."""
+    d = np.full(x.shape, np.inf)
+    for a, b in zip(poly, np.roll(poly, -1, axis=0)):
+        e = b - a
+        t = np.clip(((x - a[0]) * e[0] + (y - a[1]) * e[1]) / (e @ e), 0.0, 1.0)
+        d = np.minimum(d, np.hypot(x - a[0] - t * e[0], y - a[1] - t * e[1]))
+    return d
+
+
+def room_relocalization(seed, scans, n_beams, xy_step=0.5, yaw_step_deg=10):
+    """Relocalization on the cfg-2 room: the scans and true poses of room_sequence's trajectory, the course obstacle
+    map of room_map_observation, and a grid of candidate poses over the room's free interior that knows nothing of
+    the trajectory.
+
+    The candidates are the centres of the xy_step grid cells, aligned on the origin, whose centre lies inside the
+    room at least 0.3 m from any wall, each at the yaws -pi + i * yaw_step_deg (i = 0 .. 360 / yaw_step_deg - 1),
+    x-major, then y, then yaw.  With seed 9001 and the defaults that is 759 cells x 36 yaws = 27 324 candidates.
+
+    Returns a dict: ranges float32 (scans, n_beams) (beam angles linspace(-pi, pi, n_beams)), poses float64
+    (scans, 3) the true poses, obstacles_course (2, C), candidates float64 (H, 3), poly the room polygon (12, 2).
+    """
+    poly, r, poses, _ = _room_ranges(seed, scans, n_beams)
+    lim = np.abs(poly).max()
+    c = np.arange(-np.ceil(lim / xy_step), np.ceil(lim / xy_step) + 1) * xy_step
+    gx, gy = np.meshgrid(c, c, indexing="ij")
+    gx, gy = gx.ravel(), gy.ravel()
+    keep = _polygon_inside(poly, gx, gy) & (_polygon_wall_distance(poly, gx, gy) >= 0.3)
+    yaw_count = int(round(360.0 / yaw_step_deg))
+    yaws = -np.pi + np.arange(yaw_count) * np.deg2rad(yaw_step_deg)
+    xy = np.stack([gx[keep], gy[keep]], axis=1)
+    cand = np.concatenate([np.repeat(xy, yaw_count, axis=0), np.tile(yaws, xy.shape[0])[:, None]], axis=1)
+    return {"ranges": r.astype(np.float32), "poses": poses, "obstacles_course": _wall_cells(poly, 0.155, 129, 0.2),
+            "candidates": np.ascontiguousarray(cand), "poly": poly}
+
+
 # ------------------------------------------------------------------ cfg 3 / 5: grid streams
 
 def grid_scan_ranges(seed, scans, n_beams, half_extent_m=80.0, step_m=0.1):

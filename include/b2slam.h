@@ -88,6 +88,12 @@ int b2s_icp_batch_ranges(const float *tar_ranges, const float *src_ranges, const
                          int32_t *iters_out, void *stream);
 int b2s_icp_batch_f64(const double *tar_xy, const double *src_xy, int pairs, int n_src, int n_tar,
                       int max_iter, double tol, double *T_out, int32_t *iters_out, void *stream);
+/* b2s_icp_batch_f64 that also reports each pair's score: err_out [pairs] (may be NULL) receives the reference's
+ * mean_error = sum(dist) / N of the last iteration that ran ([ICP]:75-76), i.e. the mean matched distance before that
+ * iteration's move and the value the stop rule last compared; unmatched (inf / NaN) distances count as 0 ([ICP]:95).
+ * T_out and iters_out are those of b2s_icp_batch_f64, bit for bit.  max_iter == 0 gives 0. */
+int b2s_icp_batch_f64_err(const double *tar_xy, const double *src_xy, int pairs, int n_src, int n_tar,
+                          int max_iter, double tol, double *T_out, int32_t *iters_out, double *err_out, void *stream);
 
 /* ICP.findNearest -- replaces [ICP]:90-114.  src_xy [n][2], tar_xy [m][2] (row = point, as the
  * reference passes them); dist_out [n] float64, idx_out [n] int64.  Lowest index wins ties. */
@@ -200,6 +206,15 @@ int b2s_virtual_scan_host(const double *obs_x, const double *obs_y, int count, d
 int b2s_virtual_scan_batch(const double *obs_x, const double *obs_y, int count, const double *poses3, int scans,
                            double angle_min, double angle_increment, int beams, double far_range,
                            const double *beam_cs, double *ranges, double *tar_xy, void *stream);
+/* Selection of a relocalization (no reference counterpart: the reference has no global localization; this picks among
+ * map observations, [LOC9]:128-157, at many candidate poses).  score [scans][hyps] (b2s_icp_batch_f64_err's err_out),
+ * T [scans][hyps][9] (the transforms of those solves), candidates3 [hyps][3] = x, y, yaw.  Per scan, best_out[k] is
+ * the h with the smallest score among the hypotheses whose score and all nine entries of T are finite, the lowest h
+ * on ties; pose_out[k] = candidates3[best] composed with T[k][best] by the pose-chain step of [ICP]:185-190
+ * (x + cos(yaw) T02 - sin(yaw) T12, y + sin(yaw) T02 + cos(yaw) T12, yaw + atan2(T10, T00)), in float64: the sensor pose
+ * in the map frame.  A scan without a finite hypothesis gets -1 and a NaN pose. */
+int b2s_relocalize_select(const double *score, const double *T, const double *candidates3, int scans, int hyps,
+                          int32_t *best_out, double *pose_out, void *stream);
 
 /* Sum of per-GPU count deltas (no reference counterpart: the reference is single-process).
  * In-place ncclAllReduce(int32, sum) of both planes on an existing communicator. */
@@ -329,6 +344,18 @@ int b2s_icp_map_observation(b2s_icp *icp, const float *ranges, const double *pos
                             double clamp_inf_to, int scans, int n, double angle_min, double angle_increment,
                             double far_range, int max_iter, double tol, double *T_out, int32_t *iters_out,
                             double *virtual_out);
+/* Relocalization in the static map: the map observation ([LOC9]:128-157) of each scan at every candidate pose,
+ * scored and chosen on the device.  ranges [scans][n], candidates3 [hyps][3] = x, y, yaw, shared by all scans.
+ * Hypothesis (k, h) is b2s_icp_map_observation of ranges[k] at candidates3[h], bit for bit: the virtual scans are built
+ * once per call and reused for every scan.  score_out [scans][hyps] is its mean_error of the last iteration
+ * ([ICP]:75-76), iters_out [scans][hyps] and T_out [scans][hyps][9] its iterations and transform; best_out [scans] and
+ * pose_out [scans][3] come from b2s_relocalize_select ([ICP]:185-190).  score_out, iters_out and T_out may be NULL.
+ * hyps >= 1, n <= 2304.  A NaN candidate fails with B2S_ERR_NONFINITE before anything runs; no map set is
+ * B2S_ERR_INVALID_ARG. */
+int b2s_icp_relocalize(b2s_icp *icp, const float *ranges, const double *candidates3, const double *beam_cs,
+                       double clamp_inf_to, int scans, int hyps, int n, double angle_min, double angle_increment,
+                       double far_range, int max_iter, double tol, int32_t *best_out, double *pose_out,
+                       double *score_out, int32_t *iters_out, double *T_out);
 int b2s_icp_find_nearest(b2s_icp *icp, const double *src_xy, int n, const double *tar_xy, int m,
                          double *dist_out, int64_t *idx_out);
 int b2s_icp_get_transform(b2s_icp *icp, const double *src_xy, const double *tar_xy, int n,
