@@ -26,11 +26,33 @@ def env():
     return e
 
 
+# Every kernel arm as (grid_variant, grid_tile_layout).  The default, variant 6 with tile layout 1, is what Mapping,
+# the streamed calls and bench.py run; a loop over ARMS checks it beside the older variants.  Variants 4-6 are given a
+# workspace: b2s_grid_raycast_ws without one runs variant 3, whatever is selected.
+ARMS = ((1, 1), (2, 1), (3, 1), (4, 1), (5, 1), (6, 0), (6, 1))
+DEFAULT_ARM = (6, 1)
+
+
+def _select(env, arm):
+    L = env.lib.lib()
+    assert L.b2s_tune(b"grid_variant", arm[0]) == 0 and L.b2s_tune(b"grid_tile_layout", arm[1]) == 0
+
+
+@pytest.fixture(autouse=True)
+def _default_kernel(env):
+    """Every test starts on the default kernel and leaves it selected, whether it passes or fails."""
+    _select(env, DEFAULT_ARM)
+    try:
+        yield
+    finally:
+        _select(env, DEFAULT_ARM)
+
+
 def _variants(env):
-    for v in (1, 2, 3, 4, 5):
-        assert env.lib.lib().b2s_tune(b"grid_variant", v) == 0
-        yield v
-    env.lib.lib().b2s_tune(b"grid_variant", 5)
+    """Selects each arm in turn and yields (grid_variant, arm name); the fixture above puts the default back."""
+    for arm in ARMS:
+        _select(env, arm)
+        yield arm[0], ("v6/layout%d" % arm[1] if arm[0] == 6 else "v%d" % arm[0])
 
 
 # ----------------------------------------------------------------------------- bresenham (A7)
@@ -65,7 +87,7 @@ def test_bresenham_long_random_segments_vs_oracle(env):
 @pytest.mark.parametrize("tag,w_hit", [("w20", 20.0), ("w4", 4.0)])
 def test_mapping_class_reproduces_reference_maps(env, tag, w_hit):
     z = load_golden("mapping.npz")
-    for v in _variants(env):
+    for v, name in _variants(env):
         m = env.b2slam.Mapping(200, 200, 0.1, hit_weight=w_hit)
         assert m.pmap.shape == (200, 200) and (m.pmap == 50).all()
         for ox, oy, cx, cy in zip(z[tag + "_ox"], z[tag + "_oy"], z[tag + "_cx"], z[tag + "_cy"]):
@@ -74,7 +96,7 @@ def test_mapping_class_reproduces_reference_maps(env, tag, w_hit):
         oh = np.zeros((200, 200), dtype=np.int32)
         om = np.zeros((200, 200), dtype=np.int32)
         env.corc.grid_raycast(oh, om, 10.0, 10.0, 10.0, z[tag + "_ox"], z[tag + "_oy"], z[tag + "_cx"], z[tag + "_cy"])
-        assert np.array_equal(hit, oh) and np.array_equal(miss, om), "variant %d" % v
+        assert np.array_equal(hit, oh) and np.array_equal(miss, om), name
         amb = env.pyref.boundary_ambiguous(hit, miss, w_hit)
         assert ((pm == z[tag + "_pmap"]) | amb).all()
         if w_hit == 20.0:
@@ -152,7 +174,7 @@ def test_mapping_threshold_stream(env):
 def test_non_square_grid_and_generalised_scale(env):
     S, Hx, Hy = env.dev.grid_scale(300, 180, 0.05)
     ox, oy, cx, cy = env.synth.grid_scans(31, 12, 360, half_extent_m=3.0)
-    for v in _variants(env):
+    for v, name in _variants(env):
         m = env.b2slam.Mapping(300, 180, 0.05)
         m.update_batch(ox, oy, cx, cy)
         hit, miss = m.counts()
@@ -178,10 +200,10 @@ def test_cfg3_counts_bit_exact_vs_oracle(env):
     oh = np.zeros((G, G), dtype=np.int32)
     om = np.zeros((G, G), dtype=np.int32)
     visits = env.corc.grid_raycast(oh, om, S, Hx, Hy, *host)
-    for v in _variants(env):
+    for v, name in _variants(env):
         hit, miss = env.dev.new_planes(G, G)
         cnt = torch.zeros(4, dtype=torch.int32, device="cuda")
-        ws = env.dev.new_workspace(G, G) if v == 4 else None
+        ws = env.dev.new_workspace(G, G) if v >= 4 else None
         env.dev.grid_raycast(hit, miss, S, Hx, Hy, *devt, counters=cnt, workspace=ws)
         if ws is not None:  # the workspace comes back clean and is reusable
             torch.cuda.synchronize()
@@ -192,8 +214,8 @@ def test_cfg3_counts_bit_exact_vs_oracle(env):
             miss //= 2
         torch.cuda.synchronize()
         assert int(hit.sum().item() + miss.sum().item()) == visits
-        assert np.array_equal(hit.cpu().numpy(), oh), "variant %d" % v
-        assert np.array_equal(miss.cpu().numpy(), om), "variant %d" % v
+        assert np.array_equal(hit.cpu().numpy(), oh), name
+        assert np.array_equal(miss.cpu().numpy(), om), name
         assert cnt.tolist() == [0, 0, 0, 0]
     pmap = torch.empty((G, G), dtype=torch.int8, device="cuda")
     score = torch.empty((G, G), dtype=torch.float32, device="cuda")
@@ -247,25 +269,17 @@ def test_cfg3_full_size_properties(env):
     S, Hx, Hy = env.dev.grid_scale(G, G, reso)
     _, devt = _device_scans(env, 12001, K, N, 80.0)
     ox, oy, cx, cy = devt
-    env.lib.lib().b2s_tune(b"grid_variant", 1)
+    _select(env, ARMS[0])
     h1, m1 = env.dev.new_planes(G, G)
     env.dev.grid_raycast(h1, m1, S, Hx, Hy, ox, oy, cx, cy)
-    env.lib.lib().b2s_tune(b"grid_variant", 2)
     h2, m2 = env.dev.new_planes(G, G)
-    env.dev.grid_raycast(h2, m2, S, Hx, Hy, ox, oy, cx, cy)
-    assert torch.equal(h1, h2) and torch.equal(m1, m2)
-    env.lib.lib().b2s_tune(b"grid_variant", 3)
-    h2.zero_()
-    m2.zero_()
-    env.dev.grid_raycast(h2, m2, S, Hx, Hy, ox, oy, cx, cy)
-    assert torch.equal(h1, h2) and torch.equal(m1, m2)
     ws = env.dev.new_workspace(G, G)
-    for v in (4, 5):
-        env.lib.lib().b2s_tune(b"grid_variant", v)
+    for v, name in _variants(env):
         h2.zero_()
         m2.zero_()
-        env.dev.grid_raycast(h2, m2, S, Hx, Hy, ox, oy, cx, cy, workspace=ws)
-        assert torch.equal(h1, h2) and torch.equal(m1, m2), "variant %d" % v
+        env.dev.grid_raycast(h2, m2, S, Hx, Hy, ox, oy, cx, cy, workspace=ws if v >= 4 else None)
+        assert torch.equal(h1, h2) and torch.equal(m1, m2), name
+    _select(env, DEFAULT_ARM)
     # every beam of this workload ends inside the grid -> exactly one hit per non-degenerate beam
     assert int(h2.sum().item()) <= K * N and int(h2.sum().item()) > 0.99 * K * N
     # 4 emulated ranks: private delta planes summed == single pass (integer sums commute)
@@ -304,12 +318,12 @@ def test_clipping_out_of_grid_and_counters(env):
     om = np.zeros((G, G), dtype=np.int32)
     env.corc.grid_raycast(oh, om, S, Hx, Hy, ox, oy, cx, cy)
     assert om.sum() > 0
-    for v in _variants(env):
+    for v, name in _variants(env):
         hit, miss = env.dev.new_planes(G, G)
-        ws = env.dev.new_workspace(G, G) if v == 4 else None
+        ws = env.dev.new_workspace(G, G) if v >= 4 else None
         env.dev.grid_raycast(hit, miss, S, Hx, Hy, *[torch.from_numpy(a).cuda() for a in (ox, oy, cx, cy)],
                              workspace=ws)
-        assert np.array_equal(hit.cpu().numpy(), oh) and np.array_equal(miss.cpu().numpy(), om), v
+        assert np.array_equal(hit.cpu().numpy(), oh) and np.array_equal(miss.cpu().numpy(), om), name
     ox2 = ox.copy()
     oy2 = oy.copy()
     ox2[0, 0] = np.inf
@@ -433,12 +447,12 @@ def test_random_grids_all_variants_vs_oracle(env):
         om = np.zeros((xw, yw), dtype=np.int32)
         env.corc.grid_raycast(oh, om, S, Hx, Hy, ox, oy, cx, cy)
         dev = [torch.from_numpy(a).cuda() for a in (ox, oy, cx, cy)]
-        for v in _variants(env):
+        for v, name in _variants(env):
             hit, miss = env.dev.new_planes(xw, yw)
-            ws = env.dev.new_workspace(xw, yw) if v == 4 else None
+            ws = env.dev.new_workspace(xw, yw) if v >= 4 else None
             env.dev.grid_raycast(hit, miss, S, Hx, Hy, *dev, workspace=ws)
             ok = np.array_equal(hit.cpu().numpy(), oh) and np.array_equal(miss.cpu().numpy(), om)
-            assert ok, "trial %d variant %d grid %dx%d reso %g K %d N %d" % (trial, v, xw, yw, reso, K, N)
+            assert ok, "trial %d %s grid %dx%d reso %g K %d N %d" % (trial, name, xw, yw, reso, K, N)
         m = env.b2slam.Mapping(xw, yw, reso)
         pm = m.update_batch(ox, oy, cx, cy)
         assert np.array_equal(pm, env.corc.grid_finalize(oh, om)[1])

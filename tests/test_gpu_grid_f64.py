@@ -28,6 +28,26 @@ def env():
     return e
 
 
+# (grid_variant, grid_tile_layout) of every kernel arm; variant 6 with layout 1 is the default that Mapping runs
+ARMS = ((1, 1), (2, 1), (3, 1), (4, 1), (5, 1), (6, 0), (6, 1))
+DEFAULT_ARM = (6, 1)
+
+
+def _select(env, arm):
+    L = env.lib.lib()
+    assert L.b2s_tune(b"grid_variant", arm[0]) == 0 and L.b2s_tune(b"grid_tile_layout", arm[1]) == 0
+
+
+@pytest.fixture(autouse=True)
+def _default_kernel(env):
+    """Every test starts on the default kernel and leaves it selected, whether it passes or fails."""
+    _select(env, DEFAULT_ARM)
+    try:
+        yield
+    finally:
+        _select(env, DEFAULT_ARM)
+
+
 def _sparse_check(hit, miss, z, tag, w_hit=20.0, suffix=""):
     cells = z[tag + "_cells" + suffix]
     h, m = hit.reshape(-1), miss.reshape(-1)
@@ -46,28 +66,26 @@ def test_layer1_float64_raycast_equals_reference(env, tag):
     ox, oy, cx, cy = (torch.from_numpy(np.ascontiguousarray(z[tag + k])).cuda() for k in ("_ox", "_oy", "_cx", "_cy"))
     assert ox.dtype == torch.float64
     ws = env.dev.new_workspace(side, side)
-    variants = (1, 2, 3, 4, 5) if side <= 4096 else (4, 5)
-    try:
-        for v in variants:
-            assert env.lib.lib().b2s_tune(b"grid_variant", v) == 0
-            for workspace in (ws, None):
-                hit, miss = env.dev.new_planes(side, side)
-                cnt = torch.zeros(4, dtype=torch.int32, device="cuda")
-                env.dev.grid_raycast(hit, miss, 10.0, 10.0, 10.0, ox, oy, cx, cy, counters=cnt, workspace=workspace)
-                torch.cuda.synchronize()
-                c = cnt.cpu().numpy()
-                assert c[0] == 0 and c[1] == 0 and c[3] == 0 and c[2] == int(np.isinf(z[tag + "_ox"]).sum())
-                _sparse_check(hit.cpu().numpy(), miss.cpu().numpy(), z, tag)
-                pm = torch.empty((side, side), dtype=torch.int8, device="cuda")
-                env.dev.grid_finalize(hit, miss, pmap=pm)
-                pmh = pm.cpu().numpy().reshape(-1)
-                assert np.array_equal(pmh[z[tag + "_cells"]], z[tag + "_pmap"])
-                rest = np.ones(side * side, dtype=bool)
-                rest[z[tag + "_cells"]] = False
-                assert (pmh[rest] == 50).all()
-                del hit, miss, pm
-    finally:
-        env.lib.lib().b2s_tune(b"grid_variant", 5)
+    arms = ARMS if side <= 4096 else ((4, 1), (5, 1), (6, 0), (6, 1))
+    for arm in arms:
+        _select(env, arm)
+        # without a workspace b2s_grid_raycast_ws_f64 runs variant 3 whatever is selected
+        for workspace in (ws, None):
+            hit, miss = env.dev.new_planes(side, side)
+            cnt = torch.zeros(4, dtype=torch.int32, device="cuda")
+            env.dev.grid_raycast(hit, miss, 10.0, 10.0, 10.0, ox, oy, cx, cy, counters=cnt, workspace=workspace)
+            torch.cuda.synchronize()
+            c = cnt.cpu().numpy()
+            assert c[0] == 0 and c[1] == 0 and c[3] == 0 and c[2] == int(np.isinf(z[tag + "_ox"]).sum()), arm
+            _sparse_check(hit.cpu().numpy(), miss.cpu().numpy(), z, tag)
+            pm = torch.empty((side, side), dtype=torch.int8, device="cuda")
+            env.dev.grid_finalize(hit, miss, pmap=pm)
+            pmh = pm.cpu().numpy().reshape(-1)
+            assert np.array_equal(pmh[z[tag + "_cells"]], z[tag + "_pmap"]), arm
+            rest = np.ones(side * side, dtype=bool)
+            rest[z[tag + "_cells"]] = False
+            assert (pmh[rest] == 50).all(), arm
+            del hit, miss, pm
 
 
 @pytest.mark.parametrize("w_hit,suffix", [(20.0, ""), (4.0, "_w4")])
