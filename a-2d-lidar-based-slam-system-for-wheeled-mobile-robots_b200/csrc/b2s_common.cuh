@@ -42,6 +42,10 @@ int laser_points(const float *ranges, const double *beam_cs, double clamp, int s
                  cudaStream_t stream);
 // `copies` consecutive copies of the `row` doubles at src into dst (b2s_next.cu).
 int replicate_row(const double *src, size_t row, size_t copies, double *dst, cudaStream_t stream);
+// Refinement rows of a coarse-to-fine relocalization (b2s_next.cu): pair k * keep + j gets target row kept[k][j] of
+// `tar` and source row k of `src` (rows of `row` doubles) in tar_out / src_out.
+int relocalize_gather(const double *tar, const double *src, const int32_t *kept, int scans, int keep, size_t row,
+                      double *tar_out, double *src_out, cudaStream_t stream);
 
 // Growable device / pinned-host staging buffer.
 struct Buf {

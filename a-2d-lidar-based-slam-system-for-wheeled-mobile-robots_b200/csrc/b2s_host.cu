@@ -916,50 +916,63 @@ extern "C" int b2s_icp_map_observation(b2s_icp *c, const float *ranges, const do
     return icp_read_back(c, tr, scans, T_out, iters_out);
 }
 
-// Relocalization: the map observation of every scan at every candidate.  The H virtual scans depend on the candidate
-// only, so they are built once into the target layout and shared by all scans; per scan, laserToNumpy forms its source
-// cloud once, replicated into the H source rows, and the H-pair ICP runs with its score output, the scans alternating
-// between stream and stream2.  One selection launch over all scans follows on stream, then the read-back.
-extern "C" int b2s_icp_relocalize(b2s_icp *c, const float *ranges, const double *candidates3, const double *beam_cs,
-                                  double clamp_inf_to, int scans, int hyps, int n, double angle_min, double angle_increment,
-                                  double far_range, int max_iter, double tol, int32_t *best_out, double *pose_out,
-                                  double *score_out, int32_t *iters_out, double *T_out)
+static int invalid(const char *fn, const char *what)
 {
-    B2S_REQUIRE(scans >= 0 && hyps > 0 && n > 0 && max_iter >= 0 && (long long)scans * hyps <= 0x7fffffffLL,
-                "b2s_icp_relocalize: bad sizes");
+    set_error("%s: %s", fn, what);
+    return B2S_ERR_INVALID_ARG;
+}
+
+// The argument checks the relocalization calls share, with the messages of the call `fn`.
+static int relocalize_check(const char *fn, b2s_icp *c, const float *ranges, const double *candidates3,
+                            const double *beam_cs, double clamp_inf_to, int scans, int hyps, int n,
+                            double angle_increment, int max_iter, double tol, const void *best_out, const void *pose_out)
+{
+    if (!(scans >= 0 && hyps > 0 && n > 0 && max_iter >= 0 && (long long)scans * hyps <= 0x7fffffffLL))
+        return invalid(fn, "bad sizes");
     B2S_REQUIRE(n <= ICP_MAX_POINTS, "b2s_icp_batch: more than 2304 source points per scan is not supported");
-    B2S_REQUIRE(angle_increment != 0.0 && angle_increment == angle_increment, "b2s_icp_relocalize: angle_increment");
-    B2S_REQUIRE(clamp_inf_to == clamp_inf_to && tol == tol, "b2s_icp_relocalize: NaN clamp / tolerance");
-    B2S_REQUIRE(c, "b2s_icp_relocalize: null handle");
-    B2S_REQUIRE(c->map_count > 0, "b2s_icp_relocalize: no static map set (b2s_icp_set_map)");
+    if (!(angle_increment != 0.0 && angle_increment == angle_increment)) return invalid(fn, "angle_increment");
+    if (!(clamp_inf_to == clamp_inf_to && tol == tol)) return invalid(fn, "NaN clamp / tolerance");
+    if (!c) return invalid(fn, "null handle");
+    if (!(c->map_count > 0)) return invalid(fn, "no static map set (b2s_icp_set_map)");
     if (scans == 0) return B2S_OK;
-    B2S_REQUIRE(ranges && candidates3 && beam_cs && best_out && pose_out, "b2s_icp_relocalize: null pointer");
+    if (!(ranges && candidates3 && beam_cs && best_out && pose_out)) return invalid(fn, "null pointer");
     for (size_t i = 0; i < (size_t)hyps * 3; ++i)  // as in b2s_icp_map_observation
         if (candidates3[i] != candidates3[i]) {
             set_error("%s", NAN_TO_INT);
             return B2S_ERR_NONFINITE;
         }
-    DeviceGuard g(c->device);
-    Trace tr(c->stream);
+    return B2S_OK;
+}
+
+// Where relocalize_scans left its uploads and the H virtual scans (target rows of 2n doubles), for the steps after it.
+struct RelocInputs {
+    const double *cs, *cand;
+    const float *ranges;
+    const double *tar;
+};
+
+// The map observation of every scan at every candidate, as both relocalization calls run it.  The H virtual scans
+// depend on the candidate only, so they are built once into the target layout and shared by all scans; per scan,
+// laserToNumpy forms its source cloud once, replicated into the H source rows, and the H-pair ICP runs with max_iter
+// iterations and its score output into T / iters / score at k * H, the scans alternating between stream and stream2.
+// Everything after it is ordered on stream.
+static int relocalize_scans(b2s_icp *c, Trace &tr, const float *ranges, const double *candidates3, const double *beam_cs,
+                            double clamp_inf_to, int scans, int hyps, int n, double angle_min, double angle_increment,
+                            double far_range, int max_iter, double tol, double *d_T, int32_t *d_iters, double *d_score,
+                            const char *scan_mark, RelocInputs *in_out)
+{
     const size_t H = (size_t)hyps, K = (size_t)scans, cloud = H * 2 * n;  // doubles of one set of H clouds
     const size_t cs_bytes = (size_t)n * 2 * sizeof(double), cand_bytes = H * 3 * sizeof(double);
     const size_t cand_off = cs_bytes, range_off = (cand_off + cand_bytes + 15) & ~(size_t)15;
-    // d_aux: scores [K][H] | best [K] | poses [K][3] (+ one scan's source cloud per compute stream)
-    const size_t score_bytes = K * H * sizeof(double), best_off = score_bytes;
-    const size_t pose_off = (best_off + K * sizeof(int32_t) + 15) & ~(size_t)15, cloud_off = pose_off + K * 3 * sizeof(double);
     int rc;
     if ((rc = c->d_map_in.reserve(range_off + K * n * sizeof(float)))) return rc;
     if ((rc = c->d_map_tar.reserve(cloud * sizeof(double)))) return rc;
-    if ((rc = c->d_map_src.reserve(2 * cloud * sizeof(double)))) return rc;
-    if ((rc = c->d_T.reserve(K * H * 9 * sizeof(double)))) return rc;
-    if ((rc = c->d_iters.reserve(K * H * sizeof(int32_t)))) return rc;
-    if ((rc = c->d_aux.reserve(cloud_off + 2 * cs_bytes))) return rc;
-    char *in = (char *)c->d_map_in.p, *aux = (char *)c->d_aux.p;
+    // d_map_src: the H source rows per compute stream, then one scan's source cloud per compute stream
+    if ((rc = c->d_map_src.reserve((2 * cloud + 4 * (size_t)n) * sizeof(double)))) return rc;
+    char *in = (char *)c->d_map_in.p;
     const double *d_cs = (const double *)in, *d_cand = (const double *)(in + cand_off);
     const float *d_ranges = (const float *)(in + range_off);
-    double *d_tar = (double *)c->d_map_tar.p, *d_T = (double *)c->d_T.p, *d_score = (double *)aux;
-    int32_t *d_iters = (int32_t *)c->d_iters.p, *d_best = (int32_t *)(aux + best_off);
-    double *d_pose = (double *)(aux + pose_off);
+    double *d_tar = (double *)c->d_map_tar.p;
     const double *map_x = (const double *)c->d_map.p, *map_y = map_x + c->map_count;
     // (every call ends with a synchronize, so the device buffers are free to overwrite here)
     B2S_CUDA(cudaMemcpyAsync(in, beam_cs, cs_bytes, cudaMemcpyHostToDevice, c->stream));
@@ -973,24 +986,120 @@ extern "C" int b2s_icp_relocalize(b2s_icp *c, const float *ranges, const double 
     B2S_CUDA(cudaStreamWaitEvent(c->stream2, c->chunk_ready[0], 0));
     for (size_t k = 0; k < K; ++k) {
         cudaStream_t ks = (k & 1) ? c->stream2 : c->stream;
-        double *one = (double *)(aux + cloud_off) + (k & 1) * 2 * n, *src = (double *)c->d_map_src.p + (k & 1) * cloud;
+        double *src = (double *)c->d_map_src.p + (k & 1) * cloud, *one = (double *)c->d_map_src.p + 2 * cloud + (k & 1) * 2 * n;
         if ((rc = laser_points(d_ranges + k * n, d_cs, clamp_inf_to, 1, n, one, ks))) return rc;
         if ((rc = replicate_row(one, (size_t)2 * n, H, src, ks))) return rc;
         if ((rc = b2s_icp_batch_f64_err(d_tar, src, hyps, n, n, max_iter, tol, d_T + k * H * 9, d_iters + k * H,
                                         d_score + k * H, ks)))
             return rc;
-        tr.mark("relocalize scan done", (int)k, ks);
+        tr.mark(scan_mark, (int)k, ks);
     }
     if (K > 1) {
         B2S_CUDA(cudaEventRecord(c->joined, c->stream2));
         B2S_CUDA(cudaStreamWaitEvent(c->stream, c->joined, 0));
     }
-    if ((rc = b2s_relocalize_select(d_score, d_T, d_cand, scans, hyps, d_best, d_pose, c->stream))) return rc;
+    *in_out = {d_cs, d_cand, d_ranges, d_tar};
+    return B2S_OK;
+}
+
+// Relocalization: the map observation of every scan at every candidate (relocalize_scans), then one selection launch
+// over all scans on stream and the read-back.
+extern "C" int b2s_icp_relocalize(b2s_icp *c, const float *ranges, const double *candidates3, const double *beam_cs,
+                                  double clamp_inf_to, int scans, int hyps, int n, double angle_min, double angle_increment,
+                                  double far_range, int max_iter, double tol, int32_t *best_out, double *pose_out,
+                                  double *score_out, int32_t *iters_out, double *T_out)
+{
+    int rc = relocalize_check("b2s_icp_relocalize", c, ranges, candidates3, beam_cs, clamp_inf_to, scans, hyps, n,
+                              angle_increment, max_iter, tol, best_out, pose_out);
+    if (rc || scans == 0) return rc;
+    DeviceGuard g(c->device);
+    Trace tr(c->stream);
+    const size_t H = (size_t)hyps, K = (size_t)scans;
+    // d_aux: scores [K][H] | best [K] | poses [K][3]
+    const size_t score_bytes = K * H * sizeof(double), best_off = score_bytes;
+    const size_t pose_off = (best_off + K * sizeof(int32_t) + 15) & ~(size_t)15;
+    if ((rc = c->d_T.reserve(K * H * 9 * sizeof(double)))) return rc;
+    if ((rc = c->d_iters.reserve(K * H * sizeof(int32_t)))) return rc;
+    if ((rc = c->d_aux.reserve(pose_off + K * 3 * sizeof(double)))) return rc;
+    char *aux = (char *)c->d_aux.p;
+    double *d_score = (double *)aux, *d_pose = (double *)(aux + pose_off);
+    int32_t *d_best = (int32_t *)(aux + best_off);
+    RelocInputs in;
+    if ((rc = relocalize_scans(c, tr, ranges, candidates3, beam_cs, clamp_inf_to, scans, hyps, n, angle_min,
+                               angle_increment, far_range, max_iter, tol, (double *)c->d_T.p, (int32_t *)c->d_iters.p,
+                               d_score, "relocalize scan done", &in)))
+        return rc;
+    if ((rc = b2s_relocalize_select(d_score, (const double *)c->d_T.p, in.cand, scans, hyps, d_best, d_pose, c->stream)))
+        return rc;
     tr.mark("select done", 0, c->stream);
     B2S_CUDA(cudaMemcpyAsync(best_out, d_best, K * sizeof(int32_t), cudaMemcpyDeviceToHost, c->stream));
     B2S_CUDA(cudaMemcpyAsync(pose_out, d_pose, K * 3 * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
     if (score_out) B2S_CUDA(cudaMemcpyAsync(score_out, d_score, score_bytes, cudaMemcpyDeviceToHost, c->stream));
     return icp_read_back(c, tr, (int)(K * H), T_out, iters_out);
+}
+
+// Coarse-to-fine relocalization: relocalize_scans with coarse_iters iterations into scratch, the keep step, the
+// survivors' target rows gathered out of the H virtual scans and each scan's source cloud replicated beside them, one
+// ICP launch over all K * M survivors with max_iter (from the candidate, not from the coarse state, so that each
+// survivor's result is the exhaustive call's), the selection among them, then the read-back.  The refined T and
+// iterations go to d_T / d_iters, so the read-back is icp_read_back's.
+extern "C" int b2s_icp_relocalize_keep(b2s_icp *c, const float *ranges, const double *candidates3, const double *beam_cs,
+                                       double clamp_inf_to, int scans, int hyps, int n, double angle_min,
+                                       double angle_increment, double far_range, int max_iter, double tol, int keep,
+                                       int coarse_iters, int32_t *best_out, double *pose_out, int32_t *kept_out,
+                                       double *score_out, int32_t *iters_out, double *T_out)
+{
+    const char *fn = "b2s_icp_relocalize_keep";
+    if (keep < 1) return invalid(fn, "keep must be >= 1");
+    if (coarse_iters < 1 || coarse_iters > max_iter) return invalid(fn, "coarse_iters must be in [1, max_iter]");
+    const int M = keep < hyps ? keep : hyps;
+    if ((long long)scans * M > 0x7fffffffLL) return invalid(fn, "scans * min(keep, hyps) exceeds 2^31 - 1");
+    int rc = relocalize_check(fn, c, ranges, candidates3, beam_cs, clamp_inf_to, scans, hyps, n, angle_increment,
+                              max_iter, tol, best_out, pose_out);
+    if (rc || scans == 0) return rc;
+    DeviceGuard g(c->device);
+    Trace tr(c->stream);
+    const size_t H = (size_t)hyps, K = (size_t)scans, row = (size_t)2 * n;
+    auto a16 = [](size_t b) { return (b + 15) & ~(size_t)15; };
+    // d_aux: coarse scores [K][H] | coarse T [K][H][9] | keys [K][H] | coarse iterations [K][H] | kept [K][M] |
+    //        refined scores [K][M] | best [K] | poses [K][3] | source clouds [K][2n]
+    const size_t T1_off = K * H * sizeof(double), key_off = T1_off + K * H * 9 * sizeof(double);
+    const size_t it1_off = key_off + K * H * sizeof(uint64_t), kept_off = a16(it1_off + K * H * sizeof(int32_t));
+    const size_t score_off = a16(kept_off + K * M * sizeof(int32_t)), best_off = score_off + K * M * sizeof(double);
+    const size_t pose_off = a16(best_off + K * sizeof(int32_t)), cloud_off = pose_off + K * 3 * sizeof(double);
+    if ((rc = c->d_aux.reserve(cloud_off + K * row * sizeof(double)))) return rc;
+    if ((rc = c->d_tar.reserve(K * M * row * sizeof(double)))) return rc;
+    if ((rc = c->d_src.reserve(K * M * row * sizeof(double)))) return rc;
+    if ((rc = c->d_T.reserve(K * M * 9 * sizeof(double)))) return rc;
+    if ((rc = c->d_iters.reserve(K * M * sizeof(int32_t)))) return rc;
+    char *aux = (char *)c->d_aux.p;
+    double *d_score1 = (double *)aux, *d_T1 = (double *)(aux + T1_off), *d_score = (double *)(aux + score_off);
+    double *d_pose = (double *)(aux + pose_off), *d_cloud = (double *)(aux + cloud_off);
+    int32_t *d_it1 = (int32_t *)(aux + it1_off), *d_kept = (int32_t *)(aux + kept_off), *d_best = (int32_t *)(aux + best_off);
+    RelocInputs in;
+    if ((rc = relocalize_scans(c, tr, ranges, candidates3, beam_cs, clamp_inf_to, scans, hyps, n, angle_min,
+                               angle_increment, far_range, coarse_iters, tol, d_T1, d_it1, d_score1, "coarse scan done",
+                               &in)))
+        return rc;
+    if ((rc = b2s_relocalize_keep(d_score1, d_T1, scans, hyps, M, (uint64_t *)(aux + key_off), d_kept, c->stream)))
+        return rc;
+    tr.mark("keep done", 0, c->stream);
+    double *d_tar = (double *)c->d_tar.p, *d_src = (double *)c->d_src.p;
+    if ((rc = laser_points(in.ranges, in.cs, clamp_inf_to, scans, n, d_cloud, c->stream))) return rc;
+    if ((rc = relocalize_gather(in.tar, d_cloud, d_kept, scans, M, row, d_tar, d_src, c->stream))) return rc;
+    if ((rc = b2s_icp_batch_f64_err(d_tar, d_src, scans * M, n, n, max_iter, tol, (double *)c->d_T.p,
+                                    (int32_t *)c->d_iters.p, d_score, c->stream)))
+        return rc;
+    tr.mark("refine done", 0, c->stream);
+    if ((rc = b2s_relocalize_select_kept(d_score, (const double *)c->d_T.p, in.cand, d_kept, scans, M, d_best, d_pose,
+                                         c->stream)))
+        return rc;
+    tr.mark("select done", 0, c->stream);
+    B2S_CUDA(cudaMemcpyAsync(best_out, d_best, K * sizeof(int32_t), cudaMemcpyDeviceToHost, c->stream));
+    B2S_CUDA(cudaMemcpyAsync(pose_out, d_pose, K * 3 * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
+    if (kept_out) B2S_CUDA(cudaMemcpyAsync(kept_out, d_kept, K * M * sizeof(int32_t), cudaMemcpyDeviceToHost, c->stream));
+    if (score_out) B2S_CUDA(cudaMemcpyAsync(score_out, d_score, K * M * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
+    return icp_read_back(c, tr, scans * M, T_out, iters_out);
 }
 
 extern "C" int b2s_icp_find_nearest(b2s_icp *c, const double *src_xy, int n, const double *tar_xy,

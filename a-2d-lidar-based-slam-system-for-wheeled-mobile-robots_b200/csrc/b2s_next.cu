@@ -8,7 +8,8 @@
 //                 reduces each pose's bins in shared memory and can write them as the ICP's target cloud.
 //   laserToNumpy  [ICP]:216-229 / [SLAM]:115-123 of float32 ranges into float64 points (the ICP's source cloud).
 //   relocalize    the selection among map observations at many candidate poses: per scan the lowest finite
-//                 mean_error ([ICP]:75), ties to the lower index, composed with its candidate ([ICP]:185-190).
+//                 mean_error ([ICP]:75), ties to the lower index, composed with its candidate ([ICP]:185-190); for the
+//                 coarse-to-fine form, the `keep` best coarse hypotheses per scan (radix select) and their rows.
 #include "b2s_common.cuh"
 
 #include <math.h>
@@ -17,29 +18,31 @@ namespace b2s {
 
 constexpr int CHAIN_THREADS = 1024;
 
-// Exclusive prefix over the CTA of one double per thread; returns this thread's offset, total in *total.
-__device__ __forceinline__ double cta_exclusive_scan(double v, double *scratch, double *total)
+// Exclusive prefix over a CTA of 1024 threads of one value per thread; returns this thread's offset, total in *total.
+// scratch: 64 values of shared memory.
+template <class V>
+__device__ __forceinline__ V cta_exclusive_scan(V v, V *scratch, V *total)
 {
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    double inc = v;
+    V inc = v;
 #pragma unroll
     for (int o = 1; o < 32; o <<= 1) {
-        const double up = __shfl_up_sync(0xffffffffu, inc, o);
+        const V up = __shfl_up_sync(0xffffffffu, inc, o);
         if (lane >= o) inc += up;
     }
     if (lane == 31) scratch[warp] = inc;
     __syncthreads();
     if (warp == 0) {
-        double w = scratch[lane];  // CHAIN_THREADS / 32 == 32 warps
+        V w = scratch[lane];  // CHAIN_THREADS / 32 == 32 warps
 #pragma unroll
         for (int o = 1; o < 32; o <<= 1) {
-            const double up = __shfl_up_sync(0xffffffffu, w, o);
+            const V up = __shfl_up_sync(0xffffffffu, w, o);
             if (lane >= o) w += up;
         }
         scratch[32 + lane] = w;  // inclusive over warps
     }
     __syncthreads();
-    const double before_warp = warp ? scratch[32 + warp - 1] : 0.0;
+    const V before_warp = warp ? scratch[32 + warp - 1] : V(0);
     *total = scratch[63];
     __syncthreads();
     return before_warp + inc - v;
@@ -222,6 +225,8 @@ replicate_row_kernel(const double *__restrict__ src, size_t row, size_t copies, 
 // whose score and transform are finite, then composes the winner's pose.  (score, h) with the lower h winning equal
 // scores is a strict total order in which every h occurs once, so the minimum is one element whatever the order of
 // the comparisons: the result does not depend on the CTA's thread count or on how the reduction is cut.
+// KEPT: row j of scan k is candidate kept[k][j] (the survivors of relocalize_keep_kernel, ascending), so the lowest j
+// among equal scores is also the lowest candidate; the candidate is reported and composed.
 constexpr int SELECT_THREADS = 256;
 
 __device__ __forceinline__ void select_better(double &bs, int &bh, double s, int h)
@@ -232,10 +237,11 @@ __device__ __forceinline__ void select_better(double &bs, int &bh, double s, int
     }
 }
 
+template <bool KEPT>
 __global__ void __launch_bounds__(SELECT_THREADS)
 relocalize_select_kernel(const double *__restrict__ score, const double *__restrict__ T,
-                         const double *__restrict__ cand, int hyps, int32_t *__restrict__ best_out,
-                         double *__restrict__ pose_out)
+                         const double *__restrict__ cand, const int32_t *__restrict__ kept, int hyps,
+                         int32_t *__restrict__ best_out, double *__restrict__ pose_out)
 {
     __shared__ double ws[SELECT_THREADS / 32];
     __shared__ int wh[SELECT_THREADS / 32];
@@ -264,7 +270,8 @@ relocalize_select_kernel(const double *__restrict__ score, const double *__restr
     __syncthreads();
     if (threadIdx.x != 0) return;
     for (int w = 1; w < (int)(blockDim.x >> 5); ++w) select_better(bs, bh, ws[w], wh[w]);
-    best_out[k] = bh;
+    const int bc = (KEPT && bh >= 0) ? kept[(size_t)k * hyps + bh] : bh;  // the winner's candidate
+    best_out[k] = bc;
     double *pose = pose_out + 3 * (size_t)k;
     if (bh < 0) {
         pose[0] = pose[1] = pose[2] = __longlong_as_double(0x7ff8000000000000LL);
@@ -272,11 +279,129 @@ relocalize_select_kernel(const double *__restrict__ score, const double *__restr
     }
     // [ICP]:185-190, the pose-chain step of one transform
     const double *t = Tk + (size_t)bh * 9;
-    const double x = cand[3 * (size_t)bh], y = cand[3 * (size_t)bh + 1], yaw = cand[3 * (size_t)bh + 2];
+    const double x = cand[3 * (size_t)bc], y = cand[3 * (size_t)bc + 1], yaw = cand[3 * (size_t)bc + 2];
     const double c = cos(yaw), s = sin(yaw);
     pose[0] = x + c * t[2] - s * t[5];
     pose[1] = y + s * t[2] + c * t[5];
     pose[2] = yaw + atan2(t[3], t[0]);
+}
+
+// Coarse-to-fine relocalization, the keep step: CTA k picks the `keep` best of scan k's `hyps` coarse hypotheses and
+// writes their indices to kept[k][0..keep) in ascending order.  Each hypothesis gets a 64-bit key that orders like
+// (finite score, with -0 == +0) and puts every non-finite hypothesis (score or any entry of T) above every finite one;
+// the keep-th smallest key is found by a radix select of 8-bit digits (a 256-bin histogram in shared memory per
+// digit, over the keys staged in `keys` [scans][hyps]), and the survivors are the keys below it plus, in ascending h,
+// as many of the keys equal to it as are still missing.  That is the first `keep` of the strict order (key, h), the
+// order of relocalize_select_kernel's finite rule followed by the non-finite hypotheses by h.
+constexpr int KEEP_THREADS = 1024;  // cta_exclusive_scan's CTA
+
+__device__ __forceinline__ unsigned long long keep_key(const double *__restrict__ s, const double *__restrict__ T, size_t h)
+{
+    bool finite = fabs(s[h]) < INFINITY;
+    for (int i = 0; i < 9; ++i) finite = finite && fabs(T[h * 9 + i]) < INFINITY;
+    if (!finite) return ~0ull;
+    unsigned long long b = (unsigned long long)__double_as_longlong(s[h]);
+    if (b == 0x8000000000000000ull) b = 0;  // -0.0 ties with +0.0
+    return (b >> 63) ? ~b : b | 0x8000000000000000ull;  // negative: all bits flipped; positive: the sign bit set
+}
+
+__global__ void __launch_bounds__(KEEP_THREADS)
+relocalize_keep_kernel(const double *__restrict__ score, const double *__restrict__ T, int hyps, int keep,
+                       unsigned long long *__restrict__ keys, int32_t *__restrict__ kept)
+{
+    __shared__ unsigned int hist[256];
+    __shared__ unsigned long long scratch[64];
+    __shared__ unsigned int pick[2];  // the digit of this pass, the rank still wanted among keys with its prefix
+    const int k = blockIdx.x, lane = threadIdx.x & 31;
+    const size_t H = (size_t)hyps;
+    const double *sk = score + (size_t)k * H, *Tk = T + (size_t)k * H * 9;
+    unsigned long long *key = keys + (size_t)k * H;
+    int32_t *out = kept + (size_t)k * keep;
+    unsigned long long prefix = 0, mask = 0;
+    unsigned int want = (unsigned int)keep;  // 1-based rank of the threshold among the keys that match prefix
+    for (int shift = 56; shift >= 0; shift -= 8) {
+        for (int i = threadIdx.x; i < 256; i += KEEP_THREADS) hist[i] = 0;
+        __syncthreads();
+        // warp-uniform trip count, so that every lane takes part in __match_any_sync
+        for (size_t base = threadIdx.x - lane; base < H; base += KEEP_THREADS) {
+            const size_t h = base + lane;
+            unsigned long long v = 0;
+            if (h < H) {
+                if (shift == 56) key[h] = v = keep_key(sk, Tk, h);  // every later pass of this thread reads its own h
+                else v = key[h];
+            }
+            const bool in = h < H && (v & mask) == prefix;
+            const unsigned int d = in ? (unsigned int)(v >> shift) & 255u : 256u;
+            const unsigned int peers = __match_any_sync(0xffffffffu, d);
+            if (in && lane == __ffs(peers) - 1) atomicAdd(&hist[d], (unsigned int)__popc(peers));
+        }
+        __syncthreads();
+        if (threadIdx.x < 32) {  // the digit whose bin holds rank `want`: lane l sums bins 8l .. 8l + 7
+            unsigned int sum = 0;
+#pragma unroll
+            for (int i = 0; i < 8; ++i) sum += hist[8 * lane + i];
+            unsigned int inc = sum;
+#pragma unroll
+            for (int o = 1; o < 32; o <<= 1) {
+                const unsigned int up = __shfl_up_sync(0xffffffffu, inc, o);
+                if (lane >= o) inc += up;
+            }
+            unsigned int before = inc - sum;
+            if (before < want && want <= inc) {
+                int d = 8 * lane;
+                while (before + hist[d] < want) before += hist[d++];
+                pick[0] = (unsigned int)d;
+                pick[1] = want - before;
+            }
+        }
+        __syncthreads();
+        prefix |= (unsigned long long)pick[0] << shift;
+        mask |= 255ull << shift;
+        want = pick[1];
+    }
+    // prefix is the keep-th key: the keys below it survive, and the first `want` of the keys equal to it.  One
+    // exclusive scan per tile of KEEP_THREADS hypotheses counts both (below: low word, equal: high word); a survivor's
+    // slot is the number of survivors before it, below + min(equal, want).
+    const unsigned int below_all = (unsigned int)keep - want;
+    unsigned long long seen = 0;
+    for (size_t base = 0; base < H; base += KEEP_THREADS) {
+        const size_t h = base + threadIdx.x;
+        const unsigned long long v = h < H ? key[h] : 0;
+        const bool lt = h < H && v < prefix, eq = h < H && v == prefix;
+        unsigned long long total;
+        const unsigned long long before = seen + cta_exclusive_scan<unsigned long long>(
+            (unsigned long long)lt | ((unsigned long long)eq << 32), scratch, &total);
+        const unsigned int lt_before = (unsigned int)before, eq_before = (unsigned int)(before >> 32);
+        if (lt || (eq && eq_before < want)) out[lt_before + min(eq_before, want)] = (int32_t)h;
+        seen += total;
+        if ((unsigned int)seen == below_all && (unsigned int)(seen >> 32) >= want) break;  // all survivors written
+    }
+}
+
+// Rows of the refinement of a coarse-to-fine relocalization: pair p = k * keep + j gets the target row of candidate
+// kept[p] (one of the `row`-double rows of `tar`, shared by every scan) and the source row of scan k.
+__global__ void __launch_bounds__(256)
+relocalize_gather_kernel(const double *__restrict__ tar, const double *__restrict__ src, const int32_t *__restrict__ kept,
+                         size_t keep, size_t row, size_t pairs, double *__restrict__ tar_out, double *__restrict__ src_out)
+{
+    const size_t total = row * pairs;
+    for (size_t j = (size_t)blockIdx.x * blockDim.x + threadIdx.x; j < total; j += (size_t)gridDim.x * blockDim.x) {
+        const size_t p = j / row, i = j - p * row;
+        tar_out[j] = tar[(size_t)kept[p] * row + i];
+        src_out[j] = src[(p / keep) * row + i];
+    }
+}
+
+int relocalize_gather(const double *tar, const double *src, const int32_t *kept, int scans, int keep, size_t row,
+                      double *tar_out, double *src_out, cudaStream_t st)
+{
+    const size_t total = row * (size_t)scans * keep;
+    if (total == 0) return B2S_OK;
+    const size_t want = (total + 255) / 256, cap = (size_t)sm_count() * 16;
+    relocalize_gather_kernel<<<(unsigned)(want < cap ? want : cap), 256, 0, st>>>(tar, src, kept, (size_t)keep, row,
+                                                                                  (size_t)scans * keep, tar_out, src_out);
+    B2S_CUDA(cudaGetLastError());
+    return B2S_OK;
 }
 
 int replicate_row(const double *src, size_t row, size_t copies, double *dst, cudaStream_t st)
@@ -391,8 +516,34 @@ extern "C" int b2s_relocalize_select(const double *score, const double *T, const
     B2S_REQUIRE(scans >= 0 && hyps > 0, "b2s_relocalize_select: bad sizes");
     if (scans == 0) return B2S_OK;
     B2S_REQUIRE(score && T && candidates3 && best_out && pose_out, "b2s_relocalize_select: null pointer");
-    relocalize_select_kernel<<<scans, SELECT_THREADS, 0, (cudaStream_t)stream>>>(score, T, candidates3, hyps, best_out,
-                                                                                 pose_out);
+    relocalize_select_kernel<false><<<scans, SELECT_THREADS, 0, (cudaStream_t)stream>>>(score, T, candidates3, nullptr, hyps,
+                                                                                        best_out, pose_out);
+    B2S_CUDA(cudaGetLastError());
+    return B2S_OK;
+}
+
+extern "C" int b2s_relocalize_select_kept(const double *score, const double *T, const double *candidates3,
+                                          const int32_t *kept, int scans, int keep, int32_t *best_out, double *pose_out,
+                                          void *stream)
+{
+    B2S_REQUIRE(scans >= 0 && keep > 0, "b2s_relocalize_select_kept: bad sizes");
+    if (scans == 0) return B2S_OK;
+    B2S_REQUIRE(score && T && candidates3 && kept && best_out && pose_out, "b2s_relocalize_select_kept: null pointer");
+    relocalize_select_kernel<true><<<scans, SELECT_THREADS, 0, (cudaStream_t)stream>>>(score, T, candidates3, kept, keep,
+                                                                                       best_out, pose_out);
+    B2S_CUDA(cudaGetLastError());
+    return B2S_OK;
+}
+
+extern "C" int b2s_relocalize_keep(const double *score, const double *T, int scans, int hyps, int keep, uint64_t *keys,
+                                   int32_t *kept_out, void *stream)
+{
+    B2S_REQUIRE(scans >= 0 && hyps > 0 && keep > 0 && (long long)scans * hyps <= 0x7fffffffLL,
+                "b2s_relocalize_keep: bad sizes");
+    if (scans == 0) return B2S_OK;
+    B2S_REQUIRE(score && T && keys && kept_out, "b2s_relocalize_keep: null pointer");
+    relocalize_keep_kernel<<<scans, KEEP_THREADS, 0, (cudaStream_t)stream>>>(score, T, hyps, keep < hyps ? keep : hyps,
+                                                                             (unsigned long long *)keys, kept_out);
     B2S_CUDA(cudaGetLastError());
     return B2S_OK;
 }

@@ -144,23 +144,57 @@ def icp_batch_err(tar, src, max_iter=30, tol=1e-3, T_out=None, iters_out=None, e
     return T_out, iters_out, err_out
 
 
-def relocalize_select(score, T, candidates, best_out=None, pose_out=None):
+def relocalize_select(score, T, candidates, best_out=None, pose_out=None, kept=None):
     """b2s_relocalize_select: score (K,H) float64, T (K,H,3,3) float64, candidates (H,3) float64 CUDA tensors ->
     (best (K,) int32, pose (K,3) float64): per scan the lowest-index smallest score among the hypotheses whose score
-    and T are finite (-1 and a NaN pose when none is), and candidates[best] composed with T[best] ([ICP]:185-190)."""
+    and T are finite (-1 and a NaN pose when none is), and candidates[best] composed with T[best] ([ICP]:185-190).
+
+    With kept (K,M) int32 (relocalize_keep's survivors, ascending per row), b2s_relocalize_select_kept: score (K,M)
+    and T (K,M,3,3) belong to candidates[kept[k, j]], and best is the original candidate index.  Every kept entry
+    must lie in [0, C) for candidates (C,3): like the other device-layer calls this one stays asynchronous, so the
+    entries are not checked here (relocalize_keep's output always satisfies it)."""
     K, H = score.shape
-    for t, shape, name in ((T, (K, H, 3, 3), "T"), (candidates, (H, 3), "candidates")):
+    want = ((T, (K, H, 3, 3), "T"),) + (((candidates, (H, 3), "candidates"),) if kept is None else
+                                        ((kept, (K, H), "kept"),))
+    for t, shape, name in want:
         if tuple(t.shape) != shape:
             raise ValueError("%s must have shape %s, got %s" % (name, shape, tuple(t.shape)))
+    if candidates.dim() != 2 or candidates.shape[1] != 3:
+        raise ValueError("candidates must have shape (C, 3), got %s" % (tuple(candidates.shape),))
     if best_out is None:
         best_out = torch.empty(K, dtype=torch.int32, device=score.device)
     if pose_out is None:
         pose_out = torch.empty((K, 3), dtype=torch.float64, device=score.device)
-    rc = _lib.lib().b2s_relocalize_select(
-        _chk(score, torch.float64, "score"), _chk(T, torch.float64, "T"), _chk(candidates, torch.float64, "candidates"),
-        K, H, _chk(best_out, torch.int32, "best_out"), _chk(pose_out, torch.float64, "pose_out"), _stream())
+    common = (_chk(score, torch.float64, "score"), _chk(T, torch.float64, "T"),
+              _chk(candidates, torch.float64, "candidates"))
+    outs = (_chk(best_out, torch.int32, "best_out"), _chk(pose_out, torch.float64, "pose_out"), _stream())
+    if kept is None:
+        rc = _lib.lib().b2s_relocalize_select(*common, K, H, *outs)
+    else:
+        rc = _lib.lib().b2s_relocalize_select_kept(*common, _chk(kept, torch.int32, "kept"), K, H, *outs)
     _lib.check(rc)
     return best_out, pose_out
+
+
+def relocalize_keep(score, T, keep, kept_out=None, keys=None):
+    """b2s_relocalize_keep: score (K,H) float64 and T (K,H,3,3) float64 CUDA tensors (coarse solves) -> kept (K,M)
+    int32, M = min(keep, H): per scan, in ascending h, the first M hypotheses of the order (score, h) over those whose
+    score and T are finite (-0 == +0), followed by every other hypothesis by h.  keys: (K*H,) int64 scratch."""
+    K, H = score.shape
+    if tuple(T.shape) != (K, H, 3, 3):
+        raise ValueError("T must have shape %s, got %s" % ((K, H, 3, 3), tuple(T.shape)))
+    M = max(0, min(int(keep), H))
+    if kept_out is None:
+        kept_out = torch.empty((K, M), dtype=torch.int32, device=score.device)
+    if keys is None:
+        keys = torch.empty(K * H, dtype=torch.int64, device=score.device)
+    if tuple(kept_out.shape) != (K, M) or keys.numel() < K * H:
+        raise ValueError("kept_out must be (%d, %d) and keys hold %d words" % (K, M, K * H))
+    rc = _lib.lib().b2s_relocalize_keep(
+        _chk(score, torch.float64, "score"), _chk(T, torch.float64, "T"), K, H, max(0, min(int(keep), 0x7fffffff)),
+        _chk(keys, torch.int64, "keys"), _chk(kept_out, torch.int32, "kept_out"), _stream())
+    _lib.check(rc)
+    return kept_out
 
 
 def virtual_scan_batch(obs_x, obs_y, poses, angle_min, angle_increment, beams, far_range=100.0, beam_cs=None,

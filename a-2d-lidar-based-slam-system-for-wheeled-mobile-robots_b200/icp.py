@@ -5,10 +5,16 @@ names, argument order (TARGET first), shapes and float64 NumPy in/out.  All arit
 in the CUDA library (include/b2slam.h); nothing here computes a distance or a fit.
 """
 import ctypes
+import operator
 
 import numpy as np
 
 from b2slam import _lib
+
+# ICP iterations of every hypothesis in the coarse stage of ICP.relocalize(keep=...) when coarse_iters is not given,
+# and the keep INTEGRATION.md recommends; both chosen from the measurement in DESIGN.md section 8, round 9.
+RELOCALIZE_COARSE_ITERS = 5
+RELOCALIZE_KEEP_RECOMMENDED = 1024
 
 
 def _ros_param(name, default):
@@ -298,7 +304,7 @@ class ICP(object):
         return (T, iters, virt) if return_virtual else (T, iters)
 
     def relocalize(self, ranges, candidates, angle_min, angle_max, angle_increment=None, clamp_inf_to=None,
-                   far_range=100.0, max_iter=None, tolerance=None, return_T=False):
+                   far_range=100.0, max_iter=None, tolerance=None, return_T=False, keep=None, coarse_iters=None):
         """Relocalization in the static map (set_static_map) for a robot whose pose is unknown: at start-up, after the
         EKF has diverged, or where a recorded stream starts at an unknown place.  The map observation is run at every
         candidate pose and the best one is kept; the caller supplies the candidates (synth.room_relocalization shows
@@ -318,6 +324,19 @@ class ICP(object):
         Returns (best (K,) int32, pose (K,3), score (K,H), iterations (K,H) int32), plus T (K,H,3,3) with
         return_T=True; for one (N,) scan the K axis is dropped.  Errors are those of map_observation: a NaN candidate
         raises ValueError like the reference's int(), before any device work.
+
+        keep=M (an int >= 1) searches coarse to fine instead, which is faster on large candidate sets and may give a
+        different answer: every hypothesis first runs coarse_iters ICP iterations (default RELOCALIZE_COARSE_ITERS;
+        1 <= coarse_iters <= max_iter), giving the score, T and iterations relocalize(max_iter=coarse_iters) gives.
+        Per scan the M' = min(M, H) best survive: the hypotheses whose coarse score and T are finite ordered by
+        (score, h), then every other hypothesis by h.  Each survivor then runs the whole map observation again from its
+        candidate, so its score, T and iterations are those of the exhaustive call (keep=None) at the same (k, h), and
+        best[k] is the selection rule applied to the survivors, reported as the original h.  The exhaustive winner is
+        chosen whenever it survives; otherwise the staged winner scores no better.  keep >= H gives the exhaustive
+        best and pose.  Returns (best (K,), pose (K,3), score (K,M'), iterations (K,M'), kept (K,M') int32), plus T
+        (K,M',3,3) with return_T=True, the survivors in kept order (ascending h).  keep < 1, coarse_iters outside
+        [1, max_iter], K * M' > 2^31 - 1 and coarse_iters without keep raise ValueError.  keep has no default: it
+        chooses an approximate search over the exact one (RELOCALIZE_KEEP_RECOMMENDED is the measured suggestion).
         """
         ranges = np.asarray(ranges, dtype=np.float32)
         one = ranges.ndim == 1
@@ -334,18 +353,34 @@ class ICP(object):
                 raise ValueError("a one-beam scan needs an explicit angle_increment")
             angle_increment = (float(angle_max) - float(angle_min)) / (N - 1)
         cs = self._beam_table(angle_min, angle_max, N)
+        max_iter = self.max_iter if max_iter is None else int(max_iter)
+        tolerance = self.tolerance if tolerance is None else float(tolerance)
+        args = (self._h, _lib.ptr(ranges), _lib.ptr(candidates), _lib.ptr(cs), float(clamp_inf_to or 0.0), K, H, N,
+                float(angle_min), float(angle_increment), float(far_range), max_iter, tolerance)
+        if keep is None and coarse_iters is not None:
+            raise ValueError("coarse_iters applies to the coarse-to-fine search: pass keep as well")
+        if keep is not None:
+            keep = max(0, min(operator.index(keep), 0x7fffffff))  # (the library rejects keep < 1)
+        M = H if keep is None else min(keep, H)
+        if keep is not None and K * M > 0x7fffffff:  # (checked here too, before the result arrays are allocated)
+            raise ValueError("scans * min(keep, H) = %d exceeds 2^31 - 1" % (K * M))
         best = np.empty(K, dtype=np.int32)
         pose = np.empty((K, 3))
-        score = np.empty((K, H))
-        iters = np.empty((K, H), dtype=np.int32)
-        T = np.empty((K, H, 3, 3)) if return_T else None
-        _lib.check(self._L.b2s_icp_relocalize(
-            self._h, _lib.ptr(ranges), _lib.ptr(candidates), _lib.ptr(cs), float(clamp_inf_to or 0.0), K, H, N,
-            float(angle_min), float(angle_increment), float(far_range),
-            self.max_iter if max_iter is None else int(max_iter),
-            self.tolerance if tolerance is None else float(tolerance),
-            _lib.ptr(best), _lib.ptr(pose), _lib.ptr(score), _lib.ptr(iters), _lib.ptr(T)))
-        out = (best, pose, score, iters) + ((T,) if return_T else ())
+        score = np.empty((K, M))
+        iters = np.empty((K, M), dtype=np.int32)
+        T = np.empty((K, M, 3, 3)) if return_T else None
+        if keep is None:
+            _lib.check(self._L.b2s_icp_relocalize(*args, _lib.ptr(best), _lib.ptr(pose), _lib.ptr(score),
+                                                  _lib.ptr(iters), _lib.ptr(T)))
+            out = (best, pose, score, iters)
+        else:
+            coarse = RELOCALIZE_COARSE_ITERS if coarse_iters is None else max(0, min(operator.index(coarse_iters), 0x7fffffff))
+            kept = np.empty((K, M), dtype=np.int32)
+            _lib.check(self._L.b2s_icp_relocalize_keep(*args, keep, coarse, _lib.ptr(best),
+                                                       _lib.ptr(pose), _lib.ptr(kept), _lib.ptr(score), _lib.ptr(iters),
+                                                       _lib.ptr(T)))
+            out = (best, pose, score, iters, kept)
+        out += (T,) if return_T else ()
         return tuple(a[0] for a in out) if one else out
 
     def process_scans(self, ranges, angle_min, angle_max, clamp_inf_to=None, state=None, max_iter=None,

@@ -215,6 +215,19 @@ int b2s_virtual_scan_batch(const double *obs_x, const double *obs_y, int count, 
  * in the map frame.  A scan without a finite hypothesis gets -1 and a NaN pose. */
 int b2s_relocalize_select(const double *score, const double *T, const double *candidates3, int scans, int hyps,
                           int32_t *best_out, double *pose_out, void *stream);
+/* The keep step of a coarse-to-fine relocalization.  score [scans][hyps] and T [scans][hyps][9] as for
+ * b2s_relocalize_select (the coarse solves); keys: device scratch of scans * hyps 64-bit words.  With M = min(keep,
+ * hyps), kept_out [scans][M] receives, in ascending h, the first M hypotheses of scan k in this order: those whose score
+ * and all nine entries of T are finite, by (score, h) with scores compared as doubles (-0 == +0), then every other
+ * hypothesis by h.  keep >= 1. */
+int b2s_relocalize_keep(const double *score, const double *T, int scans, int hyps, int keep, uint64_t *keys,
+                        int32_t *kept_out, void *stream);
+/* b2s_relocalize_select over the survivors of b2s_relocalize_keep: score [scans][keep] and T [scans][keep][9] are
+ * the solves of candidates3[kept[k][j]] (kept [scans][keep], ascending in each row, every entry a row of
+ * candidates3).  The rule is b2s_relocalize_select's, and best_out[k] is the original candidate index kept[k][j] of
+ * the winner (-1 and a NaN pose when no survivor is finite). */
+int b2s_relocalize_select_kept(const double *score, const double *T, const double *candidates3, const int32_t *kept,
+                               int scans, int keep, int32_t *best_out, double *pose_out, void *stream);
 
 /* Sum of per-GPU count deltas (no reference counterpart: the reference is single-process).
  * In-place ncclAllReduce(int32, sum) of both planes on an existing communicator. */
@@ -356,6 +369,18 @@ int b2s_icp_relocalize(b2s_icp *icp, const float *ranges, const double *candidat
                        double clamp_inf_to, int scans, int hyps, int n, double angle_min, double angle_increment,
                        double far_range, int max_iter, double tol, int32_t *best_out, double *pose_out,
                        double *score_out, int32_t *iters_out, double *T_out);
+/* Coarse-to-fine relocalization: b2s_icp_relocalize with every hypothesis first run for coarse_iters iterations (its
+ * score, T and iterations are those of b2s_icp_relocalize with max_iter = coarse_iters), the M = min(keep, hyps)
+ * best per scan kept by b2s_relocalize_keep's order (kept_out [scans][M], ascending), and only those refined: each
+ * survivor runs the map observation again from its candidate with max_iter and tol, so its score_out, iters_out and
+ * T_out ([scans][M], [scans][M], [scans][M][9], in kept order) are b2s_icp_relocalize's entries at (k, kept[k][j]),
+ * bit for bit.  best_out [scans] (an original candidate index) and pose_out [scans][3] follow b2s_relocalize_select
+ * among the survivors.  keep >= 1, 1 <= coarse_iters <= max_iter, scans * M <= 2^31 - 1; kept_out, score_out,
+ * iters_out and T_out may be NULL.  Errors otherwise as b2s_icp_relocalize. */
+int b2s_icp_relocalize_keep(b2s_icp *icp, const float *ranges, const double *candidates3, const double *beam_cs,
+                            double clamp_inf_to, int scans, int hyps, int n, double angle_min, double angle_increment,
+                            double far_range, int max_iter, double tol, int keep, int coarse_iters, int32_t *best_out,
+                            double *pose_out, int32_t *kept_out, double *score_out, int32_t *iters_out, double *T_out);
 int b2s_icp_find_nearest(b2s_icp *icp, const double *src_xy, int n, const double *tar_xy, int m,
                          double *dist_out, int64_t *idx_out);
 int b2s_icp_get_transform(b2s_icp *icp, const double *src_xy, const double *tar_xy, int n,
