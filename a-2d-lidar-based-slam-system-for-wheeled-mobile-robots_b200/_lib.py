@@ -33,6 +33,7 @@ SIGNATURES = {
     "b2s_icp_batch_f32": (_i32, [_vp, _vp, _i32, _i32, _i32, _i32, _dbl, _vp, _vp, _vp]),
     "b2s_icp_batch_f64": (_i32, [_vp, _vp, _i32, _i32, _i32, _i32, _dbl, _vp, _vp, _vp]),
     "b2s_icp_batch_f64_err": (_i32, [_vp, _vp, _i32, _i32, _i32, _i32, _dbl, _vp, _vp, _vp, _vp]),
+    "b2s_icp_dispatch": (_i32, [_i32, _i32, _i32, _i32, ctypes.POINTER(_i32), ctypes.POINTER(_i32), ctypes.POINTER(_i32)]),
     "b2s_icp_batch_ranges": (_i32, [_vp, _vp, _vp, _dbl, _i32, _i32, _i32, _dbl, _vp, _vp, _vp]),
     "b2s_nearest_f64": (_i32, [_vp, _i32, _vp, _i32, _vp, _vp, _vp]),
     "b2s_rigid_fit_f64": (_i32, [_vp, _vp, _i32, _vp, _vp]),

@@ -84,6 +84,88 @@ int g_icp_prune = 4;           // exact search: 4 queued (default: both pruning 
                                // 2 collective, warp-level + per-lane pruning; 3 warp-level only; 1 per-lane only; 0 plain brute force
 int g_icp_block = 0;           // targets per pruning block: 0 chooses per mode and scan size (8 up to 600 targets, 16 above); 8 / 16 / 32 force
 
+// Points per thread: work is proportional to the register slots (threads x points per thread, idle ones included).
+// Three is the measured optimum on B200 (360 and 1080 beams) and is taken unless it wastes more than 10 % over the
+// leanest choice; then 4, then 2.
+static int icp_points_per_thread(int n_src)
+{
+    if (g_icp_src_per_thread) return g_icp_src_per_thread;
+    // a CTA must fit the register file: 65536 / 80 registers (R <= 3) is 819 threads, 65536 / 104 (R = 4) is 630
+    // (the kernel's __maxnreg__); with a margin for the allocation granularity that is 768 / 576 threads, which is
+    // what bounds the scan size to ICP_MAX_POINTS = 3 x 768 (the launch re-checks against the kernel's attributes)
+    int slots[5] = {0, 0, 0, 0, 0}, least = 1 << 30;
+    for (int c = 2; c <= 4; ++c) {
+        int threads = ((((n_src + c - 1) / c) + 31) / 32) * 32;
+        if (threads < 64) threads = 64;
+        slots[c] = threads <= (c <= 3 ? 768 : 576) ? threads * c : (1 << 30);
+        if (slots[c] < least) least = slots[c];
+    }
+    const int order[3] = {3, 4, 2};
+    for (int k = 0; k < 3; ++k)
+        if (slots[order[k]] < (1 << 30) && (long long)slots[order[k]] * 10 <= (long long)least * 11) return order[k];
+    return 3;
+}
+
+int icp_dispatch(int n_src, int n_tar, int in_bytes, bool ranges, IcpInstance *out)
+{
+    B2S_REQUIRE(out, "b2s_icp_dispatch: null pointer");
+    B2S_REQUIRE(n_src > 0 && n_tar > 0 && (in_bytes == 4 || in_bytes == 8) &&
+                    (!ranges || (n_src == n_tar && in_bytes == 4)),
+                ranges ? "b2s_icp_batch_ranges: bad sizes" : "b2s_icp_batch: bad sizes");
+    B2S_REQUIRE(n_src <= ICP_MAX_POINTS, ranges ? "b2s_icp_batch_ranges: more than 2304 beams per scan is not supported"
+                                                : "b2s_icp_batch: more than 2304 source points per scan is not supported");
+    const int R = icp_points_per_thread(n_src);
+    const int forced = (g_icp_block == 8 || g_icp_block == 16 || g_icp_block == 32) ? g_icp_block : 0;
+    // queued search (icp_prune 4): block numbers travel in one byte, so at most QBLOCKS blocks, else the collective
+    // search takes over; above QSUP_MIN blocks the warp test gets its second level (PRUNE 5)
+    const int q8 = (n_tar + 7) / 8, q16 = (n_tar + 15) / 16;
+    int P, B;
+    if (ranges) {
+        // the fused-ingestion form has the two default searches: queued, and the collective one of icp_prune 0..3
+        const int blk = forced ? forced : (g_icp_prune == 4 || n_tar <= 600 ? 8 : 16);
+        if (g_icp_prune == 4 && blk == 8 && q8 <= QBLOCKS) {
+            P = q8 > QSUP_MIN ? 5 : 4;
+            B = 8;
+        } else if (g_icp_prune == 4 && q16 <= QBLOCKS) {
+            P = q16 > QSUP_MIN ? 5 : 4;
+            B = 16;
+        } else {
+            P = 2;
+            B = blk;
+        }
+    } else {
+        const int blk = forced ? forced
+                               : (g_icp_prune == 4 ? 8 : g_icp_prune >= 2 ? (n_tar <= 600 ? 8 : 16) : (n_tar <= 600 ? 16 : 32));  // measured best per mode
+        // the block bounds live in the staging area: [ceil(m/blk)] float4 must fit in 2*m*in_bytes
+        const bool fits = (size_t)((n_tar + blk - 1) / blk) * 16 <= (size_t)2 * n_tar * in_bytes;
+        if (!g_icp_prune || !fits) {
+            P = 0;
+            B = 16;
+        } else if (g_icp_prune == 4 && blk == 8 && q8 <= QBLOCKS) {
+            P = q8 > QSUP_MIN ? 5 : 4;
+            B = 8;
+        } else if (g_icp_prune == 4 && q16 <= QBLOCKS) {
+            P = q16 > QSUP_MIN ? 5 : 4;
+            B = 16;
+        } else if (g_icp_prune >= 2) {  // 2 and 3, and 4 beyond the queue's block count
+            P = g_icp_prune == 3 ? 3 : 2;
+            B = blk;
+        } else {
+            P = 1;
+            B = blk == 32 ? 32 : 16;
+        }
+    }
+    int threads = ((((n_src + R - 1) / R) + 31) / 32) * 32;
+    if (threads < 64) threads = 64;
+    B2S_REQUIRE(threads <= 1024, ranges ? "b2s_icp_batch_ranges: too many beams per scan"
+                                        : "b2s_icp_batch: too many source points per scan");
+    const size_t smem = icp_smem_bytes(P, B, R, n_tar, (size_t)(ranges ? 1 : 2) * n_tar * in_bytes, threads);
+    B2S_REQUIRE(smem <= 227 * 1024, ranges ? "b2s_icp_batch_ranges: too many beams for shared memory"
+                                           : "b2s_icp_batch: n_tar too large for shared memory");
+    *out = IcpInstance{R, P, B, threads, smem};
+    return B2S_OK;
+}
+
 }  // namespace b2s
 
 using namespace b2s;
@@ -96,6 +178,18 @@ extern "C" int b2s_nearest_f64(const double *src_xy, int n, const double *tar_xy
     B2S_REQUIRE(src_xy && dist_out && idx_out && (tar_xy || m == 0), "b2s_nearest: null pointer");
     nearest_kernel<<<(n + 127) / 128, 128, 0, (cudaStream_t)stream>>>(src_xy, n, tar_xy, m, dist_out, idx_out);
     B2S_CUDA(cudaGetLastError());
+    return B2S_OK;
+}
+
+extern "C" int b2s_icp_dispatch(int n_src, int n_tar, int in_bytes, int ranges, int *R, int *prune, int *nn_blk)
+{
+    B2S_REQUIRE(R && prune && nn_blk, "b2s_icp_dispatch: null pointer");
+    IcpInstance ins;
+    const int rc = icp_dispatch(n_src, n_tar, in_bytes, ranges != 0, &ins);
+    if (rc != B2S_OK) return rc;
+    *R = ins.R;
+    *prune = ins.prune;
+    *nn_blk = ins.nn_blk;
     return B2S_OK;
 }
 

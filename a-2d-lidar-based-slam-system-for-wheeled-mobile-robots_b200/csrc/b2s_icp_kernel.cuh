@@ -918,19 +918,15 @@ __global__ void __maxnreg__(R <= 3 ? (NN_BLK == 8 && PRUNE != 5 ? B2S_ICP_REGS_B
     }
 }
 
-extern int g_icp_src_per_thread;
-extern int g_icp_prune;
-extern int g_icp_block;
 extern int g_icp_layout;
 
 // Dynamic shared memory of one CTA (the layout at the top of the kernel); in_bytes = bytes of the staged input rows.
-template <int PRUNE, int NN_BLK, int R>
-static size_t icp_smem_bytes(int n_tar, size_t in_bytes, int threads)
+inline size_t icp_smem_bytes(int prune, int nn_blk, int R, int n_tar, size_t in_bytes, int threads)
 {
-    const size_t nblk = ((size_t)n_tar + NN_BLK - 1) / NN_BLK;
+    const size_t nblk = ((size_t)n_tar + nn_blk - 1) / nn_blk;
     size_t bytes = 16 + icp_scratch_doubles(threads / 32) * sizeof(double) + icp_stage_bytes(in_bytes, (int)nblk);
-    if (PRUNE >= 4) {
-        bytes += nblk * (NN_BLK + 1) * sizeof(double2);                       // padded targets
+    if (prune >= 4) {
+        bytes += nblk * (nn_blk + 1) * sizeof(double2);                       // padded targets
         bytes += (size_t)R * threads * sizeof(double2);                       // moved source points
         bytes += (size_t)(threads / 32) * (size_t)(R * QK * 32) * (sizeof(unsigned) + sizeof(uint2));  // queues + results
     } else {
@@ -939,16 +935,26 @@ static size_t icp_smem_bytes(int n_tar, size_t in_bytes, int threads)
     return bytes;
 }
 
+// One launch of the batched kernel: the template instance icp_batch_kernel<TIn, R, prune, nn_blk, ...> and its CTA.
+struct IcpInstance {
+    int R, prune, nn_blk;
+    int threads;
+    size_t smem;
+};
+
+// The instance a call takes (b2s_icp.cu, the only copy of that choice; exported as b2s_icp_dispatch): from the sizes
+// and the b2s_tune state, for b2s_icp_batch_f32 / _f64 (ranges = false, in_bytes = 4 / 8 per coordinate) or
+// b2s_icp_batch_ranges (ranges = true, n_src == n_tar beams, in_bytes = 4).  Host only; B2S_ERR_INVALID_ARG where the
+// launch refuses the shape (the per-kernel thread limit, which needs the device, is checked at the launch).
+int icp_dispatch(int n_src, int n_tar, int in_bytes, bool ranges, IcpInstance *out);
+
 template <typename TIn, int R, int PRUNE, int NN_BLK>
 static int launch_icp_rp(const TIn *tar_xy, const TIn *src_xy, int pairs, int n_src, int n_tar, int max_iter,
-                        double tol, double *T_out, int32_t *iters_out, double *err_out, void *stream)
+                        double tol, double *T_out, int32_t *iters_out, double *err_out, const IcpInstance &ins,
+                        void *stream)
 {
-    int threads = (n_src + R - 1) / R;
-    threads = ((threads + 31) / 32) * 32;
-    if (threads < 64) threads = 64;
-    B2S_REQUIRE(threads <= 1024, "b2s_icp_batch: too many source points per scan");
-    const size_t smem = icp_smem_bytes<PRUNE, NN_BLK, R>(n_tar, (size_t)n_tar * 2 * sizeof(TIn), threads);
-    B2S_REQUIRE(smem <= 227 * 1024, "b2s_icp_batch: n_tar too large for shared memory");
+    const int threads = ins.threads;
+    const size_t smem = ins.smem;
     // the score output exists for float64 clouds only (the relocalization's virtual scans and laserToNumpy points)
     constexpr bool HAS_ERR = sizeof(TIn) == 8;
     auto kernel = icp_batch_kernel<TIn, R, PRUNE, NN_BLK>;
@@ -970,77 +976,42 @@ static int launch_icp_rp(const TIn *tar_xy, const TIn *src_xy, int pairs, int n_
     return B2S_OK;
 }
 
+// (every (PRUNE, NN_BLK) that icp_dispatch chooses for point clouds)
 template <typename TIn, int R>
 static int launch_icp_r(const TIn *tar_xy, const TIn *src_xy, int pairs, int n_src, int n_tar, int max_iter,
-                        double tol, double *T_out, int32_t *iters_out, double *err_out, void *stream)
+                        double tol, double *T_out, int32_t *iters_out, double *err_out, const IcpInstance &ins,
+                        void *stream)
 {
-    // the block bounds live in the staging area: [ceil(m/blk)] float4 must fit in 2*m*sizeof(TIn)
-    const int blk = (g_icp_block == 8 || g_icp_block == 16 || g_icp_block == 32) ? g_icp_block
-                    : (g_icp_prune == 4 ? 8 : g_icp_prune >= 2 ? (n_tar <= 600 ? 8 : 16) : (n_tar <= 600 ? 16 : 32));  // measured best per mode
-    const bool fits = (size_t)((n_tar + blk - 1) / blk) * 16 <= (size_t)2 * n_tar * sizeof(TIn);
-#define B2S_ICP_GO(P, B) \
-    return launch_icp_rp<TIn, R, P, B>(tar_xy, src_xy, pairs, n_src, n_tar, max_iter, tol, T_out, iters_out, err_out, stream)
-    if (g_icp_prune && fits) {
-        if (g_icp_prune == 4) {  // (block numbers travel in one byte; beyond that the collective search takes over)
-            if (blk == 8 && (n_tar + 7) / 8 <= QBLOCKS) {
-                if ((n_tar + 7) / 8 > QSUP_MIN) B2S_ICP_GO(5, 8);
-                B2S_ICP_GO(4, 8);
-            }
-            if ((n_tar + 15) / 16 <= QBLOCKS) {
-                if ((n_tar + 15) / 16 > QSUP_MIN) B2S_ICP_GO(5, 16);
-                B2S_ICP_GO(4, 16);
-            }
-        }
-        if (g_icp_prune == 3) {
-            if (blk == 8) B2S_ICP_GO(3, 8);
-            if (blk == 16) B2S_ICP_GO(3, 16);
-            B2S_ICP_GO(3, 32);
-        }
-        if (g_icp_prune == 2 || g_icp_prune == 4) {
-            if (blk == 8) B2S_ICP_GO(2, 8);
-            if (blk == 16) B2S_ICP_GO(2, 16);
-            B2S_ICP_GO(2, 32);
-        }
-        if (blk == 8) B2S_ICP_GO(1, 16);
-        if (blk == 16) B2S_ICP_GO(1, 16);
-        B2S_ICP_GO(1, 32);
-    }
+#define B2S_ICP_GO(P, B)                                                                                              \
+    if (ins.prune == P && ins.nn_blk == B)                                                                            \
+    return launch_icp_rp<TIn, R, P, B>(tar_xy, src_xy, pairs, n_src, n_tar, max_iter, tol, T_out, iters_out, err_out, \
+                                       ins, stream)
+    B2S_ICP_GO(5, 8);
+    B2S_ICP_GO(4, 8);
+    B2S_ICP_GO(5, 16);
+    B2S_ICP_GO(4, 16);
+    B2S_ICP_GO(3, 8);
+    B2S_ICP_GO(3, 16);
+    B2S_ICP_GO(3, 32);
+    B2S_ICP_GO(2, 8);
+    B2S_ICP_GO(2, 16);
+    B2S_ICP_GO(2, 32);
+    B2S_ICP_GO(1, 16);
+    B2S_ICP_GO(1, 32);
     B2S_ICP_GO(0, 16);
 #undef B2S_ICP_GO
+    set_error("b2s_icp_batch: no kernel instance for PRUNE %d, NN_BLK %d", ins.prune, ins.nn_blk);
+    return B2S_ERR_INVALID_ARG;
 }
 
-// Points per thread: work is proportional to the register slots (threads x points per thread, idle ones included).
-// Three is the measured optimum on B200 (360 and 1080 beams) and is taken unless it wastes more than 10 % over the
-// leanest choice; then 4, then 2.
-static int icp_points_per_thread(int n_src)
-{
-    if (g_icp_src_per_thread) return g_icp_src_per_thread;
-    // a CTA must fit the register file: 65536 / 80 registers (R <= 3) is 819 threads, 65536 / 104 (R = 4) is 630
-    // (the kernel's __maxnreg__); with a margin for the allocation granularity that is 768 / 576 threads, which is
-    // what bounds the scan size to ICP_MAX_POINTS = 3 x 768 (the launch re-checks against the kernel's attributes)
-    int slots[5] = {0, 0, 0, 0, 0}, least = 1 << 30;
-    for (int c = 2; c <= 4; ++c) {
-        int threads = ((((n_src + c - 1) / c) + 31) / 32) * 32;
-        if (threads < 64) threads = 64;
-        slots[c] = threads <= (c <= 3 ? 768 : 576) ? threads * c : (1 << 30);
-        if (slots[c] < least) least = slots[c];
-    }
-    const int order[3] = {3, 4, 2};
-    for (int k = 0; k < 3; ++k)
-        if (slots[order[k]] < (1 << 30) && (long long)slots[order[k]] * 10 <= (long long)least * 11) return order[k];
-    return 3;
-}
-
-// Fused-ingestion form: raw ranges + beam table (always the default search, PRUNE = 2).
+// Fused-ingestion form: raw ranges + beam table.
 template <int R, int NN_BLK, int PRUNE>
 static int launch_icp_ranges_rbp(const float *tar_r, const float *src_r, const double *beam_cs, double clamp, int pairs,
-                                int n, int max_iter, double tol, double *T_out, int32_t *iters_out, void *stream)
+                                int n, int max_iter, double tol, double *T_out, int32_t *iters_out,
+                                const IcpInstance &ins, void *stream)
 {
-    int threads = ((((n + R - 1) / R) + 31) / 32) * 32;
-    if (threads < 64) threads = 64;
-    B2S_REQUIRE(threads <= 1024, "b2s_icp_batch_ranges: too many beams per scan");
-    const size_t smem = icp_smem_bytes<PRUNE, NN_BLK, R>(n, (size_t)n * sizeof(float), threads);
-    B2S_REQUIRE(smem <= 227 * 1024, "b2s_icp_batch_ranges: too many beams for shared memory");
+    const int threads = ins.threads;
+    const size_t smem = ins.smem;
     if (smem > 48 * 1024)
         B2S_CUDA(cudaFuncSetAttribute(icp_batch_kernel<float, R, PRUNE, NN_BLK, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                       (int)smem));
@@ -1056,28 +1027,26 @@ static int launch_icp_ranges_rbp(const float *tar_r, const float *src_r, const d
     return B2S_OK;
 }
 
+// (every (NN_BLK, PRUNE) that icp_dispatch chooses for raw ranges)
 template <int R>
 static int launch_icp_ranges_r(const float *tar_r, const float *src_r, const double *beam_cs, double clamp, int pairs,
-                               int n, int max_iter, double tol, double *T_out, int32_t *iters_out, void *stream)
+                               int n, int max_iter, double tol, double *T_out, int32_t *iters_out,
+                               const IcpInstance &ins, void *stream)
 {
-    // (the fused-ingestion form has the two default searches: queued, and the collective one of icp_prune 0..3)
-    const int blk = (g_icp_block == 8 || g_icp_block == 16 || g_icp_block == 32) ? g_icp_block : (g_icp_prune == 4 || n <= 600 ? 8 : 16);
-#define B2S_ICP_GO(B, P) \
-    return launch_icp_ranges_rbp<R, B, P>(tar_r, src_r, beam_cs, clamp, pairs, n, max_iter, tol, T_out, iters_out, stream)
-    if (g_icp_prune == 4) {
-        if (blk == 8 && (n + 7) / 8 <= QBLOCKS) {
-            if ((n + 7) / 8 > QSUP_MIN) B2S_ICP_GO(8, 5);
-            B2S_ICP_GO(8, 4);
-        }
-        if ((n + 15) / 16 <= QBLOCKS) {
-            if ((n + 15) / 16 > QSUP_MIN) B2S_ICP_GO(16, 5);
-            B2S_ICP_GO(16, 4);
-        }
-    }
-    if (blk == 8) B2S_ICP_GO(8, 2);
-    if (blk == 16) B2S_ICP_GO(16, 2);
+#define B2S_ICP_GO(B, P)                                                                                             \
+    if (ins.prune == P && ins.nn_blk == B)                                                                           \
+    return launch_icp_ranges_rbp<R, B, P>(tar_r, src_r, beam_cs, clamp, pairs, n, max_iter, tol, T_out, iters_out, \
+                                          ins, stream)
+    B2S_ICP_GO(8, 5);
+    B2S_ICP_GO(8, 4);
+    B2S_ICP_GO(16, 5);
+    B2S_ICP_GO(16, 4);
+    B2S_ICP_GO(8, 2);
+    B2S_ICP_GO(16, 2);
     B2S_ICP_GO(32, 2);
 #undef B2S_ICP_GO
+    set_error("b2s_icp_batch_ranges: no kernel instance for PRUNE %d, NN_BLK %d", ins.prune, ins.nn_blk);
+    return B2S_ERR_INVALID_ARG;
 }
 
 static int launch_icp_ranges(const float *tar_r, const float *src_r, const double *beam_cs, double clamp, int pairs, int n,
@@ -1088,11 +1057,13 @@ static int launch_icp_ranges(const float *tar_r, const float *src_r, const doubl
     B2S_REQUIRE(tar_r && src_r && beam_cs && T_out, "b2s_icp_batch_ranges: null pointer");
     B2S_REQUIRE((uintptr_t)beam_cs % 16 == 0, "b2s_icp_batch_ranges: the beam table must be 16-byte aligned");
     B2S_REQUIRE(tol == tol && clamp == clamp, "b2s_icp_batch_ranges: NaN tolerance / clamp");
-    B2S_REQUIRE(n <= ICP_MAX_POINTS, "b2s_icp_batch_ranges: more than 2304 beams per scan is not supported");
-    switch (icp_points_per_thread(n)) {
-    case 2: return launch_icp_ranges_r<2>(tar_r, src_r, beam_cs, clamp, pairs, n, max_iter, tol, T_out, iters_out, stream);
-    case 3: return launch_icp_ranges_r<3>(tar_r, src_r, beam_cs, clamp, pairs, n, max_iter, tol, T_out, iters_out, stream);
-    default: return launch_icp_ranges_r<4>(tar_r, src_r, beam_cs, clamp, pairs, n, max_iter, tol, T_out, iters_out, stream);
+    IcpInstance ins;
+    const int rc = icp_dispatch(n, n, (int)sizeof(float), true, &ins);
+    if (rc != B2S_OK) return rc;
+    switch (ins.R) {
+    case 2: return launch_icp_ranges_r<2>(tar_r, src_r, beam_cs, clamp, pairs, n, max_iter, tol, T_out, iters_out, ins, stream);
+    case 3: return launch_icp_ranges_r<3>(tar_r, src_r, beam_cs, clamp, pairs, n, max_iter, tol, T_out, iters_out, ins, stream);
+    default: return launch_icp_ranges_r<4>(tar_r, src_r, beam_cs, clamp, pairs, n, max_iter, tol, T_out, iters_out, ins, stream);
     }
 }
 
@@ -1105,12 +1076,13 @@ static int launch_icp(const TIn *tar_xy, const TIn *src_xy, int pairs, int n_src
     if (pairs == 0) return B2S_OK;
     B2S_REQUIRE(tar_xy && src_xy && T_out, "b2s_icp_batch: null pointer");
     B2S_REQUIRE(tol == tol, "b2s_icp_batch: NaN tolerance");
-    B2S_REQUIRE(n_src <= ICP_MAX_POINTS, "b2s_icp_batch: more than 2304 source points per scan is not supported");
-    const int r = icp_points_per_thread(n_src);
-    switch (r) {
-    case 2: return launch_icp_r<TIn, 2>(tar_xy, src_xy, pairs, n_src, n_tar, max_iter, tol, T_out, iters_out, err_out, stream);
-    case 3: return launch_icp_r<TIn, 3>(tar_xy, src_xy, pairs, n_src, n_tar, max_iter, tol, T_out, iters_out, err_out, stream);
-    default: return launch_icp_r<TIn, 4>(tar_xy, src_xy, pairs, n_src, n_tar, max_iter, tol, T_out, iters_out, err_out, stream);
+    IcpInstance ins;
+    const int rc = icp_dispatch(n_src, n_tar, (int)sizeof(TIn), false, &ins);
+    if (rc != B2S_OK) return rc;
+    switch (ins.R) {
+    case 2: return launch_icp_r<TIn, 2>(tar_xy, src_xy, pairs, n_src, n_tar, max_iter, tol, T_out, iters_out, err_out, ins, stream);
+    case 3: return launch_icp_r<TIn, 3>(tar_xy, src_xy, pairs, n_src, n_tar, max_iter, tol, T_out, iters_out, err_out, ins, stream);
+    default: return launch_icp_r<TIn, 4>(tar_xy, src_xy, pairs, n_src, n_tar, max_iter, tol, T_out, iters_out, err_out, ins, stream);
     }
 }
 

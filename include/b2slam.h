@@ -94,6 +94,13 @@ int b2s_icp_batch_f64(const double *tar_xy, const double *src_xy, int pairs, int
  * T_out and iters_out are those of b2s_icp_batch_f64, bit for bit.  max_iter == 0 gives 0. */
 int b2s_icp_batch_f64_err(const double *tar_xy, const double *src_xy, int pairs, int n_src, int n_tar,
                           int max_iter, double tol, double *T_out, int32_t *iters_out, double *err_out, void *stream);
+/* The kernel instance a batched ICP call of these sizes launches under the current b2s_tune settings: *R source points
+ * per thread, the search *prune (0 brute force, 1 per-lane, 2 collective, 3 warp-level only, 4 queued, 5 queued with
+ * the second-level warp test) and *nn_blk targets per pruning block.  ranges = 0: b2s_icp_batch_f32 (in_bytes 4) /
+ * _f64 and _f64_err (in_bytes 8); ranges != 0: b2s_icp_batch_ranges (n_src == n_tar beams, in_bytes 4).  Returns
+ * B2S_ERR_INVALID_ARG for sizes those calls refuse before launching (more than 2304 source points, more than 1024
+ * threads, more than 227 KB of shared memory).  Launches nothing and needs no device. */
+int b2s_icp_dispatch(int n_src, int n_tar, int in_bytes, int ranges, int *R, int *prune, int *nn_blk);
 
 /* ICP.findNearest -- replaces [ICP]:90-114.  src_xy [n][2], tar_xy [m][2] (row = point, as the
  * reference passes them); dist_out [n] float64, idx_out [n] int64.  Lowest index wins ties. */

@@ -30,6 +30,8 @@ def lib():
         L.orc_rigid_fit.restype = None
         L.orc_icp_batch.argtypes = [vp, vp, i32, i32, i32, i32, dbl, vp, vp]
         L.orc_icp_batch.restype = i32
+        L.orc_icp_batch_err.argtypes = [vp, vp, i32, i32, i32, i32, dbl, vp, vp, vp]
+        L.orc_icp_batch_err.restype = i32
         L.orc_bresenham.argtypes = [i64, i64, i64, i64, vp, i64]
         L.orc_bresenham.restype = i64
         L.orc_grid_raycast.argtypes = [vp, vp, i32, i32, dbl, dbl, dbl, vp, vp, vp, vp, i32, i32]
@@ -65,18 +67,23 @@ def rigid_fit(src, tar):
     return T.reshape(3, 3)
 
 
-def icp_batch(tar, src, max_iter=30, tol=1e-3):
-    """tar (P,2,M), src (P,2,N) (x/y rows, any float dtype) -> (T (P,3,3), iters (P,))."""
+def icp_batch(tar, src, max_iter=30, tol=1e-3, return_err=False):
+    """tar (P,2,M), src (P,2,N) (x/y rows, any float dtype) -> (T (P,3,3), iters (P,)), and with return_err=True
+    err (P,) as well: each pair's mean_error of its last iteration ([ICP]:75), 0 when none ran."""
     tar = np.ascontiguousarray(np.transpose(np.asarray(tar, dtype=np.float64), (0, 2, 1)))
     src = np.ascontiguousarray(np.transpose(np.asarray(src, dtype=np.float64), (0, 2, 1)))
     P, N, M = src.shape[0], src.shape[1], tar.shape[1]
     T = np.empty((P, 9))
     iters = np.empty(P, dtype=np.int32)
-    rc = lib().orc_icp_batch(_p(tar), _p(src), P, N, M, int(max_iter), float(tol), _p(T),
-                             _p(iters))
+    if return_err:
+        err = np.empty(P)
+        rc = lib().orc_icp_batch_err(_p(tar), _p(src), P, N, M, int(max_iter), float(tol), _p(T), _p(iters), _p(err))
+    else:
+        rc = lib().orc_icp_batch(_p(tar), _p(src), P, N, M, int(max_iter), float(tol), _p(T),
+                                 _p(iters))
     if rc != 0:
         raise ValueError("orc_icp_batch: bad arguments")
-    return T.reshape(P, 3, 3), iters
+    return (T.reshape(P, 3, 3), iters, err) if return_err else (T.reshape(P, 3, 3), iters)
 
 
 def bresenham(start, end):

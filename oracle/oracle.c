@@ -108,11 +108,12 @@ void orc_rigid_fit(const double *src_xy, const double *tar_xy, const int32_t *pi
 }
 
 /* [ICP]:38-88  one scan pair.  src_xy [n][2], tar_xy [m][2]; scratch sized by caller. */
+/* *err_out: mean_error of the last iteration that ran ([ICP]:75), 0 when none did. */
 static int icp_one(const double *tar_xy, int m, const double *src_xy, int n, int max_iter,
-                   double tol, double *T_out, double *cur, double *dist, int32_t *idx)
+                   double tol, double *T_out, double *err_out, double *cur, double *dist, int32_t *idx)
 {
     memcpy(cur, src_xy, sizeof(double) * 2 * (size_t)n);
-    double prev = 0.0;
+    double prev = 0.0, err = 0.0;
     int iters = 0;
     double T[9];
     for (int it = 0; it < max_iter; ++it) {
@@ -126,17 +127,19 @@ static int icp_one(const double *tar_xy, int m, const double *src_xy, int n, int
         ++iters;
         double total = 0.0;
         for (int i = 0; i < n; ++i) total += dist[i];
-        const double err = total / (double)n; /* [ICP]:75 distances from BEFORE the move */
+        err = total / (double)n;               /* [ICP]:75 distances from BEFORE the move */
         if (fabs(prev - err) < tol) break;     /* [ICP]:76 strict '<' */
         prev = err;
     }
     orc_rigid_fit(src_xy, cur, NULL, n, T_out); /* [ICP]:81 final re-fit */
+    *err_out = err;
     return iters;
 }
 
-/* Batch of independent pairs.  tar [P][m][2], src [P][n][2] float64; T_out [P][9]. */
-int orc_icp_batch(const double *tar_xy, const double *src_xy, int pairs, int n, int m,
-                  int max_iter, double tol, double *T_out, int32_t *iters_out)
+/* Batch of independent pairs.  tar [P][m][2], src [P][n][2] float64; T_out [P][9]; err_out [P] (may be NULL) the
+ * mean_error of each pair's last iteration, summed left to right. */
+int orc_icp_batch_err(const double *tar_xy, const double *src_xy, int pairs, int n, int m,
+                      int max_iter, double tol, double *T_out, int32_t *iters_out, double *err_out)
 {
     if (pairs < 0 || n <= 0 || m <= 0 || max_iter < 0) return -1;
     {
@@ -144,14 +147,22 @@ int orc_icp_batch(const double *tar_xy, const double *src_xy, int pairs, int n, 
         double *dist = (double *)malloc(sizeof(double) * (size_t)n);
         int32_t *idx = (int32_t *)malloc(sizeof(int32_t) * (size_t)n);
         for (int p = 0; p < pairs; ++p) {
+            double err;
             iters_out[p] = icp_one(tar_xy + (size_t)p * m * 2, m, src_xy + (size_t)p * n * 2, n,
-                                   max_iter, tol, T_out + (size_t)p * 9, cur, dist, idx);
+                                   max_iter, tol, T_out + (size_t)p * 9, &err, cur, dist, idx);
+            if (err_out) err_out[p] = err;
         }
         free(cur);
         free(dist);
         free(idx);
     }
     return 0;
+}
+
+int orc_icp_batch(const double *tar_xy, const double *src_xy, int pairs, int n, int m,
+                  int max_iter, double tol, double *T_out, int32_t *iters_out)
+{
+    return orc_icp_batch_err(tar_xy, src_xy, pairs, n, m, max_iter, tol, T_out, iters_out, NULL);
 }
 
 /* ------------------------------------------------------------------ Bresenham / grid */
