@@ -62,6 +62,8 @@ SIGNATURES = {
     "b2s_relocalize_select": (_i32, [_vp, _vp, _vp, _i32, _i32, _vp, _vp, _vp]),
     "b2s_relocalize_keep": (_i32, [_vp, _vp, _i32, _i32, _i32, _vp, _vp, _vp]),
     "b2s_relocalize_select_kept": (_i32, [_vp, _vp, _vp, _vp, _i32, _i32, _vp, _vp, _vp]),
+    "b2s_track_step": (_i32, [_vp, _vp, _vp, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "b2s_track_select": (_i32, [_vp, _vp, _i32, _vp, _vp]),
     "b2s_grid_allreduce": (_i32, [_vp, _vp, _sz, _vp, _vp]),
     "b2s_grid_merge_p2p": (_i32, [_vp, _vp, _vp, _i32, _sz, _sz, _vp, _vp, _dbl, _dbl, _dbl, _vp]),
     "b2s_grid_merge_p2p_tiles": (_i32, [_vp, _vp, _vp, _vp, _i32, _i32, _i32, _i32, _i32, _vp, _vp, _dbl, _dbl,
@@ -102,6 +104,8 @@ SIGNATURES = {
                                   _vp, _vp, _vp]),
     "b2s_icp_relocalize_keep": (_i32, [_vp, _vp, _vp, _vp, _dbl, _i32, _i32, _i32, _dbl, _dbl, _dbl, _i32, _dbl, _i32,
                                        _i32, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "b2s_icp_track": (_i32, [_vp, _vp, _vp, _vp, _dbl, _i32, _i32, _i32, _dbl, _dbl, _dbl, _i32, _dbl, _vp, _vp, _vp,
+                             _vp, _vp, _vp]),
     "b2s_icp_find_nearest": (_i32, [_vp, _vp, _i32, _vp, _i32, _vp, _vp]),
     "b2s_icp_get_transform": (_i32, [_vp, _vp, _vp, _i32, _vp]),
     "b2s_mapping_create": (_i32, [_pp, _i32, _i32, _dbl, _dbl, _dbl, _dbl, _i32]),

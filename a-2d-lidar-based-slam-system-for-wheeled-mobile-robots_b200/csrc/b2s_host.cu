@@ -1102,6 +1102,88 @@ extern "C" int b2s_icp_relocalize_keep(b2s_icp *c, const float *ranges, const do
     return icp_read_back(c, tr, scans * M, T_out, iters_out);
 }
 
+// Pose tracking: H hypotheses through K scans.  The odometry of the K scans (the ranges-form ICP of
+// b2s_icp_process_scans, on the same uploads) runs on stream2 under stage 0, which does not need it; the K source
+// clouds are formed once.  Then, per stage on stream: the virtual scans at the H priors, scan k's cloud replicated into
+// the H source rows, the H-pair ICP with its score, and b2s_track_step, which writes the next stage's priors where its
+// virtual scans read them.  Stage k + 1 needs stage k's poses, so the stages run one after the other.
+extern "C" int b2s_icp_track(b2s_icp *c, const float *ranges, const double *starts3, const double *beam_cs,
+                             double clamp_inf_to, int scans, int hyps, int n, double angle_min, double angle_increment,
+                             double far_range, int max_iter, double tol, int32_t *best_out, double *pose_out,
+                             double *score_out, int32_t *iters_out, double *joint_out, double *prior_out)
+{
+    const char *fn = "b2s_icp_track";
+    if (scans < 1) return invalid(fn, "bad sizes");
+    int rc = relocalize_check(fn, c, ranges, starts3, beam_cs, clamp_inf_to, scans, hyps, n, angle_increment, max_iter,
+                              tol, best_out, pose_out);
+    if (rc) return rc;
+    DeviceGuard g(c->device);
+    Trace tr(c->stream);
+    const size_t H = (size_t)hyps, K = (size_t)scans, row = (size_t)2 * n;
+    auto a16 = [](size_t b) { return (b + 15) & ~(size_t)15; };
+    // d_map_in: beam table | ranges [K][n]; d_map_src: the H source rows | the K source clouds
+    // d_aux: scores [K][H] | priors [K][H][3] | poses [K][H][3] | joint [H] | odometry T [K-1][9] | finite [H] |
+    //        odometry iterations [K-1] | best
+    const size_t cs_bytes = (size_t)n * 2 * sizeof(double);
+    const size_t prior_off = K * H * sizeof(double), pose_off = prior_off + K * H * 3 * sizeof(double);
+    const size_t joint_off = pose_off + K * H * 3 * sizeof(double), odo_off = joint_off + H * sizeof(double);
+    const size_t fin_off = odo_off + (K - 1) * 9 * sizeof(double), oit_off = a16(fin_off + H * sizeof(int32_t));
+    const size_t best_off = a16(oit_off + (K - 1) * sizeof(int32_t));
+    if ((rc = c->d_map_in.reserve(cs_bytes + K * n * sizeof(float)))) return rc;
+    if ((rc = c->d_map_tar.reserve(H * row * sizeof(double)))) return rc;
+    if ((rc = c->d_map_src.reserve((H + K) * row * sizeof(double)))) return rc;
+    if ((rc = c->d_T.reserve(H * 9 * sizeof(double)))) return rc;
+    if ((rc = c->d_iters.reserve(K * H * sizeof(int32_t)))) return rc;
+    if ((rc = c->d_aux.reserve(best_off + sizeof(int32_t)))) return rc;
+    char *in = (char *)c->d_map_in.p, *aux = (char *)c->d_aux.p;
+    const double *d_cs = (const double *)in;
+    const float *d_ranges = (const float *)(in + cs_bytes);
+    double *d_tar = (double *)c->d_map_tar.p, *d_src = (double *)c->d_map_src.p, *d_clouds = d_src + H * row;
+    double *d_score = (double *)aux, *d_prior = (double *)(aux + prior_off), *d_pose = (double *)(aux + pose_off);
+    double *d_joint = (double *)(aux + joint_off), *d_odo = (double *)(aux + odo_off), *d_T = (double *)c->d_T.p;
+    int32_t *d_fin = (int32_t *)(aux + fin_off), *d_oit = (int32_t *)(aux + oit_off), *d_best = (int32_t *)(aux + best_off);
+    int32_t *d_iters = (int32_t *)c->d_iters.p;
+    const double *map_x = (const double *)c->d_map.p, *map_y = map_x + c->map_count;
+    // (every call ends with a synchronize, so the device buffers are free to overwrite here)
+    B2S_CUDA(cudaMemcpyAsync(in, beam_cs, cs_bytes, cudaMemcpyHostToDevice, c->stream));
+    B2S_CUDA(cudaMemcpyAsync(in + cs_bytes, ranges, K * n * sizeof(float), cudaMemcpyHostToDevice, c->stream));
+    B2S_CUDA(cudaMemcpyAsync(d_prior, starts3, H * 3 * sizeof(double), cudaMemcpyHostToDevice, c->stream));
+    if (K > 1) {
+        B2S_CUDA(cudaEventRecord(c->chunk_ready[0], c->stream));
+        B2S_CUDA(cudaStreamWaitEvent(c->stream2, c->chunk_ready[0], 0));
+        if ((rc = b2s_icp_batch_ranges(d_ranges, d_ranges + n, d_cs, clamp_inf_to, scans - 1, n, max_iter, tol, d_odo, d_oit,
+                                       c->stream2)))
+            return rc;
+        tr.mark("odometry done", 0, c->stream2);
+        B2S_CUDA(cudaEventRecord(c->joined, c->stream2));
+    }
+    if ((rc = laser_points(d_ranges, d_cs, clamp_inf_to, scans, n, d_clouds, c->stream))) return rc;
+    for (size_t k = 0; k < K; ++k) {
+        double *prior = d_prior + k * H * 3, *next = k + 1 < K ? prior + H * 3 : nullptr;
+        if ((rc = b2s_virtual_scan_batch(map_x, map_y, c->map_count, prior, hyps, angle_min, angle_increment, n, far_range,
+                                         d_cs, nullptr, d_tar, c->stream)))
+            return rc;
+        if ((rc = replicate_row(d_clouds + k * row, row, H, d_src, c->stream))) return rc;
+        if ((rc = b2s_icp_batch_f64_err(d_tar, d_src, hyps, n, n, max_iter, tol, d_T, d_iters + k * H, d_score + k * H,
+                                        c->stream)))
+            return rc;
+        if (k == 0 && K > 1) B2S_CUDA(cudaStreamWaitEvent(c->stream, c->joined, 0));  // the odometry, for the next prior
+        if ((rc = b2s_track_step(d_T, d_score + k * H, next ? d_odo + k * 9 : nullptr, hyps, (int)k, prior,
+                                 d_pose + k * H * 3, next, d_joint, d_fin, c->stream)))
+            return rc;
+        tr.mark("track stage done", (int)k, c->stream);
+    }
+    if ((rc = b2s_track_select(d_joint, d_fin, hyps, d_best, c->stream))) return rc;
+    tr.mark("select done", 0, c->stream);
+    B2S_CUDA(cudaMemcpyAsync(best_out, d_best, sizeof(int32_t), cudaMemcpyDeviceToHost, c->stream));
+    B2S_CUDA(cudaMemcpyAsync(pose_out, d_pose, K * H * 3 * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
+    if (score_out) B2S_CUDA(cudaMemcpyAsync(score_out, d_score, K * H * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
+    if (joint_out) B2S_CUDA(cudaMemcpyAsync(joint_out, d_joint, H * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
+    if (prior_out)
+        B2S_CUDA(cudaMemcpyAsync(prior_out, d_prior, K * H * 3 * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
+    return icp_read_back(c, tr, (int)(K * H), nullptr, iters_out);
+}
+
 extern "C" int b2s_icp_find_nearest(b2s_icp *c, const double *src_xy, int n, const double *tar_xy,
                                     int m, double *dist_out, int64_t *idx_out)
 {

@@ -10,6 +10,8 @@
 //   relocalize    the selection among map observations at many candidate poses: per scan the lowest finite
 //                 mean_error ([ICP]:75), ties to the lower index, composed with its candidate ([ICP]:185-190); for the
 //                 coarse-to-fine form, the `keep` best coarse hypotheses per scan (radix select) and their rows.
+//   track         hypotheses carried through consecutive scans: per stage the map observation's pose, the next
+//                 prior moved by the odometry, the summed score; then the lowest finite joint score.
 #include "b2s_common.cuh"
 
 #include <math.h>
@@ -237,6 +239,16 @@ __device__ __forceinline__ void select_better(double &bs, int &bh, double s, int
     }
 }
 
+// [ICP]:185-190, the pose-chain step p (+) t of one transform t [9]: the relocalization's and the tracking's poses
+__device__ __forceinline__ void pose_step(const double *p, const double *t, double *out)
+{
+    const double x = p[0], y = p[1], yaw = p[2];
+    const double c = cos(yaw), s = sin(yaw);
+    out[0] = x + c * t[2] - s * t[5];
+    out[1] = y + s * t[2] + c * t[5];
+    out[2] = yaw + atan2(t[3], t[0]);
+}
+
 template <bool KEPT>
 __global__ void __launch_bounds__(SELECT_THREADS)
 relocalize_select_kernel(const double *__restrict__ score, const double *__restrict__ T,
@@ -277,13 +289,65 @@ relocalize_select_kernel(const double *__restrict__ score, const double *__restr
         pose[0] = pose[1] = pose[2] = __longlong_as_double(0x7ff8000000000000LL);
         return;
     }
-    // [ICP]:185-190, the pose-chain step of one transform
-    const double *t = Tk + (size_t)bh * 9;
-    const double x = cand[3 * (size_t)bc], y = cand[3 * (size_t)bc + 1], yaw = cand[3 * (size_t)bc + 2];
-    const double c = cos(yaw), s = sin(yaw);
-    pose[0] = x + c * t[2] - s * t[5];
-    pose[1] = y + s * t[2] + c * t[5];
-    pose[2] = yaw + atan2(t[3], t[0]);
+    pose_step(cand + 3 * (size_t)bc, Tk + (size_t)bh * 9, pose);
+}
+
+// Pose tracking, the step after stage k's solves: thread h composes pose[h] = prior[h] (+) T[h], adds the stage's
+// score to joint[h] (from 0.0 at stage 0, in ascending k) and keeps finite[h] only while the score, all nine entries
+// of T and the pose stay finite; before the last stage it also writes the next prior, pose[h] (+) odo, into the pose
+// rows the next stage's virtual scans read.  A track that went non-finite keeps running on whatever it holds.
+constexpr int TRACK_THREADS = 256;
+
+__global__ void __launch_bounds__(TRACK_THREADS)
+track_step_kernel(const double *__restrict__ T, const double *__restrict__ score, const double *__restrict__ odo,
+                  int hyps, int stage, const double *__restrict__ prior, double *__restrict__ pose,
+                  double *__restrict__ next_prior, double *__restrict__ joint, int32_t *__restrict__ finite)
+{
+    const int h = blockIdx.x * blockDim.x + threadIdx.x;
+    if (h >= hyps) return;
+    const double s = score[h];
+    const double *t = T + (size_t)h * 9;
+    bool fin = fabs(s) < INFINITY;  // false for NaN and +-inf
+    for (int i = 0; i < 9; ++i) fin = fin && fabs(t[i]) < INFINITY;
+    double q[3];
+    pose_step(prior + 3 * (size_t)h, t, q);
+    fin = fin && fabs(q[0]) < INFINITY && fabs(q[1]) < INFINITY && fabs(q[2]) < INFINITY;
+    pose[3 * (size_t)h] = q[0];
+    pose[3 * (size_t)h + 1] = q[1];
+    pose[3 * (size_t)h + 2] = q[2];
+    joint[h] = (stage == 0 ? 0.0 : joint[h]) + s;
+    finite[h] = (stage == 0 || finite[h]) && fin;
+    if (odo) pose_step(q, odo, next_prior + 3 * (size_t)h);
+}
+
+// Pose tracking, the selection: the smallest (joint, h) among the finite tracks, -1 when none is (one CTA).
+constexpr int TRACK_SELECT_THREADS = 1024;
+
+__global__ void __launch_bounds__(TRACK_SELECT_THREADS)
+track_select_kernel(const double *__restrict__ joint, const int32_t *__restrict__ finite, int hyps,
+                    int32_t *__restrict__ best_out)
+{
+    __shared__ double ws[TRACK_SELECT_THREADS / 32];
+    __shared__ int wh[TRACK_SELECT_THREADS / 32];
+    double bs = 0.0;
+    int bh = -1;
+    for (int h = threadIdx.x; h < hyps; h += blockDim.x)
+        if (finite[h]) select_better(bs, bh, joint[h], h);
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        const double os = __shfl_xor_sync(0xffffffffu, bs, o);
+        const int oh = __shfl_xor_sync(0xffffffffu, bh, o);
+        select_better(bs, bh, os, oh);
+    }
+    if (lane == 0) {
+        ws[warp] = bs;
+        wh[warp] = bh;
+    }
+    __syncthreads();
+    if (threadIdx.x != 0) return;
+    for (int w = 1; w < (int)(blockDim.x >> 5); ++w) select_better(bs, bh, ws[w], wh[w]);
+    *best_out = bh;
 }
 
 // Coarse-to-fine relocalization, the keep step: CTA k picks the `keep` best of scan k's `hyps` coarse hypotheses and
@@ -544,6 +608,28 @@ extern "C" int b2s_relocalize_keep(const double *score, const double *T, int sca
     B2S_REQUIRE(score && T && keys && kept_out, "b2s_relocalize_keep: null pointer");
     relocalize_keep_kernel<<<scans, KEEP_THREADS, 0, (cudaStream_t)stream>>>(score, T, hyps, keep < hyps ? keep : hyps,
                                                                              (unsigned long long *)keys, kept_out);
+    B2S_CUDA(cudaGetLastError());
+    return B2S_OK;
+}
+
+extern "C" int b2s_track_step(const double *T, const double *score, const double *odometry, int hyps, int stage,
+                              const double *prior, double *pose, double *next_prior, double *joint, int32_t *finite,
+                              void *stream)
+{
+    B2S_REQUIRE(hyps > 0 && stage >= 0, "b2s_track_step: bad sizes");
+    B2S_REQUIRE(T && score && prior && pose && joint && finite, "b2s_track_step: null pointer");
+    B2S_REQUIRE((odometry == nullptr) == (next_prior == nullptr), "b2s_track_step: odometry and next_prior go together");
+    track_step_kernel<<<(unsigned)((hyps + TRACK_THREADS - 1) / TRACK_THREADS), TRACK_THREADS, 0, (cudaStream_t)stream>>>(
+        T, score, odometry, hyps, stage, prior, pose, next_prior, joint, finite);
+    B2S_CUDA(cudaGetLastError());
+    return B2S_OK;
+}
+
+extern "C" int b2s_track_select(const double *joint, const int32_t *finite, int hyps, int32_t *best_out, void *stream)
+{
+    B2S_REQUIRE(hyps > 0, "b2s_track_select: bad sizes");
+    B2S_REQUIRE(joint && finite && best_out, "b2s_track_select: null pointer");
+    track_select_kernel<<<1, TRACK_SELECT_THREADS, 0, (cudaStream_t)stream>>>(joint, finite, hyps, best_out);
     B2S_CUDA(cudaGetLastError());
     return B2S_OK;
 }

@@ -197,6 +197,42 @@ def relocalize_keep(score, T, keep, kept_out=None, keys=None):
     return kept_out
 
 
+def track_step(T, score, prior, pose, joint, finite, stage, odometry=None, next_prior=None):
+    """b2s_track_step: one stage of pose tracking after that stage's solves.  T (H,3,3) and score (H,) float64 (icp_batch_err
+    at the H priors), prior (H,3) float64; pose (H,3) float64 receives prior (+) T ([ICP]:185-190), joint (H,) float64
+    the running score sum (started from 0.0 at stage 0) and finite (H,) int32 the running finiteness of score, T and
+    pose.  With odometry (3,3) float64, next_prior (H,3) receives pose (+) odometry; both are None at the last stage."""
+    H = score.shape[0]
+    for t, shape, name in ((T, (H, 3, 3), "T"), (prior, (H, 3), "prior"), (pose, (H, 3), "pose"), (joint, (H,), "joint"),
+                           (finite, (H,), "finite"), (odometry, (3, 3), "odometry"), (next_prior, (H, 3), "next_prior")):
+        if t is not None and tuple(t.shape) != shape:
+            raise ValueError("%s must have shape %s, got %s" % (name, shape, tuple(t.shape)))
+    if (odometry is None) != (next_prior is None):
+        raise ValueError("odometry and next_prior go together")
+    rc = _lib.lib().b2s_track_step(
+        _chk(T, torch.float64, "T"), _chk(score, torch.float64, "score"),
+        None if odometry is None else _chk(odometry, torch.float64, "odometry"), H, int(stage),
+        _chk(prior, torch.float64, "prior"), _chk(pose, torch.float64, "pose"),
+        None if next_prior is None else _chk(next_prior, torch.float64, "next_prior"), _chk(joint, torch.float64, "joint"),
+        _chk(finite, torch.int32, "finite"), _stream())
+    _lib.check(rc)
+    return pose
+
+
+def track_select(joint, finite, best_out=None):
+    """b2s_track_select: joint (H,) float64 and finite (H,) int32 CUDA tensors -> best (1,) int32, the lowest-index
+    smallest joint score among the finite tracks, or -1."""
+    H = joint.shape[0]
+    if tuple(finite.shape) != (H,):
+        raise ValueError("finite must have shape %s, got %s" % ((H,), tuple(finite.shape)))
+    if best_out is None:
+        best_out = torch.empty(1, dtype=torch.int32, device=joint.device)
+    rc = _lib.lib().b2s_track_select(_chk(joint, torch.float64, "joint"), _chk(finite, torch.int32, "finite"), H,
+                                     _chk(best_out, torch.int32, "best_out"), _stream())
+    _lib.check(rc)
+    return best_out
+
+
 def virtual_scan_batch(obs_x, obs_y, poses, angle_min, angle_increment, beams, far_range=100.0, beam_cs=None,
                        ranges=None, tar_xy=None):
     """b2s_virtual_scan_batch: laserEstimation for K poses at once.  obs_x, obs_y float64 (C,) obstacle cell centres,

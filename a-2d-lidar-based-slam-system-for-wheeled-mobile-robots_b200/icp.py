@@ -383,6 +383,59 @@ class ICP(object):
         out += (T,) if return_T else ()
         return tuple(a[0] for a in out) if one else out
 
+    def track(self, ranges, starts, angle_min, angle_max, angle_increment=None, clamp_inf_to=None, far_range=100.0,
+              max_iter=None, tolerance=None, return_priors=False):
+        """Pose tracking in the static map (set_static_map): H pose hypotheses carried through K consecutive scans, the
+        W9 localization loop ([LOC9]:66-126) over a recorded stream with the map observation taken as the pose (no
+        EKF).  With one start it localizes a stream from a known pose; with many it relocalizes from K scans jointly.
+
+        ranges (K,N) float32, oldest first; starts (H,3) float64 x, y, yaw at scan 0, or (3,) for one track.  The
+        odometry O[k] (k >= 1) is process_scans(ranges, angle_min, angle_max, clamp_inf_to)[0][k-1], bit for bit.  Stage
+        k of track h: prior[h,0] = starts[h]; prior[h,k] = pose[h,k-1] (+) O[k]; the map observation of scan k at
+        prior[h,k] gives T, iterations and score exactly as relocalize(ranges[k:k+1], prior[h,k][None]) does; pose[h,k]
+        = prior[h,k] (+) T.  (+) is the pose-chain step of [ICP]:185-190 (yaw not wrapped).  joint[h] is the float64 sum
+        of score[h,0..K-1] in ascending k from 0.0.  best is the h with the smallest joint score among the tracks whose
+        every score, T and pose is finite, the lowest h on ties, or -1 when none is; the current pose is
+        pose[best, K-1].  A track that goes non-finite runs to the end and is excluded.
+
+        Returns (best int, pose (H,K,3), score (H,K), iterations (H,K) int32, joint (H,)), plus prior (H,K,3) with
+        return_priors=True; for starts of shape (3,) the H axis is dropped.  A NaN start raises ValueError like the
+        reference's int(), before any device work; the other errors are those of relocalize.
+        """
+        ranges = np.ascontiguousarray(ranges, dtype=np.float32)
+        if ranges.ndim != 2 or ranges.shape[0] < 1 or ranges.shape[1] < 1:
+            raise ValueError("expected ranges (K,N) with K, N >= 1, got %s" % (ranges.shape,))
+        K, N = ranges.shape
+        starts = np.asarray(starts, dtype=np.float64)
+        one = starts.ndim == 1
+        starts = np.ascontiguousarray(starts[None] if one else starts)
+        if starts.ndim != 2 or starts.shape[1] != 3 or starts.shape[0] < 1:
+            raise ValueError("expected starts (H,3) with H >= 1 or (3,), got %s" % (starts.shape,))
+        H = starts.shape[0]
+        if K * H > 0x7fffffff:  # (checked here too, before the result arrays are allocated)
+            raise ValueError("scans * hypotheses = %d exceeds 2^31 - 1" % (K * H))
+        if angle_increment is None:
+            if N < 2:
+                raise ValueError("a one-beam scan needs an explicit angle_increment")
+            angle_increment = (float(angle_max) - float(angle_min)) / (N - 1)
+        cs = self._beam_table(angle_min, angle_max, N)
+        best = np.empty(1, dtype=np.int32)
+        pose = np.empty((K, H, 3))
+        score = np.empty((K, H))
+        iters = np.empty((K, H), dtype=np.int32)
+        joint = np.empty(H)
+        prior = np.empty((K, H, 3)) if return_priors else None
+        _lib.check(self._L.b2s_icp_track(
+            self._h, _lib.ptr(ranges), _lib.ptr(starts), _lib.ptr(cs), float(clamp_inf_to or 0.0), K, H, N,
+            float(angle_min), float(angle_increment), float(far_range),
+            self.max_iter if max_iter is None else int(max_iter),
+            self.tolerance if tolerance is None else float(tolerance),
+            _lib.ptr(best), _lib.ptr(pose), _lib.ptr(score), _lib.ptr(iters), _lib.ptr(joint), _lib.ptr(prior)))
+        out = (int(best[0]), np.ascontiguousarray(pose.transpose(1, 0, 2)), np.ascontiguousarray(score.T),
+               np.ascontiguousarray(iters.T), joint)
+        out += (np.ascontiguousarray(prior.transpose(1, 0, 2)),) if return_priors else ()
+        return (out[0],) + tuple(a[0] for a in out[1:]) if one else out
+
     def process_scans(self, ranges, angle_min, angle_max, clamp_inf_to=None, state=None, max_iter=None,
                       tolerance=None):
         """process_sequence / odometry fed with what the sensor delivers: ranges (K,N) float32 (LaserScan.ranges of

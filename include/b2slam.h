@@ -235,6 +235,17 @@ int b2s_relocalize_keep(const double *score, const double *T, int scans, int hyp
  * the winner (-1 and a NaN pose when no survivor is finite). */
 int b2s_relocalize_select_kept(const double *score, const double *T, const double *candidates3, const int32_t *kept,
                                int scans, int keep, int32_t *best_out, double *pose_out, void *stream);
+/* One stage of pose tracking (b2s_icp_track), after the stage's solves of `hyps` hypotheses: T [hyps][9] and score
+ * [hyps] (b2s_icp_batch_f64_err), prior [hyps][3] the poses the stage's virtual scans were built at.  pose [hyps][3]
+ * gets prior[h] composed with T[h] by the pose-chain step of [ICP]:185-190; joint [hyps] gets score[h] added (stage 0
+ * starts it from 0.0); finite [hyps] stays 1 only while the score, all nine entries of T and the pose are finite (stage
+ * 0 starts it).  With odometry (9 doubles, the next stage's scan-to-scan transform), next_prior [hyps][3] gets pose[h]
+ * composed with it; odometry and next_prior are both NULL at the last stage. */
+int b2s_track_step(const double *T, const double *score, const double *odometry, int hyps, int stage,
+                   const double *prior, double *pose, double *next_prior, double *joint, int32_t *finite, void *stream);
+/* The selection of pose tracking: best_out[0] is the h with the smallest joint[h] among those with finite[h] != 0, the
+ * lowest h on ties, or -1 when none is. */
+int b2s_track_select(const double *joint, const int32_t *finite, int hyps, int32_t *best_out, void *stream);
 
 /* Sum of per-GPU count deltas (no reference counterpart: the reference is single-process).
  * In-place ncclAllReduce(int32, sum) of both planes on an existing communicator. */
@@ -388,6 +399,20 @@ int b2s_icp_relocalize_keep(b2s_icp *icp, const float *ranges, const double *can
                             double clamp_inf_to, int scans, int hyps, int n, double angle_min, double angle_increment,
                             double far_range, int max_iter, double tol, int keep, int coarse_iters, int32_t *best_out,
                             double *pose_out, int32_t *kept_out, double *score_out, int32_t *iters_out, double *T_out);
+/* Pose tracking in the static map: `hyps` pose hypotheses carried through `scans` consecutive scans (ranges
+ * [scans][n], oldest first) from starts3 [hyps][3] = x, y, yaw at scan 0.  The odometry O[k] (k >= 1) is
+ * b2s_icp_process_scans' transform of pair (k - 1, k), bit for bit.  Stage k of hypothesis h: prior[h][0] = starts3[h],
+ * prior[h][k] = pose[h][k - 1] composed with O[k]; the map observation of ranges[k] at prior[h][k] (b2s_icp_relocalize
+ * of that scan at that one candidate, bit for bit) gives T, iterations and score; pose[h][k] = prior[h][k] composed
+ * with T (b2s_track_step).  joint[h] is the float64 sum of the scores in ascending k from 0.0; best_out[0]
+ * (b2s_track_select) is the h with the smallest joint score among the tracks whose every score, T and pose is finite,
+ * the lowest h on ties, or -1.  pose_out and prior_out are [scans][hyps][3], score_out and iters_out [scans][hyps],
+ * joint_out [hyps]; score_out, iters_out, joint_out and prior_out may be NULL.  scans >= 1; the other sizes and errors
+ * are b2s_icp_relocalize's. */
+int b2s_icp_track(b2s_icp *icp, const float *ranges, const double *starts3, const double *beam_cs, double clamp_inf_to,
+                  int scans, int hyps, int n, double angle_min, double angle_increment, double far_range, int max_iter,
+                  double tol, int32_t *best_out, double *pose_out, double *score_out, int32_t *iters_out,
+                  double *joint_out, double *prior_out);
 int b2s_icp_find_nearest(b2s_icp *icp, const double *src_xy, int n, const double *tar_xy, int m,
                          double *dist_out, int64_t *idx_out);
 int b2s_icp_get_transform(b2s_icp *icp, const double *src_xy, const double *tar_xy, int n,
