@@ -21,7 +21,8 @@ namespace b2s {
 constexpr int CHAIN_THREADS = 1024;
 
 // Exclusive prefix over a CTA of 1024 threads of one value per thread; returns this thread's offset, total in *total.
-// scratch: 64 values of shared memory.
+// scratch: 64 values of shared memory.  The offset is a sum of the values below this thread only: it is the inclusive
+// value of the lane below, never inclusive minus own, so a NaN or inf of this thread cannot reach its own offset.
 template <class V>
 __device__ __forceinline__ V cta_exclusive_scan(V v, V *scratch, V *total)
 {
@@ -32,6 +33,8 @@ __device__ __forceinline__ V cta_exclusive_scan(V v, V *scratch, V *total)
         const V up = __shfl_up_sync(0xffffffffu, inc, o);
         if (lane >= o) inc += up;
     }
+    const V below = __shfl_up_sync(0xffffffffu, inc, 1);
+    const V exc = lane ? below : V(0);
     if (lane == 31) scratch[warp] = inc;
     __syncthreads();
     if (warp == 0) {
@@ -47,7 +50,7 @@ __device__ __forceinline__ V cta_exclusive_scan(V v, V *scratch, V *total)
     const V before_warp = warp ? scratch[32 + warp - 1] : V(0);
     *total = scratch[63];
     __syncthreads();
-    return before_warp + inc - v;
+    return before_warp + exc;
 }
 
 __global__ void __launch_bounds__(CHAIN_THREADS)
